@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- cell-timesteps/s of the pt_gs_k run_cells hot path (BASELINE.json), one JSON line on stdout.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--cells C] [--years Y] [--window S]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--cells C] [--years Y] [--window S] [--dump-outputs DIR]
   python bench.py --impl reference ...      # the CPU path (oracle port; the real reference cannot be built here)
 
 A "step" is one pass of the hot path over the whole workload: BASELINE configs[1], pt_gs_k, 100 000 cells x 10 years
@@ -31,9 +31,12 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the tree it runs from as it found it (no __pycache__)
 
 BYTES_PER_CELL_STEP = 56  # 5 forcings read + avg_discharge, charge_m3s written (BASELINE.md section 3)
 NCU_PROFILE = os.path.join(ROOT, "profiles", "ncu_pipeline_r02_shipped.json")  # tools/ncu_pipeline_json.py of the shipped configuration
+DUMP_BYTES = 60 * 10**6   # --dump-outputs: data budget, so that the files with their .npy headers stay under 64 MB
+DUMP_SEED = 20260101
 PTGSK_DEFAULT = [-2.439, 0.966, -0.10, 1.5, -0.5, 2.0, 0.1, 1.0, 5.0, 5.0, 30.0, 0.9, 0.6, 5.0, 0.4, 0.4, 1.0, 0.0, 0.0, 0.2, 1.26, 0.04, 100.0, 0.0,
                  6.0, 1.0, 7.0, 0.0, 221.0, 0.0, 1.0]
 
@@ -50,7 +53,14 @@ def parse():
     ap.add_argument("--window", type=int, default=4096, help="time steps per forcing window (round 2, with one launch set per window: 2048 -> 9.54, 4096 -> 9.62 G cell-steps/s)")
     ap.add_argument("--cpu-seconds", type=float, default=15.0, help="target CPU work of the cpu_baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the CPU oracle legs (cpu_baseline and config.parity_check)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (catchment discharge and charge series, end states) as DIR/<name>.npy, "
+                         "float64; above %d MB together every array keeps the same seeded sample of its rows" % (DUMP_BYTES // 10**6))
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     a.cells_given = a.cells > 0
     if not a.cells_given:
@@ -125,6 +135,23 @@ def pinned_copy(a):
     v = t.numpy()
     v[...] = a
     return v, t
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BYTES):
+    """Write each array of `arrays` as out_dir/<name>.npy in float64.  When they take more than `budget` bytes together, every array
+    keeps the same fraction of its rows (axis 0), drawn with a fixed seed and kept in order, so that two runs with the same arguments
+    write the same rows.  -> {name: [rows written, rows computed]}"""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float64) for k, v in arrays.items()}
+    frac = min(1.0, budget / max(1, sum(a.nbytes for a in arrays.values())))
+    kept = {}
+    for name, a in arrays.items():
+        k = max(1, int(a.shape[0] * frac))
+        if k < a.shape[0]:
+            a = a[np.sort(np.random.default_rng(DUMP_SEED).choice(a.shape[0], k, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        kept[name] = [int(a.shape[0]), int(arrays[name].shape[0])]
+    return kept
 
 
 FORCING = ("temperature", "precipitation", "radiation", "wind_speed", "rel_hum")
@@ -383,6 +410,13 @@ def main():
     launches = m.kernel_launches() - l0
     clocks = sampler.stop() if sampler else None
     cq_device = m.catchment_discharges() if world == 1 else reduced["q"].cpu().numpy()
+    last_step = None
+    if args.dump_outputs:
+        # what a caller of the timed path receives from its last step; at N > 1 the region's all-reduced series and rank 0's end states
+        last_step = {"catchment_discharge": cq_device,
+                     "catchment_charge": m.catchment_charges() if world == 1 else
+                     sharding.global_catchment_series(m, global_cids, "charge").cpu().numpy(),
+                     "end_state": m.get_states()}
     chunk_steps = m.step_chunk_steps()
     # end-to-end leg (host buffers)
     e2e_pass()
@@ -477,6 +511,8 @@ def main():
         if not args.no_cpu_baseline and world == 1:
             out["cpu_baseline"] = cpu_baseline(args, geo, ta, env, args.cpu_seconds)
             out["config"]["parity_check"] = parity_check(sb, args, geo, ta, env)
+        if last_step is not None:
+            out["config"]["dump_outputs"] = {"dir": args.dump_outputs, "rows_written_of": dump_outputs(args.dump_outputs, last_step)}
         print(json.dumps(out))
     if world > 1:
         dist.barrier()
