@@ -2078,8 +2078,11 @@ int sb2_run_windowed(sb2_model* m, const sb2_interpolation_parameter* ip, int st
                 m->forcing_rows = W;
             }
             m->forcing_first = w0;
+            // a variable without sources reads NaN; so do the cells outside the calculation filter, which interpolation skips
+            // (the reused window buffers would otherwise show them the previous window's or the previous run's values)
+            const bool filtered = !m->catchment_filter.empty();
             for (int v = 0; v < SB2_N_FORCING; ++v)
-                if (m->src[v].n_src == 0) fill_nan(m, m->d_forcing[v].p, W * m->n);
+                if (m->src[v].n_src == 0 || filtered) fill_nan(m, m->d_forcing[v].p, W * m->n);
             time_begin(m, 0);
             interpolate_range(m, w0, wn, 0);
             CUDA_OK(cudaEventRecord(m->ev[1], m->stream));
