@@ -1449,7 +1449,8 @@ int sb2_set_region_parameter(sb2_model* m, const double* p, int n) {
         if (n != m->n_param) throw Error("parameter vector size does not match parameter::size()");
         m->region_param.assign(p, p + n);
         m->param_dirty = true;
-        m->route.reset();
+        m->route.reset();  // the cells' unit hydrographs carry the routing velocity / alpha / beta of the parameter set
+        m->rlocal_valid = m->rnet_valid = false;
     });
 }
 int sb2_get_region_parameter(const sb2_model* m, double* p, int n) {
@@ -1463,7 +1464,8 @@ int sb2_set_catchment_parameter(sb2_model* m, int64_t cid, const double* p, int 
         if (n != m->n_param) throw Error("parameter vector size does not match parameter::size()");
         m->catch_param[cid].assign(p, p + n);
         m->param_dirty = true;
-        m->route.reset();
+        m->route.reset();  // as sb2_remove_catchment_parameter
+        m->rlocal_valid = m->rnet_valid = false;
     });
 }
 int sb2_get_catchment_parameter(const sb2_model* m, int64_t cid, double* p, int n) {

@@ -26,19 +26,21 @@ constexpr int ROUTE_TT = 64;      // time steps per block
 // local_inflow[r][g0 + t] = sum over the river's cells (ascending cell order, 128 at a time) of sum_j w_c[j] * q_c[t-j], t in [0, n_rows).
 // `q` points at row 0 of a [rows][n_cells] block that also has `hist` valid rows BEFORE row 0 (the tail of the previous
 // window); rows further back are before the start of the axis or not needed and read as zero (USE_ZERO, time_series.h:966-975).
-// grid (time tiles, rivers); dynamic smem: (ROUTE_TT + max_len - 1) * ROUTE_CELLS doubles
+// uhg_w rows are w_stride apart; depth (>= every cell UHG length, <= w_stride) is the tile's history depth: the river UHGs that
+// share the table may be longer, but they never go through this tile.
+// grid (time tiles, rivers); dynamic smem: (ROUTE_TT + depth - 1) * ROUTE_CELLS doubles
 __global__ void __launch_bounds__(ROUTE_CELLS) route_local_inflow_kernel(const double* __restrict__ q, int64_t n_cells, int64_t n_rows, int64_t hist,
                                                                          int64_t g0, int64_t T, const int32_t* __restrict__ riv_ptr,
                                                                          const int32_t* __restrict__ riv_cells,
                                                                          const int32_t* __restrict__ cell_uhg_id /* per gathered cell */,
                                                                          const int32_t* __restrict__ uhg_len, const double* __restrict__ uhg_w,
-                                                                         int max_len, double* __restrict__ local /* [n_riv][T] */) {
-    extern __shared__ double sq[];  // [(ROUTE_TT + max_len - 1)][ROUTE_CELLS]
+                                                                         int w_stride, int depth, double* __restrict__ local /* [n_riv][T] */) {
+    extern __shared__ double sq[];  // [(ROUTE_TT + depth - 1)][ROUTE_CELLS]
     __shared__ double acc[ROUTE_TT];
     const int r = blockIdx.y;
     const int64_t t0 = (int64_t)blockIdx.x * ROUTE_TT;
     const int nt = int(min((int64_t)ROUTE_TT, n_rows - t0));
-    const int rows = ROUTE_TT + max_len - 1;
+    const int rows = ROUTE_TT + depth - 1;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     if (threadIdx.x < ROUTE_TT) acc[threadIdx.x] = 0.0;
     for (int k0 = riv_ptr[r]; k0 < riv_ptr[r + 1]; k0 += ROUTE_CELLS) {
@@ -48,7 +50,7 @@ __global__ void __launch_bounds__(ROUTE_CELLS) route_local_inflow_kernel(const d
             const int c = threadIdx.x;
             const int64_t cell = c < nc ? riv_cells[k0 + c] : -1;
             for (int row = 0; row < rows; ++row) {
-                const int64_t t = t0 - (max_len - 1) + row;  // row of the block, may be negative (history)
+                const int64_t t = t0 - (depth - 1) + row;  // row of the block, may be negative (history)
                 sq[row * ROUTE_CELLS + c] = (cell >= 0 && t >= -hist && t < n_rows && g0 + t >= 0) ? q[t * n_cells + cell] : 0.0;
             }
         }
@@ -59,9 +61,9 @@ __global__ void __launch_bounds__(ROUTE_CELLS) route_local_inflow_kernel(const d
             for (int c = lane; c < nc; c += 32) {
                 const int id = cell_uhg_id[k0 + c];
                 const int len = uhg_len[id];
-                const double* w = uhg_w + (int64_t)id * max_len;
+                const double* w = uhg_w + (int64_t)id * w_stride;
                 double v = 0.0;
-                for (int j = 0; j < len; ++j) v += w[j] * sq[(ti + max_len - 1 - j) * ROUTE_CELLS + c];
+                for (int j = 0; j < len; ++j) v += w[j] * sq[(ti + depth - 1 - j) * ROUTE_CELLS + c];
                 s += v;
             }
 #pragma unroll
@@ -182,8 +184,11 @@ inline std::unique_ptr<RoutingPlan> build_routing_plan(const std::vector<double>
         riv_uhg[r] = tab.id_of(host::uhg_steps(rivers[6 * r + 2], rivers[6 * r + 3], dt_us), rivers[6 * r + 4], rivers[6 * r + 5]);
     }
     for (auto& w : tab.w) pl->max_len = std::max(pl->max_len, int(w.size()));
-    if (size_t(ROUTE_TT + pl->max_len - 1) * ROUTE_CELLS * sizeof(double) > 200 * 1024)
-        throw std::runtime_error("routing: unit hydrograph too long for the shared-memory tile");
+    // the shared-memory tiles: cell discharge of the local-inflow kernel, input sum of the river-level kernel
+    if (size_t(ROUTE_TT + pl->cell_max_len - 1) * ROUTE_CELLS * sizeof(double) > 200 * 1024)
+        throw std::runtime_error("routing: cell unit hydrograph too long for the shared-memory tile");
+    if (size_t(ROUTE_TT + pl->max_len - 1) * sizeof(double) > 200 * 1024)
+        throw std::runtime_error("routing: river unit hydrograph too long for the shared-memory tile");
     std::vector<int32_t> uhg_len(tab.w.size());
     std::vector<double> uhg_w(tab.w.size() * pl->max_len, 0.0);
     for (size_t i = 0; i < tab.w.size(); ++i) {
@@ -237,11 +242,11 @@ inline std::unique_ptr<RoutingPlan> build_routing_plan(const std::vector<double>
 // cell -> river: the local inflow of every river over block rows [0, n_rows) = global steps [g0, g0 + n_rows)
 inline void routing_local_inflow(const RoutingPlan& pl, const double* d_q_row0, int64_t n_cells, int64_t n_rows, int64_t hist, int64_t g0, int64_t T,
                                  double* d_local, cudaStream_t stream, int64_t* launches) {
-    const size_t smem = size_t(ROUTE_TT + pl.max_len - 1) * ROUTE_CELLS * sizeof(double);
+    const size_t smem = size_t(ROUTE_TT + pl.cell_max_len - 1) * ROUTE_CELLS * sizeof(double);
     if (smem > 48 * 1024) cudaFuncSetAttribute(route_local_inflow_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
     const unsigned tiles = unsigned((n_rows + ROUTE_TT - 1) / ROUTE_TT);
     route_local_inflow_kernel<<<dim3(tiles, pl.n_riv), ROUTE_CELLS, smem, stream>>>(d_q_row0, n_cells, n_rows, hist, g0, T, pl.d_ptr, pl.d_cells, pl.d_cuhg,
-                                                                                  pl.d_len, pl.d_w, pl.max_len, d_local);
+                                                                                  pl.d_len, pl.d_w, pl.max_len, pl.cell_max_len, d_local);
     ++*launches;
     if (cudaGetLastError() != cudaSuccess) throw std::runtime_error("routing: kernel launch failed");
 }
@@ -251,6 +256,7 @@ inline void routing_network(const RoutingPlan& pl, int64_t T, const double* d_lo
     cudaMemsetAsync(d_up, 0, size_t(pl.n_riv) * T * sizeof(double), stream);
     const unsigned tiles = unsigned((T + ROUTE_TT - 1) / ROUTE_TT);
     const size_t smem = size_t(ROUTE_TT + pl.max_len - 1) * sizeof(double);
+    if (smem > 48 * 1024) cudaFuncSetAttribute(route_river_level_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
     for (int lv = 0; lv < pl.n_levels; ++lv) {
         const int cnt = pl.level_begin[lv + 1] - pl.level_begin[lv];
         route_river_level_kernel<<<dim3(tiles, cnt), ROUTE_TT, smem, stream>>>(pl.d_order + pl.level_begin[lv], pl.d_upp, pl.d_upi, pl.d_ruhg, pl.d_len,
