@@ -6,6 +6,7 @@ torch / Python dependency: it is the C-ABI of include/shyft_b200.h and nothing e
 import os
 import shutil
 import subprocess
+import tempfile
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
@@ -41,32 +42,34 @@ def nvcc_path():
     return p
 
 
-def build_library(force=False, verbose=False, extra_flags=(), output=None):
+def build_library(force=False, verbose=False):
     """Compile shyft_b200/csrc/sb2_capi.cu -> shyft_b200/libshyft_b200.so for sm_100a."""
-    out = output or LIB
-    if not force and not _stale(out, _sources()):
-        return out
-    tmp = out + ".tmp%d" % os.getpid()   # written aside and renamed: a concurrent reader never sees a half-written library
-    cmd = [nvcc_path()] + NVCC_FLAGS + list(extra_flags) + ["-shared", "-o", tmp, os.path.join(CSRC, "sb2_capi.cu")]
+    if not force and not _stale(LIB, _sources()):
+        return LIB
+    tmp = LIB + ".tmp%d" % os.getpid()   # written aside and renamed: a concurrent reader never sees a half-written library
+    cmd = [nvcc_path()] + NVCC_FLAGS + ["-shared", "-o", tmp, os.path.join(CSRC, "sb2_capi.cu")]
     if verbose:
         cmd.insert(1, "-Xptxas=-v")
     try:
         subprocess.check_call(cmd, cwd=CSRC)
-        os.replace(tmp, out)
+        os.replace(tmp, LIB)
     finally:
         if os.path.exists(tmp):
             os.remove(tmp)
-    return out
+    return LIB
 
 
 def build_host_shim_test(force=False):
-    """g++ build of the C++ host shim self test (include/shyft_b200/region_model.hpp over the C ABI)."""
+    """g++ build of the C++ host shim self test (include/shyft_b200/region_model.hpp over the C ABI).  In a read-only checkout a
+    missing or stale executable is built into a temporary directory instead of tests/cpp; returns the executable's path."""
     src = os.path.join(ROOT, "tests", "cpp", "shim_selftest.cpp")
     out = os.path.join(ROOT, "tests", "cpp", "shim_selftest")
     if not os.path.exists(src):
         return None
     deps = [src, os.path.join(ROOT, "include", "shyft_b200.h"), os.path.join(ROOT, "include", "shyft_b200", "region_model.hpp"), LIB]
     if force or _stale(out, deps):
+        if not os.access(os.path.dirname(out), os.W_OK):
+            out = os.path.join(tempfile.mkdtemp(prefix="shyft_b200_shim_"), "shim_selftest")
         subprocess.check_call(["g++", "-O2", "-std=c++17", "-I", os.path.join(ROOT, "include"), "-o", out, src, "-L", HERE, "-lshyft_b200",
                                "-Wl,-rpath," + HERE, "-Wl,-rpath,$ORIGIN/../../shyft_b200"])
     return out

@@ -95,7 +95,7 @@ def lib():
     global _LIB
     if _LIB is not None:
         return _LIB
-    path = os.environ.get("SB2_LIB") or _build.LIB   # SB2_LIB: a build variant produced by tools/ (tuning runs only)
+    path = os.environ.get("SB2_LIB") or _build.LIB   # SB2_LIB: another build of the library, e.g. for an A/B timing
     if not os.path.exists(path) or os.environ.get("SB2_REBUILD"):
         try:  # normally __graft_entry__.build() has produced the file and it travels with the tree
             _build.build_library(force=bool(os.environ.get("SB2_REBUILD")))
@@ -125,9 +125,9 @@ def f64(a):
 UNIT_FUNCTIONS = dict(exp=(0, 1, 1), log=(1, 1, 1), pow=(2, 2, 1), lgamma=(3, 1, 1), gamma_p=(4, 2, 1), corr_lwc=(5, 5, 1), calc_snow_state=(6, 7, 2),
                       kirchner_step=(7, 7, 3),
                       # the forms the production kernels use (sb2_unit.cuh)
-                      exp_flat=(8, 1, 1), log_flat=(9, 1, 1), pow_flat=(10, 2, 1), calc_snow_state_hot=(11, 7, 2), kirchner_step_warp=(12, 7, 3),
-                      gamma_p_pair=(13, 4, 2), div_by=(14, 2, 2), kirchner_step_warp_udt=(15, 7, 3), corr_lwc_warp=(16, 6, 1), skaugen_step=(17, 18, 11), sca_rel_red=(18, 4, 2),
-                      hps_step=(19, 41, 27))
+                      exp_flat=(8, 1, 1), log_flat=(9, 1, 1), pow_flat=(10, 2, 1), kirchner_step_warp=(11, 7, 3),
+                      div_by=(12, 2, 2), kirchner_step_warp_udt=(13, 7, 3), skaugen_step=(14, 18, 11), sca_rel_red=(15, 4, 2),
+                      hps_step=(16, 41, 27))
 
 
 def check_guards():

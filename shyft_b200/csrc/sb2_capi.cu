@@ -231,15 +231,8 @@ inline int grid_for(int64_t n, int block) { return int((n + block - 1) / block);
 
 }  // namespace
 
-#ifndef SB2_HBV_UNIT_STEPS
-#define SB2_HBV_UNIT_STEPS 64      // steps per time slice of the pt_hs_k / hbv_stack step kernel (0: whole chunks)
-#endif
-#ifndef SB2_DENSE_TILE_COMPACT
+#define SB2_HBV_UNIT_STEPS 64      // steps per time slice of the pt_ss_k / pt_hps_k / pt_hs_k / hbv_stack step kernels (128: within +-0.7 %)
 #define SB2_DENSE_TILE_COMPACT 32  // steps staged per buffer, compacted inverse distance over 64-station rows
-#endif
-#ifndef SB2_DENSE_TILE_BTK
-#define SB2_DENSE_TILE_BTK 0       // 0 = the default of dense_tile_steps
-#endif
 
 struct sb2_model {
     int stack = 0, device = 0;
@@ -522,10 +515,8 @@ void launch_step_range(sb2_model* m, int64_t first, int64_t n_steps, bool collec
     const double dt_seconds = double(m->dt) / 1e6;
     if (m->partial_steps == 0) {
         // Steps per launch: at most 4 096, and the scratch within 16 GB (measured on 100 000 cells: chunks of 512 / 1 024 / 2 048 / 4 096
-        // steps -> 9.23 / 9.42 / 9.54 / 9.62 G cell-steps/s: every launch ends with a tail of one time slice).  SB2_CHUNK_STEPS /
-        // SB2_SCRATCH_GB in the environment override the two bounds (tuning).
-        static const int64_t cap = [] { const char* e = std::getenv("SB2_CHUNK_STEPS"); return e ? std::max<int64_t>(16, std::atoll(e)) : 4096; }();
-        static const int64_t scratch_gb = [] { const char* e = std::getenv("SB2_SCRATCH_GB"); return e ? std::max<int64_t>(1, std::atoll(e)) : 16; }();
+        // steps -> 9.23 / 9.42 / 9.54 / 9.62 G cell-steps/s: every launch ends with a tail of one time slice).
+        constexpr int64_t cap = 4096, scratch_gb = 16;
         // the per-slot partial sums [ps][n_slots][2] within cap / 4 MB (1 GB at the default)
         int64_t ps = std::max<int64_t>(1, std::min<int64_t>(cap, (int64_t(cap / 4) << 20) / std::max<int64_t>(1, m->n_slots * 16)));
         // pt_gs_k: the five scratch arrays of the phase pipeline are [ps][n] too
@@ -614,7 +605,7 @@ void launch_step_range(sb2_model* m, int64_t first, int64_t n_steps, bool collec
             a.slot = m->d_slot.p; a.partial = m->d_partial.p; a.n_slots = m->n_slots; a.error_flag = m->d_error_flag.p;
             a.collect = m->collect_bits & 15;
             const int g = grid_for(n, block);
-            const bool split = use_time_split(g) && SB2_HBV_UNIT_STEPS > 0;
+            const bool split = use_time_split(g);
             const int n_slices = split ? grid_for(chunk, SB2_HBV_UNIT_STEPS) : 1;
             m->d_tickets.ensure(size_t(1 + g));
             a.unit_steps = split ? SB2_HBV_UNIT_STEPS : 0; a.tickets = m->d_tickets.p; a.progress = m->d_tickets.p + 1;
@@ -638,7 +629,7 @@ void launch_step_range(sb2_model* m, int64_t first, int64_t n_steps, bool collec
             a.slot = m->d_slot.p; a.partial = m->d_partial.p; a.n_slots = m->n_slots; a.error_flag = m->d_error_flag.p;
             a.collect = m->collect_bits & 15;
             const int g = grid_for(n, block);
-            const bool split = use_time_split(g) && SB2_HBV_UNIT_STEPS > 0;
+            const bool split = use_time_split(g);
             const int n_slices = split ? grid_for(chunk, SB2_HBV_UNIT_STEPS) : 1;
             m->d_tickets.ensure(size_t(1 + g));
             a.unit_steps = split ? SB2_HBV_UNIT_STEPS : 0; a.tickets = m->d_tickets.p; a.progress = m->d_tickets.p + 1;
@@ -665,7 +656,7 @@ void launch_step_range(sb2_model* m, int64_t first, int64_t n_steps, bool collec
             a.collect = m->collect_bits & 15;
             const int g = grid_for(n, block);
             // time slices handed out by ticket while the launch is only a few waves of one-warp blocks (see the kernel)
-            const bool split = use_time_split(g) && SB2_HBV_UNIT_STEPS > 0;
+            const bool split = use_time_split(g);
             const int n_slices = split ? grid_for(chunk, SB2_HBV_UNIT_STEPS) : 1;
             m->d_tickets.ensure(size_t(1 + g));
             a.unit_steps = split ? SB2_HBV_UNIT_STEPS : 0; a.tickets = m->d_tickets.p; a.progress = m->d_tickets.p + 1;
@@ -939,7 +930,7 @@ void run_btk(sb2_model* m, int64_t first, int64_t n_steps, double* out) {
     } while (0)
         if (nv <= 16) SB2_BTK(4, 4, 0);
         else if (nv <= 32) SB2_BTK(8, 4, 0);
-        else if (nv <= 64) SB2_BTK(16, 2, SB2_DENSE_TILE_BTK);
+        else if (nv <= 64) SB2_BTK(16, 2, 0);
         else if (nv <= 96) SB2_BTK(24, 1, 0);
         else {  // more stations than the register-resident operator tile holds: one thread per cell, operator rows streamed
             const int tile = idw_tile_steps(nv);
@@ -2406,7 +2397,7 @@ int sb2_calculate_goal_function_batch(sb2_model* m, int64_t n_sets, const double
 // ---- diagnostics ---------------------------------------------------------------------------------------------------------------
 int sb2_unit_eval(int device, int fn, int64_t n, const double* in, int n_in, double* out, int n_out) {
     try {
-        static const int need_in[UNIT_N] = {1, 1, 2, 1, 2, 5, 7, 7, 1, 1, 2, 7, 7, 4, 2, 7, 6, 18, 4, 41}, need_out[UNIT_N] = {1, 1, 1, 1, 1, 1, 2, 3, 1, 1, 1, 2, 3, 2, 2, 3, 1, 11, 2, 27};
+        static const int need_in[UNIT_N] = {1, 1, 2, 1, 2, 5, 7, 7, 1, 1, 2, 7, 2, 7, 18, 4, 41}, need_out[UNIT_N] = {1, 1, 1, 1, 1, 1, 2, 3, 1, 1, 1, 3, 2, 3, 11, 2, 27};
         if (fn < 0 || fn >= UNIT_N) throw Error("unknown unit function");
         if (n_in < need_in[fn] || n_out < need_out[fn]) throw Error("unit function: too few input or output columns");
         CUDA_OK(cudaSetDevice(device));

@@ -243,15 +243,11 @@ __device__ __forceinline__ bool hbv_snow_step(double (&sp)[HBV_NB], double (&sw)
 }
 
 // launch bounds = (threads the register allocation assumes per block, blocks per SM it aims at); blocks are one warp (SB2_BLOCK), so
-// (128, 4) = 128 registers -> 16 resident warps, (128, 5) = 96 registers -> 20.  Measured on 400 000 cells (tools/tune_c3.sh):
+// (128, 4) = 128 registers -> 16 resident warps, (128, 5) = 96 registers -> 20.  Measured on 400 000 cells:
 // pt_hs_k 87.8 ms at the compiler's 146 registers, 78.4 at 128, 79.4 at 96, 89.7 at 80; hbv_stack 49.1 at 122, 49.5 at 128, 46.2 at 96,
 // 47.2 at 80.
-#ifndef SB2_HBV_MINBLOCKS_K
 #define SB2_HBV_MINBLOCKS_K 4   // pt_hs_k (Kirchner)
-#endif
-#ifndef SB2_HBV_MINBLOCKS_S
 #define SB2_HBV_MINBLOCKS_S 5   // hbv_stack (soil + tank)
-#endif
 // UPAR: no catchment override in use -- every cell reads the region parameter set (a.par0) from the kernel's constant bank
 template <bool HBV_STACK, bool UPAR>
 __global__ void __launch_bounds__(128, (HBV_STACK ? SB2_HBV_MINBLOCKS_S : SB2_HBV_MINBLOCKS_K)) hbv_run_kernel(const __grid_constant__ HbvRunArgs a) {
@@ -337,7 +333,7 @@ __global__ void __launch_bounds__(128, (HBV_STACK ? SB2_HBV_MINBLOCKS_S : SB2_HB
             const int64_t o1 = o + n;
             f_t = a.f[0][o1]; f_p = a.f[1][o1]; f_r = a.f[2][o1]; f_h = a.f[4][o1];
         }
-        if (SB2_PREFETCH_AHEAD > 1 && i + SB2_PREFETCH_AHEAD < a.n_steps) {
+        if (i + SB2_PREFETCH_AHEAD < a.n_steps) {
             const int64_t o2 = o + SB2_PREFETCH_AHEAD * n;
             prefetch_l1(a.f[0] + o2); prefetch_l1(a.f[1] + o2); prefetch_l1(a.f[2] + o2); prefetch_l1(a.f[4] + o2);
         }
@@ -352,7 +348,7 @@ __global__ void __launch_bounds__(128, (HBV_STACK ? SB2_HBV_MINBLOCKS_S : SB2_HB
             if (!hbv_snow_step(sp, sw, swe, sca, snow_outflow, p, a.dt_hours, a.step_in_days, a.inv_dt_hours, prec, temp)) failed_snow = true;
             const double sca_m2 = cell_area_m2 * sca;
             gm_melt_m3s = (glacier_area_m2 <= sca_m2 || temp <= 0.0) ? 0.0 : p.gm_dtf * temp * (glacier_area_m2 - sca_m2) * SB2_K(K_GM);  // 0.001 / 86400.0
-            pot = pt_potential_evapotranspiration<true>(p.pt_albedo, p.pt_alpha, temp, rad, rel_hum) * 3600.0;
+            pot = pt_potential_evapotranspiration(p.pt_albedo, p.pt_alpha, temp, rad, rel_hum) * 3600.0;
             gm_mmh = div_pos(gm_melt_m3s, SB2_K(K_MMH_M3S) * cell_area_m2);  // m3s_to_mmh; mostly 0 / x (no melt)
             if (HBV_STACK) {
                 const double snow_fraction = dmax(sca, glacier_fraction);

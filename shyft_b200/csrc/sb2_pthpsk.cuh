@@ -274,9 +274,7 @@ __device__ __forceinline__ bool hps_step(HpsState& s, double& r_outflow, double&
     return ok;
 }
 
-#ifndef SB2_HPS_MINBLOCKS
 #define SB2_HPS_MINBLOCKS 4
-#endif
 __global__ void __launch_bounds__(128, SB2_HPS_MINBLOCKS) pthpsk_run_kernel(const __grid_constant__ HpsRunArgs a) {
     sb_math_stage_tables();
     int64_t group = blockIdx.x;
@@ -353,7 +351,7 @@ __global__ void __launch_bounds__(128, SB2_HPS_MINBLOCKS) pthpsk_run_kernel(cons
             const int64_t o1 = o + n;
             f_t = a.f[0][o1]; f_p = a.f[1][o1]; f_r = a.f[2][o1]; f_w = a.f[3][o1]; f_h = a.f[4][o1];
         }
-        if (SB2_PREFETCH_AHEAD > 1 && i + SB2_PREFETCH_AHEAD < a.n_steps) {
+        if (i + SB2_PREFETCH_AHEAD < a.n_steps) {
             const int64_t o2 = o + SB2_PREFETCH_AHEAD * n;
             prefetch_l1(a.f[0] + o2); prefetch_l1(a.f[1] + o2); prefetch_l1(a.f[2] + o2); prefetch_l1(a.f[3] + o2); prefetch_l1(a.f[4] + o2);
         }
@@ -366,7 +364,7 @@ __global__ void __launch_bounds__(128, SB2_HPS_MINBLOCKS) pthpsk_run_kernel(cons
             if (!hps_step(hs, snow_outflow, r_sca, r_storage, p, a.dt_seconds, a.dt_us, a.bb0, a.inv_dt_seconds, temp, rad, prec, wind, rel_hum)) failed_snow = true;
             const double sca_m2 = cell_area_m2 * hs.sca;
             gm_melt_m3s = (glacier_area_m2 <= sca_m2 || temp <= 0.0) ? 0.0 : p.gm_dtf * temp * (glacier_area_m2 - sca_m2) * SB2_K(K_GM);  // 0.001 / 86400.0
-            pot = pt_potential_evapotranspiration<true>(p.pt_albedo, p.pt_alpha, temp, rad, rel_hum) * 3600.0;
+            pot = pt_potential_evapotranspiration(p.pt_albedo, p.pt_alpha, temp, rad, rel_hum) * 3600.0;
             gm_mmh = div_pos(gm_melt_m3s, SB2_K(K_MMH_M3S) * cell_area_m2);
             ae = pot * (1.0 - sb_exp_flat<true>(div_by(-kq * 3.0, p.inv_ae_scale))) * (1.0 - dmax(hs.sca, glacier_fraction));
         }

@@ -417,7 +417,7 @@ __global__ void __launch_bounds__(128, 4) ptssk_run_kernel(const __grid_constant
             const int64_t o1 = o + n;
             f_t = a.f[0][o1]; f_p = a.f[1][o1]; f_r = a.f[2][o1]; f_h = a.f[4][o1];
         }
-        if (SB2_PREFETCH_AHEAD > 1 && i + SB2_PREFETCH_AHEAD < a.n_steps) {
+        if (i + SB2_PREFETCH_AHEAD < a.n_steps) {
             const int64_t o2 = o + SB2_PREFETCH_AHEAD * n;
             prefetch_l1(a.f[0] + o2); prefetch_l1(a.f[1] + o2); prefetch_l1(a.f[2] + o2); prefetch_l1(a.f[4] + o2);
         }
@@ -432,7 +432,7 @@ __global__ void __launch_bounds__(128, 4) ptssk_run_kernel(const __grid_constant
             failed_snow = failed_snow || bad;
             const double sca_m2 = cell_area_m2 * ss.sca;
             gm_melt_m3s = (glacier_area_m2 <= sca_m2 || temp <= 0.0) ? 0.0 : p.gm_dtf * temp * (glacier_area_m2 - sca_m2) * SB2_K(K_GM);  // 0.001 / 86400.0
-            pot = pt_potential_evapotranspiration<true>(p.pt_albedo, p.pt_alpha, temp, rad, rel_hum) * 3600.0;
+            pot = pt_potential_evapotranspiration(p.pt_albedo, p.pt_alpha, temp, rad, rel_hum) * 3600.0;
             gm_mmh = div_pos(gm_melt_m3s, SB2_K(K_MMH_M3S) * cell_area_m2);
             ae = pot * (1.0 - sb_exp_flat<true>(div_by(-kq * 3.0, p.inv_ae_scale))) * (1.0 - dmax(ss.sca, glacier_fraction));
         }

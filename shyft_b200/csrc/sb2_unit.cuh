@@ -8,12 +8,10 @@
 namespace sb2 {
 
 enum { UNIT_EXP = 0, UNIT_LOG, UNIT_POW, UNIT_LGAMMA, UNIT_GAMMA_P, UNIT_CORR_LWC, UNIT_CALC_SNOW_STATE, UNIT_KIRCHNER_STEP,
-       // the forms the production kernels use: branch-free exp/log/pow, the in-place snow state, the warp-synchronous Kirchner step
-       UNIT_EXP_FLAT, UNIT_LOG_FLAT, UNIT_POW_FLAT, UNIT_CALC_SNOW_STATE_HOT, UNIT_KIRCHNER_STEP_WARP, UNIT_GAMMA_P_PAIR,
+       // the forms the production kernels use: branch-free exp/log/pow, the warp-synchronous Kirchner step
+       UNIT_EXP_FLAT, UNIT_LOG_FLAT, UNIT_POW_FLAT, UNIT_KIRCHNER_STEP_WARP,
        // a / d through the reciprocal of a step-invariant divisor (div_by) and as the IEEE division; the Kirchner step with the host-evaluated dt * tableau
        UNIT_DIV_BY, UNIT_KIRCHNER_STEP_WARP_UDT,
-       // corr_lwc searched warp-cooperatively (gs_corr_lwc_warp): in z1 a1 b1 a2 b2 need(0/1) -> z
-       UNIT_CORR_LWC_WARP,
        // skaugen::calculator::step: in par8 (alpha_0 d_range unit_size max_water_fraction tx cx ts cfr), state7, dt_hours, temp, prec -> state7, outflow, sca, swe, bad
        // skaugen::statistics::sca_rel_red: in u n nu_a alpha -> value, bad
        UNIT_SKAUGEN_STEP, UNIT_SCA_REL_RED,
@@ -55,23 +53,10 @@ __global__ void unit_eval_kernel(int fn, int64_t n, const double* __restrict__ i
         case UNIT_EXP_FLAT: o[0] = sb_exp_flat<true>(a[0]); break;
         case UNIT_LOG_FLAT: o[0] = sb_log_flat<true>(a[0]); break;
         case UNIT_POW_FLAT: o[0] = sb_pow_flat<true>(a[0], a[1]); break;
-        case UNIT_CALC_SNOW_STATE_HOT: {
-            double lg_key = nan_(), lg_val = 0.0;
-            gs_calc_snow_state_hot(a[0], a[1], a[2], a[3], a[4], make_inv_divisor(a[5]), a[6], o[0], o[1], lg_key, lg_val);
-            break;
-        }
         case UNIT_KIRCHNER_STEP_WARP: {
             double q = a[4], q_avg = 0.0;
             const bool ok = kirchner_step_warp<false>(UnitDtb{}, a[0], a[1], a[2], a[3], q, q_avg, a[5], a[6]);
             o[0] = q; o[1] = q_avg; o[2] = ok ? 1.0 : 0.0;
-            break;
-        }
-        case UNIT_GAMMA_P_PAIR: {  // in: a1, x1, a2, x2 -> P(a1,x1), P(a2,x2) advanced together
-            const double pre1 = sb_exp_flat(a[0] * sb_log_flat(a[1]) - a[1] - sb_lgamma(a[0]));
-            const double pre2 = sb_exp_flat(a[2] * sb_log_flat(a[3]) - a[3] - sb_lgamma(a[2]));
-            double P1 = 0.0, P2 = 0.0;
-            gamma_p_pair_inl(a[0], a[1], a[1] > 0.0, pre1, a[2], a[3], a[3] > 0.0, pre2, P1, P2);
-            o[0] = P1; o[1] = P2;
             break;
         }
         case UNIT_DIV_BY: o[0] = div_by(a[0], make_inv_divisor(a[1])); o[1] = a[0] / a[1]; break;
@@ -81,7 +66,6 @@ __global__ void unit_eval_kernel(int fn, int64_t n, const double* __restrict__ i
             o[0] = q; o[1] = q_avg; o[2] = ok ? 1.0 : 0.0;
             break;
         }
-        case UNIT_CORR_LWC_WARP: o[0] = gs_corr_lwc_warp(in_range && a[5] != 0.0, a[0], a[1], a[2], a[3], a[4]); break;  // fn is launch-uniform: all lanes call
         case UNIT_SKAUGEN_STEP: {
             SskParam p{};
             p.alpha_0 = a[0]; p.d_range = a[1]; p.unit_size = a[2]; p.max_water_fraction = a[3]; p.tx = a[4]; p.cx = a[5]; p.ts = a[6]; p.cfr = a[7];

@@ -79,7 +79,7 @@ BTK_RTOL = 1e-12
 
 
 # ---- the dispatch, mirrored ------------------------------------------------------------------------------------------------------
-DENSE_TILE_COMPACT, DENSE_TILE_BTK = 32, 0   # the defaults of SB2_DENSE_TILE_COMPACT and SB2_DENSE_TILE_BTK in sb2_capi.cu
+DENSE_TILE_COMPACT, DENSE_TILE_BTK = 32, 0   # steps staged per buffer: SB2_DENSE_TILE_COMPACT in sb2_capi.cu; kriging 0 = dense_tile_steps' default
 
 
 def _dmma(ks, nt, mode, compact, krow, ts):
