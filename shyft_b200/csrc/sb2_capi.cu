@@ -1169,23 +1169,30 @@ double evaluate_goal_single(sb2_model* m) {
     return combine_goal(m, partial.data());
 }
 
-// ensemble of region-parameter sets for pt_gs_k: member e = one grid layer of the phase pipeline, stepping its own copy of the state
-void goal_batch_ptgsk(sb2_model* m, int64_t n_sets, const double* P, double* goals) {
+// ensemble of region-parameter sets for pt_gs_k, pt_hs_k and hbv_stack: member e = one grid layer of the step kernels run_cells
+// launches, stepping its own copy of the state; the model's parameters, state and catchment series are left as they are
+void goal_batch(sb2_model* m, int64_t n_sets, const double* P, double* goals) {
     sync_parameters(m);
     sync_filter(m);
+    const bool gsk = m->stack == SB2_PT_GS_K;
     const int64_t n = m->n, T = m->T, nc = m->n_catch();
     const size_t state_sz = size_t(m->n_state) * n;
     // members per pass from a ~12 GB budget: state + catchment series (discharge, charge)
     const size_t per_member = state_sz * 8 + size_t(T) * nc * 16;
     const int64_t E = std::max<int64_t>(1, std::min<int64_t>(std::min<int64_t>(n_sets, 65535), int64_t((12ULL << 30) / per_member)));
-    // steps per pass: ~1 GB of per-slot partial sums and ~4 GB of phase-pipeline scratch (five [E][ps][n] arrays)
-    const int64_t ps = std::max<int64_t>(1, std::min<int64_t>(std::min<int64_t>(T, int64_t((1ULL << 30) / (size_t(E) * m->n_slots * 16))),
-                                                               std::max<int64_t>(8, int64_t((4ULL << 30) / (size_t(E) * n * 40)))));
+    // steps per pass: ~1 GB of per-slot partial sums; pt_gs_k also ~4 GB of phase-pipeline scratch (five [E][ps][n] arrays)
+    int64_t ps = std::min<int64_t>(T, int64_t((1ULL << 30) / (size_t(E) * m->n_slots * 16)));
+    if (gsk) ps = std::min<int64_t>(ps, std::max<int64_t>(8, int64_t((4ULL << 30) / (size_t(E) * n * 40))));
+    ps = std::max<int64_t>(1, ps);
     DevArray<double> d_state, d_partial, d_cq, d_cc, d_out, d_scr[5];
-    for (auto& b : d_scr) b.resize(size_t(E) * ps * n);
-    DevArray<int> d_tickets;  // [E] ticket counters, then [E][cell groups] finished slices (response kernel time split)
-    d_tickets.resize(size_t(E) * (1 + std::max(grid_for(n, SB2_BLOCK_B), grid_for(n, SB2_BLOCK_C))));
+    if (gsk)
+        for (auto& b : d_scr) b.resize(size_t(E) * ps * n);
+    // [E] ticket counters, then [E][cell groups] finished slices (time split of the snow / response or HBV step kernels)
+    const int groups = gsk ? std::max(grid_for(n, SB2_BLOCK_B), grid_for(n, SB2_BLOCK_C)) : grid_for(n, SB2_BLOCK);
+    DevArray<int> d_tickets;
+    d_tickets.resize(size_t(E) * (1 + groups));
     DevArray<PtgskParam> d_par;
+    DevArray<HbvParam> d_hbv_par;
     DevArray<GoalTarget> d_gt;
     d_state.resize(size_t(E) * state_sz);
     d_partial.resize(size_t(E) * ps * m->n_slots * 2);
@@ -1199,43 +1206,74 @@ void goal_batch_ptgsk(sb2_model* m, int64_t n_sets, const double* P, double* goa
     std::vector<double> partial(size_t(E) * gt.size());
     for (int64_t e0 = 0; e0 < n_sets; e0 += E) {
         const int64_t ne = std::min<int64_t>(E, n_sets - e0);
-        std::vector<PtgskParam> tab;
-        for (int64_t e = 0; e < ne; ++e) tab.push_back(make_ptgsk_param(P + (e0 + e) * m->n_param, m->dt));
-        d_par.upload(tab, m->stream);
+        if (gsk) {
+            std::vector<PtgskParam> tab;
+            for (int64_t e = 0; e < ne; ++e) tab.push_back(make_ptgsk_param(P + (e0 + e) * m->n_param, m->dt));
+            d_par.upload(tab, m->stream);
+        } else {  // the table sync_parameters builds for the region set, so every derived divisor is the single evaluation's
+            std::vector<HbvParam> tab;
+            for (int64_t e = 0; e < ne; ++e) tab.push_back(make_hbv_param(m->stack == SB2_HBV_STACK, P + (e0 + e) * m->n_param));
+            d_hbv_par.upload(tab, m->stream);
+        }
         for (int64_t e = 0; e < ne; ++e)  // reset_states(): every member starts from the initial state (:833)
             CUDA_OK(cudaMemcpyAsync(d_state.p + e * state_sz, m->d_initial_state.p, state_sz * sizeof(double), cudaMemcpyDeviceToDevice, m->stream));
         for (int64_t done = 0; done < T; done += ps) {
             const int chunk = int(std::min<int64_t>(ps, T - done));
-            PtgskRunArgs a{};
-            a.n_cells = n;
-            a.z = m->d_z.p; a.area = m->d_area.p; a.glacier = m->d_glacier.p; a.lake = m->d_lake.p; a.reservoir = m->d_reservoir.p;
-            a.forest = m->d_forest.p; a.pset = m->d_pset.p; a.active = m->d_active.p; a.params = m->d_ptgsk_params.p;
-            a.state = d_state.p;
-            for (int v = 0; v < 5; ++v) a.f[v] = m->d_forcing[v].p + done * n;
-            a.n_steps = chunk; a.first_step = done;
-            a.dt_seconds = dt_seconds; a.dt_hours = dt_seconds / 3600.0; a.dt_us = double(m->dt);
-            a.bb0 = 0.98 * 5.670373e-8 * sb_pow4(273.15);
-            fill_step_constants(m, a);
-            a.day_sec_of_year = m->d_doy_soy.p;
-            a.out_first_step = 0; a.collect_end_state = 0;
-            a.slot = m->d_slot.p; a.partial = d_partial.p; a.n_slots = m->n_slots; a.error_flag = m->d_error_flag.p;
-            a.ens_params = d_par.p; a.ens_state_stride = int64_t(state_sz); a.ens_partial_stride = ps * m->n_slots * 2;
-            for (int k = 0; k < 5; ++k) a.scr[k] = d_scr[k].p;
-            a.ens_scr_stride = ps * n;
-            // the same phase pipeline as run_cells, one grid layer per member
-            ptgsk_forcing_terms_kernel<false><<<dim3((unsigned)grid_for(n, SB2_BLOCK_A), (unsigned)grid_for(chunk, SB2_STEPS_A), (unsigned)ne), SB2_BLOCK_A,
-                                                SB2_MTAB_BYTES, m->stream>>>(a);
-            {
-                const int gb = grid_for(n, SB2_BLOCK_B), gc = grid_for(n, SB2_BLOCK_C);
-                const bool split = use_time_split(int64_t(gb) * ne);
-                const int n_slices = split ? grid_for(chunk, SB2_UNIT_STEPS) : 1;
-                a.unit_steps = split ? SB2_UNIT_STEPS : 0; a.tickets = d_tickets.p; a.progress = d_tickets.p + E;
-                CUDA_OK(cudaMemsetAsync(d_tickets.p, 0, d_tickets.n * sizeof(int), m->stream));
-                ptgsk_snow_kernel<0, false><<<dim3((unsigned)(gb * n_slices), (unsigned)ne), SB2_BLOCK_B, SB2_MTAB_BYTES, m->stream>>>(a);
-                CUDA_OK(cudaMemsetAsync(d_tickets.p, 0, d_tickets.n * sizeof(int), m->stream));
-                ptgsk_response_kernel<0, false><<<dim3((unsigned)(gc * n_slices), (unsigned)ne), SB2_BLOCK_C, SB2_MTAB_BYTES, m->stream>>>(a);
+            if (gsk) {
+                PtgskRunArgs a{};
+                a.n_cells = n;
+                a.z = m->d_z.p; a.area = m->d_area.p; a.glacier = m->d_glacier.p; a.lake = m->d_lake.p; a.reservoir = m->d_reservoir.p;
+                a.forest = m->d_forest.p; a.pset = m->d_pset.p; a.active = m->d_active.p; a.params = m->d_ptgsk_params.p;
+                a.state = d_state.p;
+                for (int v = 0; v < 5; ++v) a.f[v] = m->d_forcing[v].p + done * n;
+                a.n_steps = chunk; a.first_step = done;
+                a.dt_seconds = dt_seconds; a.dt_hours = dt_seconds / 3600.0; a.dt_us = double(m->dt);
+                a.bb0 = 0.98 * 5.670373e-8 * sb_pow4(273.15);
+                fill_step_constants(m, a);
+                a.day_sec_of_year = m->d_doy_soy.p;
+                a.out_first_step = 0; a.collect_end_state = 0;
+                a.slot = m->d_slot.p; a.partial = d_partial.p; a.n_slots = m->n_slots; a.error_flag = m->d_error_flag.p;
+                a.ens_params = d_par.p; a.ens_state_stride = int64_t(state_sz); a.ens_partial_stride = ps * m->n_slots * 2;
+                for (int k = 0; k < 5; ++k) a.scr[k] = d_scr[k].p;
+                a.ens_scr_stride = ps * n;
+                // the same phase pipeline as run_cells, one grid layer per member
+                ptgsk_forcing_terms_kernel<false><<<dim3((unsigned)grid_for(n, SB2_BLOCK_A), (unsigned)grid_for(chunk, SB2_STEPS_A), (unsigned)ne), SB2_BLOCK_A,
+                                                    SB2_MTAB_BYTES, m->stream>>>(a);
+                {
+                    const int gb = grid_for(n, SB2_BLOCK_B), gc = grid_for(n, SB2_BLOCK_C);
+                    const bool split = use_time_split(int64_t(gb) * ne);
+                    const int n_slices = split ? grid_for(chunk, SB2_UNIT_STEPS) : 1;
+                    a.unit_steps = split ? SB2_UNIT_STEPS : 0; a.tickets = d_tickets.p; a.progress = d_tickets.p + E;
+                    CUDA_OK(cudaMemsetAsync(d_tickets.p, 0, d_tickets.n * sizeof(int), m->stream));
+                    ptgsk_snow_kernel<0, false><<<dim3((unsigned)(gb * n_slices), (unsigned)ne), SB2_BLOCK_B, SB2_MTAB_BYTES, m->stream>>>(a);
+                    CUDA_OK(cudaMemsetAsync(d_tickets.p, 0, d_tickets.n * sizeof(int), m->stream));
+                    ptgsk_response_kernel<0, false><<<dim3((unsigned)(gc * n_slices), (unsigned)ne), SB2_BLOCK_C, SB2_MTAB_BYTES, m->stream>>>(a);
+                }
+                m->launches += 2;
+            } else {
+                HbvRunArgs a{};
+                a.n_cells = n;
+                a.area = m->d_area.p; a.glacier = m->d_glacier.p; a.lake = m->d_lake.p; a.reservoir = m->d_reservoir.p;
+                a.pset = m->d_pset.p; a.active = m->d_active.p; a.params = m->d_hbv_params.p; a.state = d_state.p;
+                for (int v = 0; v < 5; ++v) a.f[v] = m->d_forcing[v].p + done * n;
+                a.n_steps = chunk; a.first_step = done;
+                a.dt_seconds = dt_seconds; a.dt_hours = dt_seconds / 3600.0; a.dt_us = double(m->dt);
+                fill_dopri_products(a.dt_hours, a.dtb);
+                a.inv_dt_hours = make_inv_divisor(a.dt_hours);
+                a.step_in_days = dt_seconds / 86400.0;
+                a.out_first_step = 0; a.collect_end_state = 0; a.collect = 0;
+                a.slot = m->d_slot.p; a.partial = d_partial.p; a.n_slots = m->n_slots; a.error_flag = m->d_error_flag.p;
+                a.ens_params = d_hbv_par.p; a.ens_state_stride = int64_t(state_sz); a.ens_partial_stride = ps * m->n_slots * 2;
+                // the kernel run_cells launches, one grid layer per member; time slices while the launch is only a few waves
+                const int g = grid_for(n, SB2_BLOCK);
+                const bool split = use_time_split(int64_t(g) * ne);
+                const int n_slices = split ? grid_for(chunk, SB2_HBV_UNIT_STEPS) : 1;
+                a.unit_steps = split ? SB2_HBV_UNIT_STEPS : 0; a.tickets = d_tickets.p; a.progress = d_tickets.p + E;
+                if (split) CUDA_OK(cudaMemsetAsync(d_tickets.p, 0, d_tickets.n * sizeof(int), m->stream));
+                const dim3 grid((unsigned)(g * n_slices), (unsigned)ne);
+                if (m->stack == SB2_PT_HS_K) hbv_run_kernel<false, false><<<grid, SB2_BLOCK, SB2_MTAB_BYTES, m->stream>>>(a);
+                else hbv_run_kernel<true, false><<<grid, SB2_BLOCK, SB2_MTAB_BYTES, m->stream>>>(a);
             }
-            m->launches += 2;
             CUDA_OK(cudaGetLastError());
             const int64_t total = int64_t(chunk) * nc;
             catchment_reduce_kernel<<<dim3((unsigned)grid_for(total, 256), (unsigned)ne), 256, 0, m->stream>>>(
@@ -2379,14 +2417,14 @@ int sb2_calculate_goal_function_batch(sb2_model* m, int64_t n_sets, const double
     return guarded(m, [&] {
         if (m->targets.empty()) throw Error("no target specification set");
         if (n_sets <= 0) return;
-        bool device_batch = m->stack == SB2_PT_GS_K;
+        bool device_batch = m->stack == SB2_PT_GS_K || m->stack == SB2_PT_HS_K || m->stack == SB2_HBV_STACK;
         for (auto& t : m->targets)
             if ((t->property != SB2_TARGET_DISCHARGE && t->property != SB2_TARGET_CELL_CHARGE) || !t->aligned) device_batch = false;
         if (device_batch) {
             if (!m->has_initial) throw Error("Initial state not yet established or set");
             if (!m->d_forcing[0].p || m->forcing_first != 0 || m->forcing_rows != m->T)
                 throw Error("run_cells: cell environment is not resident for the whole time axis (use interpolate / set_cell_forcing, or run_windowed)");
-            goal_batch_ptgsk(m, n_sets, P, goals);
+            goal_batch(m, n_sets, P, goals);
         } else {  // one member at a time through the single-evaluation entry
             for (int64_t e = 0; e < n_sets; ++e)
                 if (sb2_calculate_goal_function(m, P + e * m->n_param, m->n_param, goals + e) != 0) throw Error(m->err);

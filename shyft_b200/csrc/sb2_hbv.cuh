@@ -102,6 +102,11 @@ struct HbvRunArgs {
     int unit_steps;              // > 0: the chunk is stepped in time slices of this many steps handed out by ticket (as ptgsk_response_kernel)
     int* __restrict__ tickets;   // [1] ticket counter, zeroed per launch
     int* __restrict__ progress;  // [cell groups] finished slices per group, zeroed per launch
+    // parameter-set ensemble (calibration): blockIdx.y = member; member e steps its own state / partial sums with the region
+    // parameter replaced by ens_params[e] (cells with a catchment override keep it, model_calibration.h:830-832); tickets are
+    // [members] and progress [members][cell groups].  Last in the struct so that the fields above keep their constant-bank offsets.
+    const HbvParam* __restrict__ ens_params;  // null = no ensemble
+    int64_t ens_state_stride, ens_partial_stride;
 };
 
 // hbv_snow_common::integrate(f, x, n, a = x[0], b, f_b_is_zero), core/hbv_snow_common.h:14-43
@@ -248,11 +253,12 @@ __device__ __forceinline__ bool hbv_snow_step(double (&sp)[HBV_NB], double (&sw)
 // 47.2 at 80.
 #define SB2_HBV_MINBLOCKS_K 4   // pt_hs_k (Kirchner)
 #define SB2_HBV_MINBLOCKS_S 5   // hbv_stack (soil + tank)
-// UPAR: no catchment override in use -- every cell reads the region parameter set (a.par0) from the kernel's constant bank
+// UPAR: no catchment override in use and no ensemble -- every cell reads the region parameter set (a.par0) from the kernel's constant bank
 template <bool HBV_STACK, bool UPAR>
 __global__ void __launch_bounds__(128, (HBV_STACK ? SB2_HBV_MINBLOCKS_S : SB2_HBV_MINBLOCKS_K)) hbv_run_kernel(const __grid_constant__ HbvRunArgs a) {
     constexpr int NS = HBV_STACK ? 5 + 2 * HBV_NB : 3 + 2 * HBV_NB;
     sb_math_stage_tables();  // exp / log tables of the shared math spec into this block's shared memory (sb2_math.cuh)
+    const int ens = UPAR ? 0 : blockIdx.y;  // UPAR launches have no ensemble: the member offsets fold away
     // Time split by ticket (see ptgsk_response_kernel): 12 500 one-warp blocks of a 400 000-cell shard are 4-5 waves of the 2 400-3 000
     // resident ones, so whole-chunk blocks leave a ragged last wave; slices of unit_steps steps shrink that tail to one slice.  A block
     // waits until the previous slice of its cell group has published the state; tickets are handed out in start order, so that slice
@@ -263,13 +269,13 @@ __global__ void __launch_bounds__(128, (HBV_STACK ? SB2_HBV_MINBLOCKS_S : SB2_HB
     if (a.unit_steps > 0) {
         __shared__ int s_ticket;
         const int n_groups = int((a.n_cells + blockDim.x - 1) / blockDim.x);
-        if (threadIdx.x == 0) s_ticket = atomicAdd(a.tickets, 1);
+        if (threadIdx.x == 0) s_ticket = atomicAdd(a.tickets + ens, 1);
         __syncthreads();
         slice = s_ticket / n_groups;
         group = s_ticket - slice * n_groups;
         i_begin = slice * a.unit_steps;
         i_end = min(a.n_steps, i_begin + a.unit_steps);
-        progress = a.progress + group;
+        progress = a.progress + (int64_t)ens * n_groups + group;
         if (threadIdx.x == 0) {
             while (*((volatile int*)progress) < slice) __nanosleep(256);
             __threadfence();
@@ -283,7 +289,7 @@ __global__ void __launch_bounds__(128, (HBV_STACK ? SB2_HBV_MINBLOCKS_S : SB2_HB
     const unsigned lane = threadIdx.x & 31u;
     const int64_t n = a.n_cells;
 
-    const HbvParam& p = UPAR ? a.par0 : a.params[a.pset[cc]];
+    const HbvParam& p = UPAR ? a.par0 : ((a.ens_params != nullptr && a.pset[cc] == 0) ? a.ens_params[ens] : a.params[a.pset[cc]]);
     const double cell_area_m2 = a.area[cc], glacier_fraction = a.glacier[cc], lake = a.lake[cc], reservoir = a.reservoir[cc];
     const double gm_direct = p.gm_direct_response;
     const double gm_routed = 1 - gm_direct;
@@ -294,13 +300,15 @@ __global__ void __launch_bounds__(128, (HBV_STACK ? SB2_HBV_MINBLOCKS_S : SB2_HB
     const double glacier_area_m2 = cell_area_m2 * glacier_fraction;
 
     // __ldcg: the state may have been written by the previous time slice on another SM a moment ago -- read it from L2
-    double swe = __ldcg(a.state + 0 * n + cc), sca = __ldcg(a.state + 1 * n + cc);
+    // this member's state rows start at a.state + so, its partial sums at a.partial + ens * a.ens_partial_stride (both 0 without an ensemble)
+    const int64_t so = (int64_t)ens * a.ens_state_stride;
+    double swe = __ldcg(a.state + so + 0 * n + cc), sca = __ldcg(a.state + so + 1 * n + cc);
     double sp[HBV_NB], sw[HBV_NB];
 #pragma unroll
-    for (int i = 0; i < HBV_NB; ++i) { sp[i] = __ldcg(a.state + (2 + i) * n + cc); sw[i] = __ldcg(a.state + (2 + HBV_NB + i) * n + cc); }
-    double x0 = __ldcg(a.state + (2 + 2 * HBV_NB) * n + cc);                      // kirchner.q | soil.sm
-    double x1 = HBV_STACK ? __ldcg(a.state + (3 + 2 * HBV_NB) * n + cc) : 0.0;    // tank.uz
-    double x2 = HBV_STACK ? __ldcg(a.state + (4 + 2 * HBV_NB) * n + cc) : 0.0;    // tank.lz
+    for (int i = 0; i < HBV_NB; ++i) { sp[i] = __ldcg(a.state + so + (2 + i) * n + cc); sw[i] = __ldcg(a.state + so + (2 + HBV_NB + i) * n + cc); }
+    double x0 = __ldcg(a.state + so + (2 + 2 * HBV_NB) * n + cc);                      // kirchner.q | soil.sm
+    double x1 = HBV_STACK ? __ldcg(a.state + so + (3 + 2 * HBV_NB) * n + cc) : 0.0;    // tank.uz
+    double x2 = HBV_STACK ? __ldcg(a.state + so + (4 + 2 * HBV_NB) * n + cc) : 0.0;    // tank.lz
 
     int my_slot = -1;
     bool head = false;
@@ -325,7 +333,7 @@ __global__ void __launch_bounds__(128, (HBV_STACK ? SB2_HBV_MINBLOCKS_S : SB2_HB
     // the step consumes one 8-byte value per array, so without it every step waits for DRAM
     int64_t o = (int64_t)i_begin * n + cc;  // running element offset of (step i, cell), bumped by n per step (see ptgsk_snow_kernel)
     const int64_t out_shift = (a.first_step - a.out_first_step) * n;
-    int64_t po = ((int64_t)i_begin * a.n_slots + (my_slot < 0 ? 0 : my_slot)) * 2;  // likewise into partial[step][slot][2]
+    int64_t po = (int64_t)ens * a.ens_partial_stride + ((int64_t)i_begin * a.n_slots + (my_slot < 0 ? 0 : my_slot)) * 2;  // likewise into partial[step][slot][2]
     double f_t = a.f[0][o], f_p = a.f[1][o], f_r = a.f[2][o], f_h = a.f[4][o];
     for (int i = i_begin; i < i_end; ++i, o += n) {
         const double temp = f_t, rad = f_r, rel_hum = f_h, prec_raw = f_p;
@@ -425,11 +433,11 @@ __global__ void __launch_bounds__(128, (HBV_STACK ? SB2_HBV_MINBLOCKS_S : SB2_HB
     }
     if (active) {
         if ((a.collect & 8) && a.collect_end_state && i_end == a.n_steps) collect_state((a.first_step + a.n_steps - a.out_first_step) * n + cc);
-        a.state[0 * n + cc] = swe; a.state[1 * n + cc] = sca;
+        a.state[so + 0 * n + cc] = swe; a.state[so + 1 * n + cc] = sca;
 #pragma unroll
-        for (int i = 0; i < HBV_NB; ++i) { a.state[(2 + i) * n + cc] = sp[i]; a.state[(2 + HBV_NB + i) * n + cc] = sw[i]; }
-        a.state[(2 + 2 * HBV_NB) * n + cc] = x0;
-        if (HBV_STACK) { a.state[(3 + 2 * HBV_NB) * n + cc] = x1; a.state[(4 + 2 * HBV_NB) * n + cc] = x2; }
+        for (int i = 0; i < HBV_NB; ++i) { a.state[so + (2 + i) * n + cc] = sp[i]; a.state[so + (2 + HBV_NB + i) * n + cc] = sw[i]; }
+        a.state[so + (2 + 2 * HBV_NB) * n + cc] = x0;
+        if (HBV_STACK) { a.state[so + (3 + 2 * HBV_NB) * n + cc] = x1; a.state[so + (4 + 2 * HBV_NB) * n + cc] = x2; }
         if (failed_snow) atomicOr(a.error_flag, ERR_HBV_NEGATIVE_OUTFLOW);
         if (failed_k) atomicOr(a.error_flag, ERR_KIRCHNER_STEP);
         (void)NS;

@@ -2,6 +2,7 @@
 minutes; prints one JSON line per config.  Usage: python tools/bench_configs.py [3] [5]"""
 import json
 import os
+import subprocess
 import sys
 import time
 
@@ -15,6 +16,8 @@ from shyft_b200 import synthetic
 
 PTGSK = [-2.439, 0.966, -0.10, 1.5, -0.5, 2.0, 0.1, 1.0, 5.0, 5.0, 30.0, 0.9, 0.6, 5.0, 0.4, 0.4, 1.0, 0.0, 0.0, 0.2, 1.26, 0.04, 100.0, 0.0, 6.0, 1.0, 7.0, 0.0,
          221.0, 0.0, 1.0]
+PTHSK = [-2.439, 0.966, -0.10, 1.5, 0.1, 0.0, 1.0, 0.0, 0.5, 6.0, 1.0, 0.2, 1.26, 1.0, 7.0, 0.0, 0.0, 1.0]
+HBV = [300.0, 2.0, 150.0, 25.0, 0.5, 0.3, 0.8, 0.02, 0.1, 0.0, 1.0, 0.0, 0.5, 1.0, 0.2, 1.26, 6.0, 1.0, 7.0, 0.0, 0.0, 1.0]
 which = [int(a) for a in sys.argv[1:]] or [3, 5]
 
 
@@ -65,19 +68,32 @@ if 5 in which:  # calibration ensemble: parameter sets x 10k-cell catchment x 3 
     if world > 1:
         torch.cuda.set_device(local_rank)
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
+    # SB2_C5_STACK: pt_gs_k (default), pt_hs_k or hbv_stack -- the stacks whose batch runs as grid layers on the device
+    stack = os.environ.get("SB2_C5_STACK", "pt_gs_k")
     n, T, sets = 10000, 26280, int(os.environ.get("SB2_C5_SETS", "256"))
     geo, ta, env = synthetic.make_region(n, T, 64, config_index=4)
-    m = sb.PTGSKOptModel(geo, PTGSK, device=local_rank)
+    cls, par, sid = {"pt_gs_k": (sb.PTGSKOptModel, PTGSK, 0), "pt_hs_k": (sb.PTHSKOptModel, PTHSK, 1), "hbv_stack": (sb.HbvStackOptModel, HBV, 2)}[stack]
+    m = cls(geo, par, device=local_rank)
     m.run_interpolation(sb.InterpolationParameter(), ta, env)
-    m.set_states(synthetic.default_state(0, n))
+    m.set_states(synthetic.default_state(sid, n))
     m.run_cells()
     obs = m.catchment_discharges().sum(axis=1).reshape(-1, 24).mean(axis=1)
     opt = sb.Optimizer(m, [sb.TargetSpecification(obs, ta.start, 86400, list(range(1, 11)), 1.0, 0)])
     rng = np.random.default_rng(5)
-    P = np.tile(PTGSK, (sets, 1))
-    P[:, 0] = rng.uniform(-3.0, -1.9, sets); P[:, 1] = rng.uniform(0.8, 0.99, sets); P[:, 2] = rng.uniform(-0.15, -0.05, sets)
-    P[:, 3] = rng.uniform(0.5, 2.5, sets); P[:, 4] = rng.uniform(-2, 2, sets); P[:, 5] = rng.uniform(1, 4, sets)
-    P[:, 14] = rng.uniform(0.2, 0.8, sets); P[:, 16] = rng.uniform(0.8, 1.4, sets)
+    P = np.tile(par, (sets, 1))
+    if stack == "pt_gs_k":
+        P[:, 0] = rng.uniform(-3.0, -1.9, sets); P[:, 1] = rng.uniform(0.8, 0.99, sets); P[:, 2] = rng.uniform(-0.15, -0.05, sets)
+        P[:, 3] = rng.uniform(0.5, 2.5, sets); P[:, 4] = rng.uniform(-2, 2, sets); P[:, 5] = rng.uniform(1, 4, sets)
+        P[:, 14] = rng.uniform(0.2, 0.8, sets); P[:, 16] = rng.uniform(0.8, 1.4, sets)
+    elif stack == "pt_hs_k":   # c1, c2, c3, ae_scale, tx, cx, p_corr
+        P[:, 0] = rng.uniform(-3.0, -1.9, sets); P[:, 1] = rng.uniform(0.8, 0.99, sets); P[:, 2] = rng.uniform(-0.15, -0.05, sets)
+        P[:, 3] = rng.uniform(0.5, 2.5, sets); P[:, 5] = rng.uniform(-2, 2, sets); P[:, 6] = rng.uniform(0.5, 2.0, sets)
+        P[:, 10] = rng.uniform(0.8, 1.4, sets)
+    else:                      # fc, beta, lp, uz1, kuz2, kuz1, perc, klz, tx, p_corr
+        P[:, 0] = rng.uniform(150, 450, sets); P[:, 1] = rng.uniform(1, 4, sets); P[:, 2] = rng.uniform(100, 200, sets)
+        P[:, 3] = rng.uniform(10, 40, sets); P[:, 4] = rng.uniform(0.2, 0.7, sets); P[:, 5] = rng.uniform(0.1, 0.4, sets)
+        P[:, 6] = rng.uniform(0.4, 1.2, sets); P[:, 7] = rng.uniform(0.01, 0.05, sets); P[:, 9] = rng.uniform(-2, 2, sets)
+        P[:, 13] = rng.uniform(0.8, 1.4, sets)
     b, e = sharding.partition_parameter_sets(sets, world, rank)
     if world > 1:
         dist.barrier()
@@ -96,7 +112,9 @@ if 5 in which:  # calibration ensemble: parameter sets x 10k-cell catchment x 3 
     t0 = time.perf_counter()
     g1 = np.array([opt.calculate_goal_function(p) for p in P[:8]])
     s1 = (time.perf_counter() - t0) / 8
-    print(json.dumps({"config": 5, "n_gpus": world, "sets": sets, "cells": n, "steps": T, "batch_seconds": s, "cell_steps_per_s": sets * n * T / s,
+    gpu = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", str(local_rank)], capture_output=True,
+                         text=True).stdout.strip()
+    print(json.dumps({"config": 5, **({} if stack == "pt_gs_k" else {"stack": stack, "gpu": gpu}), "n_gpus": world, "sets": sets, "cells": n, "steps": T, "batch_seconds": s, "cell_steps_per_s": sets * n * T / s,
                       "one_at_a_time_seconds_per_set": s1, "cell_steps_per_s_one_at_a_time": n * T / s1, "batch_equals_single": bool(np.array_equal(g[:8], g1)),
                       "best_goal": float(g.min()), "extrapolated_4096_sets_seconds": s * 4096 / sets}))
     if world > 1:
