@@ -528,6 +528,7 @@ struct StepTarget {
     int members = 1;
     const PtgskParam* ptgsk_members = nullptr;  // the members' parameter sets, in place of the region set (null: no batch)
     const HbvParam* hbv_members = nullptr;
+    const HpsParam* hps_members = nullptr;
     double* state = nullptr;
     double* partial = nullptr;
     double *cq = nullptr, *cc = nullptr;  // catchment sums [T][n_catch]
@@ -544,7 +545,7 @@ void launch_step_chunk(sb2_model* m, const StepTarget& t, int64_t s0, int chunk,
     const bool gsk = m->stack == SB2_PT_GS_K;
     const int collect = t.series ? m->collect_bits : 0;
     // UPAR kernels: no catchment override and no member table -> every cell reads the region parameter set from the constant bank
-    const bool upar = m->catch_param.empty() && !t.ptgsk_members && !t.hbv_members;
+    const bool upar = m->catch_param.empty() && !t.ptgsk_members && !t.hbv_members && !t.hps_members;
     // snow / response or run kernel in time slices handed out by ticket (see the kernels); the tickets are read only when split
     const int groups = step_groups(m);
     const bool split = use_time_split(int64_t(groups) * t.members);
@@ -627,8 +628,10 @@ void launch_step_chunk(sb2_model* m, const StepTarget& t, int64_t s0, int chunk,
             a.params = m->d_hps_params.p;
             a.bb0 = 0.98 * 5.670373e-8 * sb_pow4(273.15);  // calculator::BB0 (hbv_physical_snow.h:208)
             a.inv_dt_seconds = make_inv_divisor(a.dt_seconds);
+            a.ens_params = t.hps_members; a.ens_state_stride = t.state_stride; a.ens_partial_stride = t.partial_stride;
             a.collect = collect & 15;
-            pthpsk_run_kernel<<<grid, SB2_BLOCK, SB2_MTAB_BYTES, m->stream>>>(a);
+            if (t.hps_members) pthpsk_run_kernel<true><<<grid, SB2_BLOCK, SB2_MTAB_BYTES, m->stream>>>(a);
+            else pthpsk_run_kernel<false><<<grid, SB2_BLOCK, SB2_MTAB_BYTES, m->stream>>>(a);
         } else {
             HbvRunArgs a{};
             common(a);
@@ -1180,8 +1183,8 @@ double evaluate_goal_single(sb2_model* m) {
     return combine_goal(m, partial.data());
 }
 
-// ensemble of region-parameter sets for pt_gs_k, pt_hs_k and hbv_stack: member e = one grid layer of the step kernels run_cells
-// launches, stepping its own copy of the state; the model's parameters, state and catchment series are left as they are
+// ensemble of region-parameter sets for pt_gs_k, pt_hs_k, hbv_stack and pt_hps_k: member e = one grid layer of the step kernels
+// run_cells launches, stepping its own copy of the state; the model's parameters, state and catchment series are left as they are
 void goal_batch(sb2_model* m, int64_t n_sets, const double* P, double* goals) {
     sync_parameters(m);
     sync_filter(m);
@@ -1202,6 +1205,7 @@ void goal_batch(sb2_model* m, int64_t n_sets, const double* P, double* goals) {
     d_tickets.resize(size_t(E) * (1 + step_groups(m)));
     DevArray<PtgskParam> d_par;
     DevArray<HbvParam> d_hbv_par;
+    DevArray<HpsParam> d_hps_par;
     DevArray<GoalTarget> d_gt;
     d_state.resize(size_t(E) * state_sz);
     d_partial.resize(size_t(E) * ps * m->n_slots * 2);
@@ -1221,6 +1225,7 @@ void goal_batch(sb2_model* m, int64_t n_sets, const double* P, double* goals) {
         std::vector<const double*> sets;
         for (int64_t e = 0; e < ne; ++e) sets.push_back(P + (e0 + e) * m->n_param);
         if (gsk) { upload_params(m, sets, d_par); t.ptgsk_members = d_par.p; }
+        else if (m->stack == SB2_PT_HPS_K) { upload_params(m, sets, d_hps_par); t.hps_members = d_hps_par.p; }
         else { upload_params(m, sets, d_hbv_par); t.hbv_members = d_hbv_par.p; }
         t.members = int(ne);
         for (int64_t e = 0; e < ne; ++e)  // reset_states(): every member starts from the initial state (:833)
@@ -2361,7 +2366,8 @@ int sb2_calculate_goal_function_batch(sb2_model* m, int64_t n_sets, const double
     return guarded(m, [&] {
         if (m->targets.empty()) throw Error("no target specification set");
         if (n_sets <= 0) return;
-        bool device_batch = m->stack == SB2_PT_GS_K || m->stack == SB2_PT_HS_K || m->stack == SB2_HBV_STACK;
+        // pt_ss_k is not among them: its batch goes one set at a time
+        bool device_batch = m->stack == SB2_PT_GS_K || m->stack == SB2_PT_HS_K || m->stack == SB2_HBV_STACK || m->stack == SB2_PT_HPS_K;
         for (auto& t : m->targets)
             if ((t->property != SB2_TARGET_DISCHARGE && t->property != SB2_TARGET_CELL_CHARGE) || !t->aligned) device_batch = false;
         if (device_batch) {

@@ -81,6 +81,12 @@ struct HpsRunArgs {
     int unit_steps;
     int* __restrict__ tickets;
     int* __restrict__ progress;
+    // parameter-set ensemble (calibration, pthpsk_run_kernel<true>): blockIdx.y = member; member e steps its own state / partial sums
+    // with the region parameter replaced by ens_params[e] (cells with a catchment override keep it, model_calibration.h:830-832);
+    // tickets are [members] and progress [members][cell groups].  Last in the struct so that the fields above keep their
+    // constant-bank offsets.
+    const HpsParam* __restrict__ ens_params;  // null = no ensemble
+    int64_t ens_state_stride, ens_partial_stride;
 };
 
 struct HpsState { double sp[HBV_NB], sw[HBV_NB], albedo[HBV_NB], iso[HBV_NB], surface_heat, swe, sca; };
@@ -275,21 +281,25 @@ __device__ __forceinline__ bool hps_step(HpsState& s, double& r_outflow, double&
 }
 
 #define SB2_HPS_MINBLOCKS 4
+// ENS: a calibration batch, one grid layer per member of a.ens_params (the launcher sets the table whenever it launches this
+// instantiation); without it the member is the constant 0 and every member offset folds away (the run_cells kernel)
+template <bool ENS>
 __global__ void __launch_bounds__(128, SB2_HPS_MINBLOCKS) pthpsk_run_kernel(const __grid_constant__ HpsRunArgs a) {
     sb_math_stage_tables();
+    const int ens = ENS ? blockIdx.y : 0;
     int64_t group = blockIdx.x;
     int i_begin = 0, i_end = a.n_steps, slice = 0;
     int* progress = nullptr;
     if (a.unit_steps > 0) {  // time slices handed out by ticket, as hbv_run_kernel
         __shared__ int s_ticket;
         const int n_groups = int((a.n_cells + blockDim.x - 1) / blockDim.x);
-        if (threadIdx.x == 0) s_ticket = atomicAdd(a.tickets, 1);
+        if (threadIdx.x == 0) s_ticket = atomicAdd(a.tickets + ens, 1);
         __syncthreads();
         slice = s_ticket / n_groups;
         group = s_ticket - slice * n_groups;
         i_begin = slice * a.unit_steps;
         i_end = min(a.n_steps, i_begin + a.unit_steps);
-        progress = a.progress + group;
+        progress = a.progress + (int64_t)ens * n_groups + group;
         if (threadIdx.x == 0) {
             while (*((volatile int*)progress) < slice) __nanosleep(256);
             __threadfence();
@@ -302,7 +312,7 @@ __global__ void __launch_bounds__(128, SB2_HPS_MINBLOCKS) pthpsk_run_kernel(cons
     const bool active = in_range && (a.active == nullptr || a.active[cc] != 0);
     const unsigned lane = threadIdx.x & 31u;
     const int64_t n = a.n_cells;
-    const HpsParam& p = a.params[a.pset[cc]];
+    const HpsParam& p = (ENS && a.pset[cc] == 0) ? a.ens_params[ens] : a.params[a.pset[cc]];
     const double cell_area_m2 = a.area[cc], glacier_fraction = a.glacier[cc], lake = a.lake[cc], reservoir = a.reservoir[cc];
     const double gm_direct = p.gm_direct_response;
     const double gm_routed = 1 - gm_direct;
@@ -312,15 +322,17 @@ __global__ void __launch_bounds__(128, SB2_HPS_MINBLOCKS) pthpsk_run_kernel(cons
     const double kirchner_fraction = 1 - direct_response_fraction;
     const double glacier_area_m2 = cell_area_m2 * glacier_fraction;
 
+    // this member's state rows start at a.state + so, its partial sums at a.partial + ens * a.ens_partial_stride (both 0 without an ensemble)
+    const int64_t so = (int64_t)ens * a.ens_state_stride;
     HpsState hs;
 #pragma unroll
     for (int i = 0; i < HBV_NB; ++i) {
-        hs.sp[i] = __ldcg(a.state + i * n + cc); hs.sw[i] = __ldcg(a.state + (HBV_NB + i) * n + cc);
-        hs.albedo[i] = __ldcg(a.state + (2 * HBV_NB + i) * n + cc); hs.iso[i] = __ldcg(a.state + (3 * HBV_NB + i) * n + cc);
+        hs.sp[i] = __ldcg(a.state + so + i * n + cc); hs.sw[i] = __ldcg(a.state + so + (HBV_NB + i) * n + cc);
+        hs.albedo[i] = __ldcg(a.state + so + (2 * HBV_NB + i) * n + cc); hs.iso[i] = __ldcg(a.state + so + (3 * HBV_NB + i) * n + cc);
     }
-    hs.surface_heat = __ldcg(a.state + (4 * HBV_NB) * n + cc); hs.swe = __ldcg(a.state + (4 * HBV_NB + 1) * n + cc);
-    hs.sca = __ldcg(a.state + (4 * HBV_NB + 2) * n + cc);
-    double kq = __ldcg(a.state + (4 * HBV_NB + 3) * n + cc);
+    hs.surface_heat = __ldcg(a.state + so + (4 * HBV_NB) * n + cc); hs.swe = __ldcg(a.state + so + (4 * HBV_NB + 1) * n + cc);
+    hs.sca = __ldcg(a.state + so + (4 * HBV_NB + 2) * n + cc);
+    double kq = __ldcg(a.state + so + (4 * HBV_NB + 3) * n + cc);
 
     int my_slot = -1;
     bool head = false;
@@ -343,7 +355,7 @@ __global__ void __launch_bounds__(128, SB2_HPS_MINBLOCKS) pthpsk_run_kernel(cons
     bool failed_snow = false, failed_k = false;
     int64_t o = (int64_t)i_begin * n + cc;  // running element offset of (step i, cell), bumped by n per step (see ptgsk_snow_kernel)
     const int64_t out_shift = (a.first_step - a.out_first_step) * n;
-    int64_t po = ((int64_t)i_begin * a.n_slots + (my_slot < 0 ? 0 : my_slot)) * 2;  // likewise into partial[step][slot][2]
+    int64_t po = (int64_t)ens * a.ens_partial_stride + ((int64_t)i_begin * a.n_slots + (my_slot < 0 ? 0 : my_slot)) * 2;  // likewise into partial[step][slot][2]
     double f_t = a.f[0][o], f_p = a.f[1][o], f_r = a.f[2][o], f_w = a.f[3][o], f_h = a.f[4][o];
     for (int i = i_begin; i < i_end; ++i, o += n) {
         const double temp = f_t, rad = f_r, wind = f_w, rel_hum = f_h, prec_raw = f_p;
@@ -411,11 +423,12 @@ __global__ void __launch_bounds__(128, SB2_HPS_MINBLOCKS) pthpsk_run_kernel(cons
         if ((a.collect & 8) && a.collect_end_state && i_end == a.n_steps) collect_state((a.first_step + a.n_steps - a.out_first_step) * n + cc);
 #pragma unroll
         for (int i = 0; i < HBV_NB; ++i) {
-            a.state[i * n + cc] = hs.sp[i]; a.state[(HBV_NB + i) * n + cc] = hs.sw[i];
-            a.state[(2 * HBV_NB + i) * n + cc] = hs.albedo[i]; a.state[(3 * HBV_NB + i) * n + cc] = hs.iso[i];
+            a.state[so + i * n + cc] = hs.sp[i]; a.state[so + (HBV_NB + i) * n + cc] = hs.sw[i];
+            a.state[so + (2 * HBV_NB + i) * n + cc] = hs.albedo[i]; a.state[so + (3 * HBV_NB + i) * n + cc] = hs.iso[i];
         }
-        a.state[(4 * HBV_NB) * n + cc] = hs.surface_heat; a.state[(4 * HBV_NB + 1) * n + cc] = hs.swe; a.state[(4 * HBV_NB + 2) * n + cc] = hs.sca;
-        a.state[(4 * HBV_NB + 3) * n + cc] = kq;
+        a.state[so + (4 * HBV_NB) * n + cc] = hs.surface_heat; a.state[so + (4 * HBV_NB + 1) * n + cc] = hs.swe;
+        a.state[so + (4 * HBV_NB + 2) * n + cc] = hs.sca;
+        a.state[so + (4 * HBV_NB + 3) * n + cc] = kq;
         if (failed_snow) atomicOr(a.error_flag, ERR_HBV_NEGATIVE_OUTFLOW);
         if (failed_k) atomicOr(a.error_flag, ERR_KIRCHNER_STEP);
     }

@@ -17,6 +17,7 @@ from shyft_b200 import synthetic
 PTGSK = [-2.439, 0.966, -0.10, 1.5, -0.5, 2.0, 0.1, 1.0, 5.0, 5.0, 30.0, 0.9, 0.6, 5.0, 0.4, 0.4, 1.0, 0.0, 0.0, 0.2, 1.26, 0.04, 100.0, 0.0, 6.0, 1.0, 7.0, 0.0,
          221.0, 0.0, 1.0]
 PTHSK = [-2.439, 0.966, -0.10, 1.5, 0.1, 0.0, 1.0, 0.0, 0.5, 6.0, 1.0, 0.2, 1.26, 1.0, 7.0, 0.0, 0.0, 1.0]
+PTHPSK = [-2.439, 0.966, -0.10, 1.5, 0.1, 0.0, 0.5, 2.0, 1.0, 30.0, 0.9, 0.6, 5.0, 5.0, 5.0, 0.0, 6.0, 1.0, 0.2, 1.26, 1.0, 7.0, 0.0, 1.0]
 HBV = [300.0, 2.0, 150.0, 25.0, 0.5, 0.3, 0.8, 0.02, 0.1, 0.0, 1.0, 0.0, 0.5, 1.0, 0.2, 1.26, 6.0, 1.0, 7.0, 0.0, 0.0, 1.0]
 which = [int(a) for a in sys.argv[1:]] or [3, 5]
 
@@ -68,11 +69,12 @@ if 5 in which:  # calibration ensemble: parameter sets x 10k-cell catchment x 3 
     if world > 1:
         torch.cuda.set_device(local_rank)
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
-    # SB2_C5_STACK: pt_gs_k (default), pt_hs_k or hbv_stack -- the stacks whose batch runs as grid layers on the device
+    # SB2_C5_STACK: pt_gs_k (default), pt_hs_k, hbv_stack or pt_hps_k -- the stacks whose batch runs as grid layers on the device
     stack = os.environ.get("SB2_C5_STACK", "pt_gs_k")
     n, T, sets = 10000, 26280, int(os.environ.get("SB2_C5_SETS", "256"))
     geo, ta, env = synthetic.make_region(n, T, 64, config_index=4)
-    cls, par, sid = {"pt_gs_k": (sb.PTGSKOptModel, PTGSK, 0), "pt_hs_k": (sb.PTHSKOptModel, PTHSK, 1), "hbv_stack": (sb.HbvStackOptModel, HBV, 2)}[stack]
+    cls, par, sid = {"pt_gs_k": (sb.PTGSKOptModel, PTGSK, 0), "pt_hs_k": (sb.PTHSKOptModel, PTHSK, 1), "hbv_stack": (sb.HbvStackOptModel, HBV, 2),
+                     "pt_hps_k": (sb.PTHPSKOptModel, PTHPSK, 4)}[stack]
     m = cls(geo, par, device=local_rank)
     m.run_interpolation(sb.InterpolationParameter(), ta, env)
     m.set_states(synthetic.default_state(sid, n))
@@ -89,6 +91,10 @@ if 5 in which:  # calibration ensemble: parameter sets x 10k-cell catchment x 3 
         P[:, 0] = rng.uniform(-3.0, -1.9, sets); P[:, 1] = rng.uniform(0.8, 0.99, sets); P[:, 2] = rng.uniform(-0.15, -0.05, sets)
         P[:, 3] = rng.uniform(0.5, 2.5, sets); P[:, 5] = rng.uniform(-2, 2, sets); P[:, 6] = rng.uniform(0.5, 2.0, sets)
         P[:, 10] = rng.uniform(0.8, 1.4, sets)
+    elif stack == "pt_hps_k":  # c1, c2, c3, ae_scale, tx, wind_scale, fast / slow albedo decay rate, p_corr
+        P[:, 0] = rng.uniform(-3.0, -1.9, sets); P[:, 1] = rng.uniform(0.8, 0.99, sets); P[:, 2] = rng.uniform(-0.15, -0.05, sets)
+        P[:, 3] = rng.uniform(0.5, 2.5, sets); P[:, 5] = rng.uniform(-2, 2, sets); P[:, 7] = rng.uniform(1.0, 3.0, sets)
+        P[:, 12] = rng.uniform(2.0, 8.0, sets); P[:, 13] = rng.uniform(2.0, 8.0, sets); P[:, 17] = rng.uniform(0.8, 1.4, sets)
     else:                      # fc, beta, lp, uz1, kuz2, kuz1, perc, klz, tx, p_corr
         P[:, 0] = rng.uniform(150, 450, sets); P[:, 1] = rng.uniform(1, 4, sets); P[:, 2] = rng.uniform(100, 200, sets)
         P[:, 3] = rng.uniform(10, 40, sets); P[:, 4] = rng.uniform(0.2, 0.7, sets); P[:, 5] = rng.uniform(0.1, 0.4, sets)
