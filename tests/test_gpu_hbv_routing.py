@@ -33,6 +33,10 @@ def test_pt_hs_k_parity(sb, oracle):
     for name in ("avg_discharge", "charge_m3s", "snow_sca", "snow_swe", "snow_outflow", "glacier_melt", "ae_output", "pe_output"):
         assert_parity(m.response(name), want[name], "pt_hs_k " + name)
     assert_parity(m.get_states(), want["state"], "pt_hs_k end state")
+    # one operation sequence on both machines (DESIGN.md "Deterministic math"): the per-cell results are in fact bit-identical
+    for name in ("avg_discharge", "charge_m3s", "snow_sca", "snow_swe", "snow_outflow", "glacier_melt", "ae_output", "pe_output"):
+        assert np.array_equal(m.response(name), want[name], equal_nan=True), "pt_hs_k " + name + " is within 1e-9 but not bit-identical"
+    assert np.array_equal(m.get_states(), want["state"])
 
 
 def test_hbv_stack_parity(sb, oracle):
@@ -42,6 +46,9 @@ def test_hbv_stack_parity(sb, oracle):
     for name in ("avg_discharge", "charge_m3s", "snow_sca", "snow_swe", "snow_outflow", "glacier_melt", "ae_output", "pe_output", "soil_outflow"):
         assert_parity(m.response(name), want[name], "hbv_stack " + name)
     assert_parity(m.get_states(), want["state"], "hbv_stack end state")
+    for name in ("avg_discharge", "charge_m3s", "snow_sca", "snow_swe", "snow_outflow", "glacier_melt", "ae_output", "pe_output", "soil_outflow"):
+        assert np.array_equal(m.response(name), want[name], equal_nan=True), "hbv_stack " + name + " is within 1e-9 but not bit-identical"
+    assert np.array_equal(m.get_states(), want["state"])
 
 
 def test_hbv_chunked_equals_one_shot_and_state_series(sb):

@@ -168,9 +168,9 @@ def test_config1_slice_parity_through_a_winter(sb, oracle, collect, n):
         assert_parity(cc[:, k], want["charge_m3s"][:, cix == k].sum(axis=1), f"catchment {k} charge", rtol=1e-9, atol_frac=1e-12)
 
 
-@pytest.mark.parametrize("n,T", [(1, 1), (1, 130), (31, 63), (33, 65), (100, 129), (257, 1)])
+@pytest.mark.parametrize("n,T", [(1, 1), (1, 130), (31, 63), (31, 127), (33, 65), (33, 128), (100, 129), (257, 1)])
 def test_ragged_sizes_are_bit_identical(sb, oracle, n, T):
-    """One cell, one step, cell counts around a warp and step counts around the 64-step slice of the time split: every series and
+    """One cell, one step, cell counts around a warp and step counts around the 128-step slice of the time split: every series and
     the end state equal the oracle's bit for bit (out-of-range lanes of the last warp shadow a cell and store nothing)."""
     geo, ta, env, st0 = _synthetic(sb, n, T, 4, config_index=30 + n % 7, cells_per_catchment=max(1, n // 3), start=1424476800)  # 2015-02-21
     st0[:, 5] = -1.0                      # acc_melt < 0: accumulation branch
@@ -299,8 +299,8 @@ def test_full_size_properties_config2_slice(sb):
 
 
 def test_time_sliced_kernels_are_deterministic_and_slicing_invariant(sb):
-    """The snow / response kernels hand a window out in 64-step slices by ticket, each slice waiting for its cell group's previous
-    one (sb2_ptgsk.cuh).  With several waves of blocks (60 000 cells x 10 slices) three runs must agree bit for bit, and so must a
+    """The snow / response kernels hand a window out in 128-step slices by ticket, each slice waiting for its cell group's previous
+    one (sb2_ptgsk.cuh).  With several waves of blocks (60 000 cells x 5 slices) three runs must agree bit for bit, and so must a
     run cut into odd chunks (other slice boundaries, other ticket order) and a windowed run."""
     n, T = 60000, 640
     geo, ta, env, st0 = _synthetic(sb, n, T, 16, config_index=21, start=1417392000)  # 2014-12-01: snow, melt events, wet-snow snowfall

@@ -90,6 +90,9 @@ def test_pt_hps_k_stack_parity_through_a_winter(sb, oracle):
     for name in ("avg_discharge", "charge_m3s", "snow_sca", "snow_swe", "snow_outflow", "glacier_melt", "ae_output", "pe_output"):
         assert_parity(m.response(name), want[name], "pt_hps_k " + name)
     assert_parity(m.get_states(), want["state"], "pt_hps_k end state")
+    for name in ("avg_discharge", "charge_m3s", "snow_sca", "snow_swe", "snow_outflow", "glacier_melt", "ae_output", "pe_output"):
+        assert np.array_equal(m.response(name), want[name], equal_nan=True), "pt_hps_k " + name + " is within 1e-9 but not bit-identical"
+    assert np.array_equal(m.get_states(), want["state"])
     # state series: T + 1 instant values; the first row is the initial state, the last the end state (swe over the cell, the rest as stored)
     s_end = m.get_states()
     frac = 1.0 - geo["lake"] - geo["reservoir"]
