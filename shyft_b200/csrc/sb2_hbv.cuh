@@ -87,7 +87,7 @@ struct HbvRunArgs {
     int64_t n_slots;
     int* __restrict__ error_flag;
     int collect;  // bits as SB2_COLLECT_*
-    int unit_steps;              // > 0: the chunk is stepped in time slices of this many steps handed out by ticket (as ptgsk_response_kernel)
+    int unit_steps;              // > 0: the chunk is stepped in time slices of this many steps handed out by ticket (step_slice_begin)
     int* __restrict__ tickets;   // [1] ticket counter, zeroed per launch
     int* __restrict__ progress;  // [cell groups] finished slices per group, zeroed per launch
     // parameter-set ensemble (calibration): blockIdx.y = member; member e steps its own state / partial sums with the region
@@ -244,33 +244,13 @@ __device__ __forceinline__ bool hbv_snow_step(double (&sp)[HBV_NB], double (&sw)
 // UPAR: no catchment override in use and no ensemble -- every cell reads the region parameter set (a.par0) from the kernel's constant bank
 template <bool HBV_STACK, bool UPAR>
 __global__ void __launch_bounds__(128, (HBV_STACK ? SB2_HBV_MINBLOCKS_S : SB2_HBV_MINBLOCKS_K)) hbv_run_kernel(const __grid_constant__ HbvRunArgs a) {
-    constexpr int NS = HBV_STACK ? 5 + 2 * HBV_NB : 3 + 2 * HBV_NB;
     sb_math_stage_tables();  // exp / log tables of the shared math spec into this block's shared memory (sb2_math.cuh)
     const int ens = UPAR ? 0 : blockIdx.y;  // UPAR launches have no ensemble: the member offsets fold away
-    // Time split by ticket (see ptgsk_response_kernel): 12 500 one-warp blocks of a 400 000-cell shard are 4-5 waves of the 2 400-3 000
-    // resident ones, so whole-chunk blocks leave a ragged last wave; slices of unit_steps steps shrink that tail to one slice.  A block
-    // waits until the previous slice of its cell group has published the state; tickets are handed out in start order, so that slice
-    // always belongs to a block already running or done.
-    int64_t group = blockIdx.x;
-    int i_begin = 0, i_end = a.n_steps, slice = 0;
-    int* progress = nullptr;
-    if (a.unit_steps > 0) {
-        __shared__ int s_ticket;
-        const int n_groups = int((a.n_cells + blockDim.x - 1) / blockDim.x);
-        if (threadIdx.x == 0) s_ticket = atomicAdd(a.tickets + ens, 1);
-        __syncthreads();
-        slice = s_ticket / n_groups;
-        group = s_ticket - slice * n_groups;
-        i_begin = slice * a.unit_steps;
-        i_end = min(a.n_steps, i_begin + a.unit_steps);
-        progress = a.progress + (int64_t)ens * n_groups + group;
-        if (threadIdx.x == 0) {
-            while (*((volatile int*)progress) < slice) __nanosleep(256);
-            __threadfence();
-        }
-        __syncthreads();
-    }
-    const int64_t c = group * blockDim.x + threadIdx.x;
+    // time split by ticket: 12 500 one-warp blocks of a 400 000-cell shard are 4-5 waves of the 2 400-3 000 resident ones, so whole-chunk
+    // blocks leave a ragged last wave
+    const StepSlice sl = step_slice_begin(a, ens);
+    const int i_begin = sl.i_begin, i_end = sl.i_end;
+    const int64_t c = sl.group * blockDim.x + threadIdx.x;
     const bool in_range = c < a.n_cells;
     const int64_t cc = in_range ? c : a.n_cells - 1;
     const bool active = in_range && (a.active == nullptr || a.active[cc] != 0);
@@ -298,13 +278,7 @@ __global__ void __launch_bounds__(128, (HBV_STACK ? SB2_HBV_MINBLOCKS_S : SB2_HB
     double x1 = HBV_STACK ? __ldcg(a.state + so + (3 + 2 * HBV_NB) * n + cc) : 0.0;    // tank.uz
     double x2 = HBV_STACK ? __ldcg(a.state + so + (4 + 2 * HBV_NB) * n + cc) : 0.0;    // tank.lz
 
-    int my_slot = -1;
-    bool head = false;
-    if (a.partial != nullptr) {
-        my_slot = in_range ? a.slot[cc] : -1;
-        const int prev = __shfl_up_sync(0xffffffffu, my_slot, 1);
-        head = in_range && (lane == 0 || prev != my_slot);
-    }
+    const LaneSlot ls = lane_slot(a, a.partial, cc, in_range, lane);
     auto collect_state = [&](int64_t orow) {
         if (HBV_STACK) {  // hbv_stack_cell_model.h:196-212
             a.st[0][orow] = swe; a.st[1][orow] = sca; a.st[2][orow] = x0; a.st[3][orow] = x1; a.st[4][orow] = x2;
@@ -316,12 +290,12 @@ __global__ void __launch_bounds__(128, (HBV_STACK ? SB2_HBV_MINBLOCKS_S : SB2_HB
         for (int i = 0; i < HBV_NB; ++i) { a.st[SP0 + i][orow] = sp[i]; a.st[SP0 + HBV_NB + i][orow] = sw[i]; }  // the bins as they are (:199-202 / :209-212)
     };
 
-    bool failed_snow = false, failed_k = false;
+    bool failed_k = false, failed_snow = false;
     // the next step's forcing is loaded one step ahead into registers and SB2_PREFETCH_AHEAD steps ahead into L1 (as the pt_gs_k kernels do):
     // the step consumes one 8-byte value per array, so without it every step waits for DRAM
     int64_t o = (int64_t)i_begin * n + cc;  // running element offset of (step i, cell), bumped by n per step (see ptgsk_snow_kernel)
     const int64_t out_shift = (a.first_step - a.out_first_step) * n;
-    int64_t po = (int64_t)ens * a.ens_partial_stride + ((int64_t)i_begin * a.n_slots + (my_slot < 0 ? 0 : my_slot)) * 2;  // likewise into partial[step][slot][2]
+    int64_t po = (int64_t)ens * a.ens_partial_stride + ((int64_t)i_begin * a.n_slots + (ls.slot < 0 ? 0 : ls.slot)) * 2;  // likewise into partial[step][slot][2]
     double f_t = a.f[0][o], f_p = a.f[1][o], f_r = a.f[2][o], f_h = a.f[4][o];
     for (int i = i_begin; i < i_end; ++i, o += n) {
         const double temp = f_t, rad = f_r, rel_hum = f_h, prec_raw = f_p;
@@ -403,19 +377,7 @@ __global__ void __launch_bounds__(128, (HBV_STACK ? SB2_HBV_MINBLOCKS_S : SB2_HB
             }
         }
         if (a.partial != nullptr) {
-            double v0 = out_q, v1 = out_charge;
-#pragma unroll
-            for (int off = 1; off < 32; off <<= 1) {
-                const double o0 = __shfl_down_sync(0xffffffffu, v0, off);
-                const double o1 = __shfl_down_sync(0xffffffffu, v1, off);
-                const int os = __shfl_down_sync(0xffffffffu, my_slot, off);
-                if (lane + off < 32 && os == my_slot) { v0 += o0; v1 += o1; }
-            }
-            if (head) {
-                double* dst = a.partial + po;  // ((int64_t)i * a.n_slots + my_slot) * 2
-                dst[0] = v0;
-                dst[1] = v1;
-            }
+            slot_sum_store(out_q, out_charge, ls, a.partial, po);
             po += 2 * a.n_slots;
         }
     }
@@ -428,13 +390,8 @@ __global__ void __launch_bounds__(128, (HBV_STACK ? SB2_HBV_MINBLOCKS_S : SB2_HB
         if (HBV_STACK) { a.state[so + (3 + 2 * HBV_NB) * n + cc] = x1; a.state[so + (4 + 2 * HBV_NB) * n + cc] = x2; }
         if (failed_snow) atomicOr(a.error_flag, ERR_HBV_NEGATIVE_OUTFLOW);
         if (failed_k) atomicOr(a.error_flag, ERR_KIRCHNER_STEP);
-        (void)NS;
     }
-    if (progress != nullptr) {  // publish this slice: the state stores above, then the counter
-        __threadfence();
-        __syncthreads();
-        if (threadIdx.x == 0) atomicExch(progress, slice + 1);
-    }
+    step_slice_publish(sl);
 }
 
 }  // namespace sb2

@@ -98,7 +98,7 @@ struct PtgskRunArgs {
     // 0 potential evapotranspiration [mm/h], 1 long-wave addend, 2 turbulent addend, 3 snow outflow [mm/h], 4 snow covered area
     double* __restrict__ scr[5];
     int64_t ens_scr_stride;  // elements between two members' scratch arrays
-    // response kernel time split (see ptgsk_response_kernel): steps per work unit (0 = one unit per cell group), ticket counter per
+    // time split of the snow / response kernels (step_slice_begin): steps per work unit (0 = one unit per cell group), ticket counter per
     // ensemble member, finished units per (member, cell group)
     int unit_steps;
     int* __restrict__ tickets;
@@ -752,6 +752,93 @@ __device__ __forceinline__ bool kirchner_step_warp(const ARGS& ka, double c1, do
 __device__ __forceinline__ void prefetch_l1(const double* p) { asm volatile("prefetch.global.L1 [%0];" ::"l"(p)); }
 #define SB2_PREFETCH_AHEAD 4   // steps; 2 and 8 measure the same, no L1 prefetch 2.5 % slower (profiles/README.md)
 
+// ---- time slices by ticket (the five step kernels) ---------------------------------------------------------------------------
+// A block steps one group of blockDim cells.  When a launch of whole-window blocks is only a few waves, the last wave leaves most of
+// the machine idle for as long as a whole window takes, so the window is cut into slices of unit_steps steps: blocks take tickets
+// (ticket t = cell group t % G, time slice t / G), wait until the same group's previous slice has published its state, step their
+// slice and publish.  Tickets are handed out in start order, so the slice a block waits for always belongs to a block that is already
+// running or done: no deadlock, and the tail shrinks to one slice.  A slice reads the state its predecessor wrote a moment ago,
+// possibly on another SM: the kernels read it with __ldcg (from L2, never from a line this SM's L1 still holds from an earlier slice).
+// The tickets buffer (launch_step_chunk, step_groups) holds [members] ticket counters, then [members][G] finished slices (`progress`),
+// zeroed before every launch.
+struct StepSlice {
+    int64_t group;       // the block's cell group: cells group * blockDim.x + threadIdx.x
+    int i_begin, i_end;  // its steps of the launch
+    int slice;
+    int* progress;       // the group's finished slices of this member; null = no time split
+};
+// a: the kernel's *RunArgs (n_cells, n_steps, unit_steps, tickets, progress), read in place where each field is needed; a.unit_steps == 0:
+// the whole launch for cell group blockIdx.x.  The order of the locals here and of the fields of LaneSlot below is the one with which
+// the kernels compile to the same SASS as when this code was written out in each of them; another order moves instructions.
+template <class ARGS>
+__device__ __forceinline__ StepSlice step_slice_begin(const ARGS& a, int member) {
+    int64_t group = blockIdx.x;
+    int* progress = nullptr;
+    int slice = 0, i_begin = 0, i_end = a.n_steps;
+    if (a.unit_steps > 0) {
+        __shared__ int s_ticket;
+        const int n_groups = int((a.n_cells + blockDim.x - 1) / blockDim.x);
+        if (threadIdx.x == 0) s_ticket = atomicAdd(a.tickets + member, 1);
+        __syncthreads();
+        slice = s_ticket / n_groups;
+        group = s_ticket - slice * n_groups;
+        i_begin = slice * a.unit_steps;
+        i_end = min(a.n_steps, i_begin + a.unit_steps);
+        progress = a.progress + (int64_t)member * n_groups + group;
+        if (threadIdx.x == 0) {
+            while (*((volatile int*)progress) < slice) __nanosleep(256);
+            __threadfence();
+        }
+        __syncthreads();
+    }
+    return StepSlice{group, i_begin, i_end, slice, progress};
+}
+// publish the slice: the block's state stores, then the counter
+__device__ __forceinline__ void step_slice_publish(const StepSlice& s) {
+    if (s.progress != nullptr) {
+        __threadfence();
+        __syncthreads();
+        if (threadIdx.x == 0) atomicExch(s.progress, s.slice + 1);
+    }
+}
+
+// ---- catchment partial sums (DESIGN §3.4) ------------------------------------------------------------------------------------
+// Each (warp, run of cells of one catchment) owns a slot (build_slots); per step, the lanes of a slot add their discharge and charge
+// by a shuffle tree and the slot's first lane stores the sums at partial[step][slot][2].  The slots and the order of every addition
+// are fixed by the cell order alone, so the sums are the same bits run to run, and in a batch member as in a single run.
+// `lane` = threadIdx.x & 31 comes from the kernel: there the launch bounds limit threadIdx.x, which can fold the mask away
+struct LaneSlot {
+    unsigned lane;
+    bool head;  // the slot's first lane: it stores the sums
+    int slot;   // -1: out-of-range lane, or no partial sums
+};
+template <class ARGS>
+__device__ __forceinline__ LaneSlot lane_slot(const ARGS& a, const double* partial, int64_t cc, bool in_range, unsigned lane) {
+    LaneSlot s{lane, false, -1};
+    if (partial != nullptr) {
+        s.slot = in_range ? a.slot[cc] : -1;
+        const int prev = __shfl_up_sync(0xffffffffu, s.slot, 1);
+        s.head = in_range && (lane == 0 || prev != s.slot);
+    }
+    return s;
+}
+// every lane of the warp calls it; partial + po is the lane's slot at this step
+__device__ __forceinline__ void slot_sum_store(double q, double charge, const LaneSlot& s, double* partial, int64_t po) {
+    double v0 = q, v1 = charge;
+#pragma unroll
+    for (int off = 1; off < 32; off <<= 1) {
+        const double o0 = __shfl_down_sync(0xffffffffu, v0, off);
+        const double o1 = __shfl_down_sync(0xffffffffu, v1, off);
+        const int os = __shfl_down_sync(0xffffffffu, s.slot, off);
+        if (s.lane + off < 32 && os == s.slot) { v0 += o0; v1 += o1; }
+    }
+    if (s.head) {
+        double* dst = partial + po;  // ((int64_t)i * n_slots + slot) * 2
+        dst[0] = v0;
+        dst[1] = v1;
+    }
+}
+
 // ---- the phase pipeline (the production path of run_cells) ----------------------------------------------------------
 // The stack of one step is a chain  forcing -> snow -> response  with no feedback from the Kirchner response into the snow
 // pack, so a window of steps is run as three kernels that hand [step][cell] arrays to each other:
@@ -810,28 +897,11 @@ template <int COLLECT, bool UPAR>
 __global__ void __launch_bounds__(SB2_BLOCK_B, SB2_MINBLOCKS_B) ptgsk_snow_kernel(const __grid_constant__ PtgskRunArgs a) {
     sb_math_stage_tables();
     const int ens = UPAR ? 0 : blockIdx.y;  // UPAR launches have no ensemble: the member offsets fold away
-    // time split by ticket, as in ptgsk_response_kernel (1.76 waves of whole-window blocks otherwise); the memo starts empty in
-    // every slice, which costs one snow-state evaluation per cell and slice
-    int64_t group = blockIdx.x;
-    int i_begin = 0, i_end = a.n_steps, slice = 0;
-    int* progress = nullptr;
-    if (a.unit_steps > 0) {
-        __shared__ int s_ticket;
-        const int n_groups = int((a.n_cells + blockDim.x - 1) / blockDim.x);
-        if (threadIdx.x == 0) s_ticket = atomicAdd(a.tickets + ens, 1);
-        __syncthreads();
-        slice = s_ticket / n_groups;
-        group = s_ticket - slice * n_groups;
-        i_begin = slice * a.unit_steps;
-        i_end = min(a.n_steps, i_begin + a.unit_steps);
-        progress = a.progress + (int64_t)ens * n_groups + group;
-        if (threadIdx.x == 0) {
-            while (*((volatile int*)progress) < slice) __nanosleep(256);
-            __threadfence();
-        }
-        __syncthreads();
-    }
-    const int64_t c = group * blockDim.x + threadIdx.x;
+    // time split by ticket (1.76 waves of whole-window blocks otherwise); the memo starts empty in every slice, which costs one
+    // snow-state evaluation per cell and slice
+    const StepSlice sl = step_slice_begin(a, ens);
+    const int i_begin = sl.i_begin, i_end = sl.i_end;
+    const int64_t c = sl.group * blockDim.x + threadIdx.x;
     const bool live = c < a.n_cells && (a.active == nullptr || a.active[c] != 0);
     if (live) {
     const PtgskParam& p = UPAR ? a.par0 : ((a.ens_params != nullptr && a.pset[c] == 0) ? a.ens_params[ens] : a.params[a.pset[c]]);
@@ -855,6 +925,16 @@ __global__ void __launch_bounds__(SB2_BLOCK_B, SB2_MINBLOCKS_B) ptgsk_snow_kerne
     gs.iso_pot_energy = __ldcg(state + 6 * n + c); gs.temp_swe = __ldcg(state + 7 * n + c);
     GsCache cache;
     gs_cache_clear(cache);
+    auto collect_state = [&](int64_t orow) {  // the state at the beginning of a step, scale_snow applied (pt_gs_k.h:213-218,367)
+        a.st[1][orow] = gs.albedo;
+        a.st[2][orow] = gs.lwc * snow_storage_fraction;
+        a.st[3][orow] = gs.surface_heat;
+        a.st[4][orow] = gs.alpha;
+        a.st[5][orow] = gs.sdc_melt_mean;
+        a.st[6][orow] = gs.acc_melt;
+        a.st[7][orow] = gs.iso_pot_energy;
+        a.st[8][orow] = gs.temp_swe * snow_storage_fraction;
+    };
     // o: running element offset of (step i, cell c) in every [step][cell] array of the chunk -- bumped by n per step instead of
     // multiplied out (the 64-bit i * n + c per array access was a sixth of this kernel's instructions)
     int64_t o = (int64_t)i_begin * n + c;
@@ -875,16 +955,7 @@ __global__ void __launch_bounds__(SB2_BLOCK_B, SB2_MINBLOCKS_B) ptgsk_snow_kerne
             prefetch_l1(a.f[0] + o2); prefetch_l1(a.f[1] + o2); prefetch_l1(a.f[2] + o2); prefetch_l1(s_lw + o2); prefetch_l1(s_tadd + o2);
         }
         const int64_t orow = o + out_shift;  // (step - a.out_first_step) * n + c
-        if (COLLECT & 8) {  // state at the beginning of the period, scale_snow applied (pt_gs_k.h:213-218,367)
-            a.st[1][orow] = gs.albedo;
-            a.st[2][orow] = gs.lwc * snow_storage_fraction;
-            a.st[3][orow] = gs.surface_heat;
-            a.st[4][orow] = gs.alpha;
-            a.st[5][orow] = gs.sdc_melt_mean;
-            a.st[6][orow] = gs.acc_melt;
-            a.st[7][orow] = gs.iso_pot_energy;
-            a.st[8][orow] = gs.temp_swe * snow_storage_fraction;
-        }
+        if (COLLECT & 8) collect_state(orow);
         double sca, storage, outflow;
         gs_step_core(gs, cache, sca, storage, outflow, p, ds.x, ds.y, a.dt_seconds, a.dt_us, gk, a.bb0, temp, rad, prec, lw, tadd, a.f[3],
                      a.f[4], o, inv_cv2);
@@ -893,26 +964,12 @@ __global__ void __launch_bounds__(SB2_BLOCK_B, SB2_MINBLOCKS_B) ptgsk_snow_kerne
         if (COLLECT & 2) { a.resp[2][orow] = sca; a.resp[3][orow] = storage * snow_storage_fraction; }
         if (COLLECT & 4) a.resp[4][orow] = mmh_to_m3s(outflow * snow_storage_fraction, cell_area_m2);
     }
-    if ((COLLECT & 8) && a.collect_end_state && i_end == a.n_steps) {
-        const int64_t orow = (a.first_step + a.n_steps - a.out_first_step) * n + c;
-        a.st[1][orow] = gs.albedo;
-        a.st[2][orow] = gs.lwc * snow_storage_fraction;
-        a.st[3][orow] = gs.surface_heat;
-        a.st[4][orow] = gs.alpha;
-        a.st[5][orow] = gs.sdc_melt_mean;
-        a.st[6][orow] = gs.acc_melt;
-        a.st[7][orow] = gs.iso_pot_energy;
-        a.st[8][orow] = gs.temp_swe * snow_storage_fraction;
-    }
+    if ((COLLECT & 8) && a.collect_end_state && i_end == a.n_steps) collect_state((a.first_step + a.n_steps - a.out_first_step) * n + c);
     state[0 * n + c] = gs.albedo; state[1 * n + c] = gs.lwc; state[2 * n + c] = gs.surface_heat; state[3 * n + c] = gs.alpha;
     state[4 * n + c] = gs.sdc_melt_mean; state[5 * n + c] = gs.acc_melt; state[6 * n + c] = gs.iso_pot_energy;
     state[7 * n + c] = gs.temp_swe;
     }  // live
-    if (progress != nullptr) {  // publish this slice: the state stores above, then the counter
-        __threadfence();
-        __syncthreads();
-        if (threadIdx.x == 0) atomicExch(progress, slice + 1);
-    }
+    step_slice_publish(sl);
 }
 
 // COLLECT bits used here: 1 avg_discharge+charge, 4 glacier_melt/ae/pe, 8 state series (kirchner discharge)
@@ -920,32 +977,11 @@ template <int COLLECT, bool UPAR>
 __global__ void __launch_bounds__(SB2_BLOCK_C, SB2_MINBLOCKS_C) ptgsk_response_kernel(const __grid_constant__ PtgskRunArgs a) {
     sb_math_stage_tables();
     const int ens = UPAR ? 0 : blockIdx.y;  // UPAR launches have no ensemble
-    // Time split.  A block steps one group of blockDim cells; with ~115 registers 2 500 of the 3 125 one-warp blocks of a 100 000-cell
-    // shard are resident, so a launch of whole-window blocks runs as 1.25 waves -- the second wave leaves three quarters of the
-    // machine idle for as long as the first took.  The window is therefore cut into units of unit_steps steps: blocks take tickets
-    // (unit = ticket: cell group ticket % G, time slice ticket / G), wait until the same group's previous slice has published its
-    // state, step their slice and publish.  Tickets are handed out in start order, so the slice a block waits for always belongs to
-    // a block that is already running or done: no deadlock, and the tail shrinks to one slice.
-    int64_t group = blockIdx.x;
-    int i_begin = 0, i_end = a.n_steps, slice = 0;
-    int* progress = nullptr;
-    if (a.unit_steps > 0) {
-        __shared__ int s_ticket;
-        const int n_groups = int((a.n_cells + blockDim.x - 1) / blockDim.x);
-        if (threadIdx.x == 0) s_ticket = atomicAdd(a.tickets + ens, 1);
-        __syncthreads();
-        slice = s_ticket / n_groups;
-        group = s_ticket - slice * n_groups;
-        i_begin = slice * a.unit_steps;
-        i_end = min(a.n_steps, i_begin + a.unit_steps);
-        progress = a.progress + (int64_t)ens * n_groups + group;
-        if (threadIdx.x == 0) {
-            while (*((volatile int*)progress) < slice) __nanosleep(256);
-            __threadfence();
-        }
-        __syncthreads();
-    }
-    const int64_t c = group * blockDim.x + threadIdx.x;
+    // time split by ticket: with ~115 registers 2 500 of the 3 125 one-warp blocks of a 100 000-cell shard are resident, so a launch of
+    // whole-window blocks runs as 1.25 waves -- the second wave leaves three quarters of the machine idle for as long as the first took
+    const StepSlice sl = step_slice_begin(a, ens);
+    const int i_begin = sl.i_begin, i_end = sl.i_end;
+    const int64_t c = sl.group * blockDim.x + threadIdx.x;
     const bool in_range = c < a.n_cells;
     const int64_t cc = in_range ? c : a.n_cells - 1;  // out-of-range lanes shadow the last cell, never store
     const bool active = in_range && (a.active == nullptr || a.active[cc] != 0);
@@ -998,15 +1034,9 @@ __global__ void __launch_bounds__(SB2_BLOCK_C, SB2_MINBLOCKS_C) ptgsk_response_k
     const int64_t n = a.n_cells;
     double kq = __ldcg(state + 8 * n + cc);  // L2, not L1: written by the previous time slice, possibly on another SM
 
-    int my_slot = -1;
-    bool head = false;
-    if (partial != nullptr) {
-        my_slot = in_range ? a.slot[cc] : -1;
-        const int prev = __shfl_up_sync(0xffffffffu, my_slot, 1);
-        head = in_range && (lane == 0 || prev != my_slot);
-    }
+    const LaneSlot ls = lane_slot(a, partial, cc, in_range, lane);
     int64_t o = (int64_t)i_begin * n + cc;  // running element offset of (step i, cell), bumped by n per step (see ptgsk_snow_kernel)
-    int64_t po = ((int64_t)i_begin * a.n_slots + (my_slot < 0 ? 0 : my_slot)) * 2;  // likewise into partial[step][slot][2]
+    int64_t po = ((int64_t)i_begin * a.n_slots + (ls.slot < 0 ? 0 : ls.slot)) * 2;  // likewise into partial[step][slot][2]
     const int64_t out_shift = (a.first_step - a.out_first_step) * n;
     double f_t = a.f[0][o], f_p = a.f[1][o], f_pot = s_pot[o], f_out = s_outflow[o], f_sca = s_sca[o];
     bool failed = false;
@@ -1056,19 +1086,7 @@ __global__ void __launch_bounds__(SB2_BLOCK_C, SB2_MINBLOCKS_C) ptgsk_response_k
             }
         }
         if (partial != nullptr) {  // warp-uniform
-            double v0 = out_q, v1 = out_charge;
-#pragma unroll
-            for (int off = 1; off < 32; off <<= 1) {
-                const double o0 = __shfl_down_sync(0xffffffffu, v0, off);
-                const double o1 = __shfl_down_sync(0xffffffffu, v1, off);
-                const int os = __shfl_down_sync(0xffffffffu, my_slot, off);
-                if (lane + off < 32 && os == my_slot) { v0 += o0; v1 += o1; }
-            }
-            if (head) {
-                double* dst = partial + po;  // ((int64_t)i * a.n_slots + my_slot) * 2
-                dst[0] = v0;
-                dst[1] = v1;
-            }
+            slot_sum_store(out_q, out_charge, ls, partial, po);
             po += 2 * a.n_slots;
         }
     }
@@ -1080,11 +1098,7 @@ __global__ void __launch_bounds__(SB2_BLOCK_C, SB2_MINBLOCKS_C) ptgsk_response_k
         state[8 * n + cc] = kq;
         if (failed) atomicOr(a.error_flag, ERR_KIRCHNER_STEP);
     }
-    if (progress != nullptr) {  // publish this slice: the state stores above, then the counter
-        __threadfence();
-        __syncthreads();
-        if (threadIdx.x == 0) atomicExch(progress, slice + 1);
-    }
+    step_slice_publish(sl);
 }
 #undef cell_area_m2
 #undef glacier_fraction

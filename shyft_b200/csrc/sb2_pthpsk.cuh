@@ -2,7 +2,7 @@
 //
 // hbv_physical_snow keeps the five quantile bins of hbv_snow (sp, sw) and melts each of them with its own gamma_snow-type energy balance
 // (albedo and iso_pot_energy per bin, one surface_heat).  One thread per cell, all 24 state values in registers, every bin loop unrolled;
-// the scaffold (forcing prefetch, time slices by ticket, warp-synchronous Kirchner, segmented catchment sums) is hbv_run_kernel's.
+// forcing prefetch as hbv_run_kernel; time slices by ticket, warp-synchronous Kirchner and segmented catchment sums from sb2_ptgsk.cuh.
 //
 // Follows, step for step:
 //   pt_hps_k::run                              core/pt_hps_k.h:201-303
@@ -287,26 +287,9 @@ template <bool ENS>
 __global__ void __launch_bounds__(128, SB2_HPS_MINBLOCKS) pthpsk_run_kernel(const __grid_constant__ HpsRunArgs a) {
     sb_math_stage_tables();
     const int ens = ENS ? blockIdx.y : 0;
-    int64_t group = blockIdx.x;
-    int i_begin = 0, i_end = a.n_steps, slice = 0;
-    int* progress = nullptr;
-    if (a.unit_steps > 0) {  // time slices handed out by ticket, as hbv_run_kernel
-        __shared__ int s_ticket;
-        const int n_groups = int((a.n_cells + blockDim.x - 1) / blockDim.x);
-        if (threadIdx.x == 0) s_ticket = atomicAdd(a.tickets + ens, 1);
-        __syncthreads();
-        slice = s_ticket / n_groups;
-        group = s_ticket - slice * n_groups;
-        i_begin = slice * a.unit_steps;
-        i_end = min(a.n_steps, i_begin + a.unit_steps);
-        progress = a.progress + (int64_t)ens * n_groups + group;
-        if (threadIdx.x == 0) {
-            while (*((volatile int*)progress) < slice) __nanosleep(256);
-            __threadfence();
-        }
-        __syncthreads();
-    }
-    const int64_t c = group * blockDim.x + threadIdx.x;
+    const StepSlice sl = step_slice_begin(a, ens);
+    const int i_begin = sl.i_begin, i_end = sl.i_end;
+    const int64_t c = sl.group * blockDim.x + threadIdx.x;
     const bool in_range = c < a.n_cells;
     const int64_t cc = in_range ? c : a.n_cells - 1;
     const bool active = in_range && (a.active == nullptr || a.active[cc] != 0);
@@ -334,13 +317,7 @@ __global__ void __launch_bounds__(128, SB2_HPS_MINBLOCKS) pthpsk_run_kernel(cons
     hs.sca = __ldcg(a.state + so + (4 * HBV_NB + 2) * n + cc);
     double kq = __ldcg(a.state + so + (4 * HBV_NB + 3) * n + cc);
 
-    int my_slot = -1;
-    bool head = false;
-    if (a.partial != nullptr) {
-        my_slot = in_range ? a.slot[cc] : -1;
-        const int prev = __shfl_up_sync(0xffffffffu, my_slot, 1);
-        head = in_range && (lane == 0 || prev != my_slot);
-    }
+    const LaneSlot ls = lane_slot(a, a.partial, cc, in_range, lane);
     auto collect_state = [&](int64_t orow) {  // state.scale_snow (pt_hps_k.h:172-176) through the state collector (pt_hps_k_cell_model.h:213-229)
         a.st[0][orow] = mmh_to_m3s(kq, cell_area_m2);
         a.st[1][orow] = hs.sca;
@@ -352,10 +329,10 @@ __global__ void __launch_bounds__(128, SB2_HPS_MINBLOCKS) pthpsk_run_kernel(cons
             a.st[4 + 2 * HBV_NB + i][orow] = hs.albedo[i]; a.st[4 + 3 * HBV_NB + i][orow] = hs.iso[i];
         }
     };
-    bool failed_snow = false, failed_k = false;
+    bool failed_k = false, failed_snow = false;
     int64_t o = (int64_t)i_begin * n + cc;  // running element offset of (step i, cell), bumped by n per step (see ptgsk_snow_kernel)
     const int64_t out_shift = (a.first_step - a.out_first_step) * n;
-    int64_t po = (int64_t)ens * a.ens_partial_stride + ((int64_t)i_begin * a.n_slots + (my_slot < 0 ? 0 : my_slot)) * 2;  // likewise into partial[step][slot][2]
+    int64_t po = (int64_t)ens * a.ens_partial_stride + ((int64_t)i_begin * a.n_slots + (ls.slot < 0 ? 0 : ls.slot)) * 2;  // likewise into partial[step][slot][2]
     double f_t = a.f[0][o], f_p = a.f[1][o], f_r = a.f[2][o], f_w = a.f[3][o], f_h = a.f[4][o];
     for (int i = i_begin; i < i_end; ++i, o += n) {
         const double temp = f_t, rad = f_r, wind = f_w, rel_hum = f_h, prec_raw = f_p;
@@ -403,19 +380,7 @@ __global__ void __launch_bounds__(128, SB2_HPS_MINBLOCKS) pthpsk_run_kernel(cons
             }
         }
         if (a.partial != nullptr) {
-            double v0 = out_q, v1 = out_charge;
-#pragma unroll
-            for (int off = 1; off < 32; off <<= 1) {
-                const double o0 = __shfl_down_sync(0xffffffffu, v0, off);
-                const double o1 = __shfl_down_sync(0xffffffffu, v1, off);
-                const int os = __shfl_down_sync(0xffffffffu, my_slot, off);
-                if (lane + off < 32 && os == my_slot) { v0 += o0; v1 += o1; }
-            }
-            if (head) {
-                double* dst = a.partial + po;  // ((int64_t)i * a.n_slots + my_slot) * 2
-                dst[0] = v0;
-                dst[1] = v1;
-            }
+            slot_sum_store(out_q, out_charge, ls, a.partial, po);
             po += 2 * a.n_slots;
         }
     }
@@ -432,11 +397,7 @@ __global__ void __launch_bounds__(128, SB2_HPS_MINBLOCKS) pthpsk_run_kernel(cons
         if (failed_snow) atomicOr(a.error_flag, ERR_HBV_NEGATIVE_OUTFLOW);
         if (failed_k) atomicOr(a.error_flag, ERR_KIRCHNER_STEP);
     }
-    if (progress != nullptr) {
-        __threadfence();
-        __syncthreads();
-        if (threadIdx.x == 0) atomicExch(progress, slice + 1);
-    }
+    step_slice_publish(sl);
 }
 
 }  // namespace sb2

@@ -1,9 +1,9 @@
 // sb2_ptssk.cuh -- the pt_ss_k cell stack (Priestley-Taylor, Skaugen snow, actual evapotranspiration, Kirchner) on sm_100a.
 //
 // One thread per cell; the seven Skaugen state values and the Kirchner discharge stay in registers over the window, forcing and collected
-// series are [time][cell], the Kirchner step is the warp-synchronous solver of sb2_ptgsk.cuh, the time split by ticket and the catchment
-// partial sums are those of hbv_run_kernel.  The snow routine is rare, branchy work (a melt step with a partly covered cell searches the
-// crossing of two gamma densities), so it sits out of line.
+// series are [time][cell]; the Kirchner step is the warp-synchronous solver of sb2_ptgsk.cuh, the time split by ticket and the catchment
+// partial sums are its step_slice_begin and slot_sum_store.  The snow routine is rare, branchy work (a melt step with a partly covered cell
+// searches the crossing of two gamma densities), so it sits out of line.
 //
 // Follows, step for step:
 //   pt_ss_k::run                             core/pt_ss_k.h:195-293
@@ -348,26 +348,9 @@ __device__ __forceinline__ void ss_step(const SskParam& p, double dt_hours, doub
 // collect bits as SB2_COLLECT_*: 1 avg_discharge + charge, 2 snow sca / swe, 4 snow_outflow / glacier_melt / ae / pe, 8 state series
 __global__ void __launch_bounds__(128, 4) ptssk_run_kernel(const __grid_constant__ SskRunArgs a) {
     sb_math_stage_tables();
-    int64_t group = blockIdx.x;
-    int i_begin = 0, i_end = a.n_steps, slice = 0;
-    int* progress = nullptr;
-    if (a.unit_steps > 0) {  // time slices handed out by ticket, as hbv_run_kernel
-        __shared__ int s_ticket;
-        const int n_groups = int((a.n_cells + blockDim.x - 1) / blockDim.x);
-        if (threadIdx.x == 0) s_ticket = atomicAdd(a.tickets, 1);
-        __syncthreads();
-        slice = s_ticket / n_groups;
-        group = s_ticket - slice * n_groups;
-        i_begin = slice * a.unit_steps;
-        i_end = min(a.n_steps, i_begin + a.unit_steps);
-        progress = a.progress + group;
-        if (threadIdx.x == 0) {
-            while (*((volatile int*)progress) < slice) __nanosleep(256);
-            __threadfence();
-        }
-        __syncthreads();
-    }
-    const int64_t c = group * blockDim.x + threadIdx.x;
+    const StepSlice sl = step_slice_begin(a, 0);
+    const int i_begin = sl.i_begin, i_end = sl.i_end;
+    const int64_t c = sl.group * blockDim.x + threadIdx.x;
     const bool in_range = c < a.n_cells;
     const int64_t cc = in_range ? c : a.n_cells - 1;
     const bool active = in_range && (a.active == nullptr || a.active[cc] != 0);
@@ -389,13 +372,7 @@ __global__ void __launch_bounds__(128, 4) ptssk_run_kernel(const __grid_constant
     ss.num_units = (unsigned long long)__ldcg(a.state + 6 * n + cc);
     double kq = __ldcg(a.state + 7 * n + cc);
 
-    int my_slot = -1;
-    bool head = false;
-    if (a.partial != nullptr) {
-        my_slot = in_range ? a.slot[cc] : -1;
-        const int prev = __shfl_up_sync(0xffffffffu, my_slot, 1);
-        head = in_range && (lane == 0 || prev != my_slot);
-    }
+    const LaneSlot ls = lane_slot(a, a.partial, cc, in_range, lane);
     auto collect_state = [&](int64_t orow) {  // state.scale_snow (pt_ss_k.h:165-171) through the state collector (pt_ss_k_cell_model.h:190-199)
         const double swe = ss.swe * snow_storage_fraction, fw = ss.free_water * snow_storage_fraction;
         a.st[0][orow] = mmh_to_m3s(kq, cell_area_m2);
@@ -409,7 +386,7 @@ __global__ void __launch_bounds__(128, 4) ptssk_run_kernel(const __grid_constant
     bool failed_snow = false, failed_k = false;
     int64_t o = (int64_t)i_begin * n + cc;  // running element offset of (step i, cell), bumped by n per step (see ptgsk_snow_kernel)
     const int64_t out_shift = (a.first_step - a.out_first_step) * n;
-    int64_t po = ((int64_t)i_begin * a.n_slots + (my_slot < 0 ? 0 : my_slot)) * 2;  // likewise into partial[step][slot][2]
+    int64_t po = ((int64_t)i_begin * a.n_slots + (ls.slot < 0 ? 0 : ls.slot)) * 2;  // likewise into partial[step][slot][2]
     double f_t = a.f[0][o], f_p = a.f[1][o], f_r = a.f[2][o], f_h = a.f[4][o];
     for (int i = i_begin; i < i_end; ++i, o += n) {
         const double temp = f_t, rad = f_r, rel_hum = f_h, prec_raw = f_p;
@@ -459,19 +436,7 @@ __global__ void __launch_bounds__(128, 4) ptssk_run_kernel(const __grid_constant
             }
         }
         if (a.partial != nullptr) {
-            double v0 = out_q, v1 = out_charge;
-#pragma unroll
-            for (int off = 1; off < 32; off <<= 1) {
-                const double o0 = __shfl_down_sync(0xffffffffu, v0, off);
-                const double o1 = __shfl_down_sync(0xffffffffu, v1, off);
-                const int os = __shfl_down_sync(0xffffffffu, my_slot, off);
-                if (lane + off < 32 && os == my_slot) { v0 += o0; v1 += o1; }
-            }
-            if (head) {
-                double* dst = a.partial + po;  // ((int64_t)i * a.n_slots + my_slot) * 2
-                dst[0] = v0;
-                dst[1] = v1;
-            }
+            slot_sum_store(out_q, out_charge, ls, a.partial, po);
             po += 2 * a.n_slots;
         }
     }
@@ -483,11 +448,7 @@ __global__ void __launch_bounds__(128, 4) ptssk_run_kernel(const __grid_constant
         if (failed_snow) atomicOr(a.error_flag, ERR_SKAUGEN_SEARCH);
         if (failed_k) atomicOr(a.error_flag, ERR_KIRCHNER_STEP);
     }
-    if (progress != nullptr) {
-        __threadfence();
-        __syncthreads();
-        if (threadIdx.x == 0) atomicExch(progress, slice + 1);
-    }
+    step_slice_publish(sl);
 }
 
 }  // namespace sb2

@@ -14,6 +14,8 @@ BUDGET = {
     "ptgsk_response_kernelILi1E": (122, 0),         # 16 one-warp blocks per SM, no spills
     "hbv_run_kernelILb0E": (128, 64),               # pt_hs_k: 16 resident warps
     "hbv_run_kernelILb1E": (96, 160),               # hbv_stack: 20 resident warps
+    "pthpsk_run_kernelILb0E": (128, 184),           # pt_hps_k run_cells: 16 resident warps (launch bound (128, 4)); 184 B as before the batch existed
+    "pthpsk_run_kernelILb1E": (128, 248),           # pt_hps_k calibration batch: measured 128 / 192, allowed up to 64 B over the run_cells kernel
     "dense_apply_dmma_kernelILi6ELi2ELi0ELb1ELi16ELi32E": (80, 0),   # compacted IDW, 10 neighbours
     "dense_apply_dmma_kernelILi16ELi2ELi1ELb0ELi16ELi0E": (128, 0),  # Bayesian kriging, 64 stations
 }
