@@ -536,6 +536,9 @@ struct StepTarget {
     int64_t state_stride = 0, partial_stride = 0, catch_stride = 0, scr_stride = 0;
     int* tickets = nullptr;               // [members] + [members][step_groups]
     bool series = false;                  // write the model's collected series (m->collect_bits)
+    // a batch with a routed target: avg_discharge / charge of the chunk's step i and cell c at q / charge + e * resp_stride + i * n
+    double *q = nullptr, *charge = nullptr;
+    int64_t resp_stride = 0;
 };
 
 // One chunk of steps [s0, s0 + chunk) for the model's stack: its step kernels, then catchment_reduce_kernel
@@ -543,7 +546,7 @@ void launch_step_chunk(sb2_model* m, const StepTarget& t, int64_t s0, int chunk,
     const int64_t n = m->n;
     const unsigned ne = unsigned(t.members);
     const bool gsk = m->stack == SB2_PT_GS_K;
-    const int collect = t.series ? m->collect_bits : 0;
+    const int collect = t.series ? m->collect_bits : (t.q ? SB2_COLLECT_DISCHARGE : 0);
     // UPAR kernels: no catchment override and no member table -> every cell reads the region parameter set from the constant bank
     const bool upar = m->catch_param.empty() && !t.ptgsk_members && !t.hbv_members && !t.hps_members;
     // snow / response or run kernel in time slices handed out by ticket (see the kernels); the tickets are read only when split
@@ -568,6 +571,9 @@ void launch_step_chunk(sb2_model* m, const StepTarget& t, int64_t s0, int chunk,
             for (size_t r = 0; r < std::size(a.resp); ++r) a.resp[r] = m->d_resp[r].p;
             for (size_t s = 0; s < std::size(a.st); ++s) a.st[s] = m->d_st[s].p;
             a.out_first_step = m->out_first;
+        } else if (t.q) {
+            a.resp[0] = t.q; a.resp[1] = t.charge;
+            a.out_first_step = s0;
         }
         a.collect_end_state = collect_end_state ? 1 : 0;
         a.slot = m->d_slot.p; a.partial = t.partial; a.n_slots = m->n_slots; a.error_flag = m->d_error_flag.p;
@@ -582,7 +588,7 @@ void launch_step_chunk(sb2_model* m, const StepTarget& t, int64_t s0, int chunk,
         a.inv_dt_us = make_inv_divisor(a.dt_us);
         a.par0 = make_ptgsk_param(m->region_param.data(), param_dt(m));
         a.day_sec_of_year = m->d_doy_soy.p;
-        a.ens_params = t.ptgsk_members; a.ens_state_stride = t.state_stride; a.ens_partial_stride = t.partial_stride;
+        a.ens_params = t.ptgsk_members; a.ens_state_stride = t.state_stride; a.ens_partial_stride = t.partial_stride; a.ens_resp_stride = t.resp_stride;
         for (int k = 0; k < 5; ++k) a.scr[k] = t.scr[k].p;
         a.ens_scr_stride = t.scr_stride;
         // phase pipeline: forcing terms -> snow -> response (sb2_ptgsk.cuh)
@@ -628,7 +634,7 @@ void launch_step_chunk(sb2_model* m, const StepTarget& t, int64_t s0, int chunk,
             a.params = m->d_hps_params.p;
             a.bb0 = 0.98 * 5.670373e-8 * sb_pow4(273.15);  // calculator::BB0 (hbv_physical_snow.h:208)
             a.inv_dt_seconds = make_inv_divisor(a.dt_seconds);
-            a.ens_params = t.hps_members; a.ens_state_stride = t.state_stride; a.ens_partial_stride = t.partial_stride;
+            a.ens_params = t.hps_members; a.ens_state_stride = t.state_stride; a.ens_partial_stride = t.partial_stride; a.ens_resp_stride = t.resp_stride;
             a.collect = collect & 15;
             if (t.hps_members) pthpsk_run_kernel<true><<<grid, SB2_BLOCK, SB2_MTAB_BYTES, m->stream>>>(a);
             else pthpsk_run_kernel<false><<<grid, SB2_BLOCK, SB2_MTAB_BYTES, m->stream>>>(a);
@@ -639,7 +645,7 @@ void launch_step_chunk(sb2_model* m, const StepTarget& t, int64_t s0, int chunk,
             a.inv_dt_hours = make_inv_divisor(a.dt_hours);
             a.step_in_days = a.dt_seconds / 86400.0;
             a.par0 = make_hbv_param(m->stack == SB2_HBV_STACK, m->region_param.data());
-            a.ens_params = t.hbv_members; a.ens_state_stride = t.state_stride; a.ens_partial_stride = t.partial_stride;
+            a.ens_params = t.hbv_members; a.ens_state_stride = t.state_stride; a.ens_partial_stride = t.partial_stride; a.ens_resp_stride = t.resp_stride;
             a.collect = collect & 15;
             if (m->stack == SB2_PT_HS_K) {
                 if (upar) hbv_run_kernel<false, true><<<grid, SB2_BLOCK, SB2_MTAB_BYTES, m->stream>>>(a);
@@ -1183,20 +1189,54 @@ double evaluate_goal_single(sb2_model* m) {
     return combine_goal(m, partial.data());
 }
 
+// the longest cell unit hydrograph (routing.h:119-123) any of the n_sets parameter sets gives a routed cell, cells under a catchment
+// override with the override's velocity: a routed batch carries this minus one rows of cell discharge from one chunk of steps to the
+// next.  uhg_steps is monotone in the distance, so for a member's own cells the shortest and the longest distance decide it.
+int64_t batch_cell_uhg_max_len(const sb2_model* m, int64_t n_sets, const double* P) {
+    const int off = kStacks[m->stack].routing_velocity;
+    auto len = [&](double distance, double velocity) { return std::max<int64_t>(1, host::uhg_steps(distance, velocity, m->dt)); };
+    int64_t max_len = 1;
+    double dmin = INFINITY, dmax = -INFINITY;
+    for (int64_t i = 0; i < m->n; ++i) {
+        if (m->geo[i].routing_id <= 0) continue;
+        auto f = m->catch_param.find(m->geo[i].catchment_id);
+        if (f != m->catch_param.end()) max_len = std::max(max_len, len(m->geo[i].routing_distance, f->second[off]));
+        else { dmin = std::min(dmin, m->geo[i].routing_distance); dmax = std::max(dmax, m->geo[i].routing_distance); }
+    }
+    if (dmin <= dmax)
+        for (int64_t e = 0; e < n_sets; ++e) {
+            const double v = P[e * m->n_param + off];
+            max_len = std::max(max_len, std::max(len(dmin, v), len(dmax, v)));
+        }
+    return max_len;
+}
+
 // ensemble of region-parameter sets for pt_gs_k, pt_hs_k, hbv_stack and pt_hps_k: member e = one grid layer of the step kernels
-// run_cells launches, stepping its own copy of the state; the model's parameters, state and catchment series are left as they are
+// run_cells launches, stepping its own copy of the state; the model's parameters, state, catchment series and river flows are left
+// as they are.  A ROUTED_DISCHARGE target routes every member as sb2_river_flows routes a run: each chunk's cell discharge goes through
+// the local-inflow kernel with the previous chunks' last H rows in front of it (as run_windowed does per window), then the river
+// network is routed level by level, all members in one launch each, with the member's own cell unit hydrographs.
 void goal_batch(sb2_model* m, int64_t n_sets, const double* P, double* goals) {
     sync_parameters(m);
     sync_filter(m);
     const bool gsk = m->stack == SB2_PT_GS_K;
     const int64_t n = m->n, T = m->T, nc = m->n_catch();
     const size_t state_sz = size_t(m->n_state) * n;
-    // members per pass from a ~12 GB budget: state + catchment series (discharge, charge)
-    const size_t per_member = state_sz * 8 + size_t(T) * nc * 16;
+    bool routed = false;
+    for (auto& tp : m->targets) routed = routed || tp->property == SB2_TARGET_ROUTED_DISCHARGE;
+    if (routed && m->rivers.empty()) throw Error("routing: the river network is empty");
+    const int64_t n_riv = int64_t(m->rivers.size() / 6);
+    const int64_t H = routed ? batch_cell_uhg_max_len(m, n_sets, P) - 1 : 0;
+    // members per pass from a ~12 GB budget: state + catchment series (discharge, charge); with a routed target also the river series
+    // (local inflow, upstream inflow, output: [n_riv][T] each) and the H history rows of the two cell-discharge buffers below
+    size_t per_member = state_sz * 8 + size_t(T) * nc * 16;
+    if (routed) per_member += size_t(3) * n_riv * T * 8 + size_t(2) * H * n * 8;
     const int64_t E = std::max<int64_t>(1, std::min<int64_t>(std::min<int64_t>(n_sets, 65535), int64_t((12ULL << 30) / per_member)));
-    // steps per pass: ~1 GB of per-slot partial sums; pt_gs_k also ~4 GB of phase-pipeline scratch (five [E][ps][n] arrays)
+    // steps per pass: ~1 GB of per-slot partial sums; pt_gs_k also ~4 GB of phase-pipeline scratch (five [E][ps][n] arrays); a routed
+    // target ~2 GB for the step rows of the two cell-discharge buffers ([E][H + ps][n] each)
     int64_t ps = std::min<int64_t>(T, int64_t((1ULL << 30) / (size_t(E) * m->n_slots * 16)));
     if (gsk) ps = std::min<int64_t>(ps, std::max<int64_t>(8, int64_t((4ULL << 30) / (size_t(E) * n * 40))));
+    if (routed) ps = std::min<int64_t>(ps, int64_t((2ULL << 30) / (size_t(E) * n * 16)));
     ps = std::max<int64_t>(1, ps);
     DevArray<double> d_state, d_partial, d_cq, d_cc, d_out, d_scr[5];
     if (gsk)
@@ -1212,13 +1252,33 @@ void goal_batch(sb2_model* m, int64_t n_sets, const double* P, double* goals) {
     d_cq.resize(size_t(E) * T * nc);
     d_cc.resize(size_t(E) * T * nc);
     d_out.resize(size_t(E) * m->targets.size());
+    // routed: a pair of [E][H + ps][n] cell-discharge buffers.  A chunk's steps write buffer `cur` from row H on, after the history
+    // rows; its last H rows are then copied to the front of the other buffer, which the next chunk writes.  The members' cell charge,
+    // needed by nothing here, goes to the other buffer's step rows, which the next chunk overwrites.  Cells outside the calculation
+    // filter are never written and read NaN, as in the NaN-initialised series of run_cells.
+    const int64_t qrows = H + ps;
+    DevArray<double> d_qbuf[2], d_rlocal, d_rup, d_rout;
+    if (routed) {
+        for (auto& b : d_qbuf) { b.resize(size_t(E) * qrows * n); fill_nan(m, b.p, E * qrows * n); }
+        d_rlocal.resize(size_t(E) * n_riv * T);
+        d_rup.resize(size_t(E) * n_riv * T);
+        d_rout.resize(size_t(E) * n_riv * T);
+    }
     std::vector<GoalTarget> gt;
     build_goal_targets(m, gt, d_cq.p, d_cc.p, T * nc);
+    std::vector<int64_t> riv_ix(gt.size(), -1);  // a routed target's river: the position in the network table, as in the plan
+    for (size_t k = 0; k < gt.size(); ++k) {
+        if (m->targets[k]->property != SB2_TARGET_ROUTED_DISCHARGE) continue;
+        for (int64_t r = 0; r < n_riv; ++r)
+            if (int64_t(m->rivers[6 * r]) == m->targets[k]->river_id) riv_ix[k] = r;
+        if (riv_ix[k] >= 0) { gt[k].series = d_rout.p + riv_ix[k] * T; gt[k].ens_stride = n_riv * T; }
+    }
     d_gt.upload(gt, m->stream);
     StepTarget t;
     t.state = d_state.p; t.partial = d_partial.p; t.cq = d_cq.p; t.cc = d_cc.p; t.scr = d_scr;
     t.state_stride = int64_t(state_sz); t.partial_stride = ps * m->n_slots * 2; t.catch_stride = T * nc; t.scr_stride = ps * n;
     t.tickets = d_tickets.p;
+    t.resp_stride = qrows * n;
     std::vector<double> partial(size_t(E) * gt.size());
     for (int64_t e0 = 0; e0 < n_sets; e0 += E) {
         const int64_t ne = std::min<int64_t>(E, n_sets - e0);
@@ -1228,9 +1288,45 @@ void goal_batch(sb2_model* m, int64_t n_sets, const double* P, double* goals) {
         else if (m->stack == SB2_PT_HPS_K) { upload_params(m, sets, d_hps_par); t.hps_members = d_hps_par.p; }
         else { upload_params(m, sets, d_hbv_par); t.hbv_members = d_hbv_par.p; }
         t.members = int(ne);
+        std::unique_ptr<RoutingPlan> route;
+        if (routed) {  // the cells' routing triples as ensure_routing_plan takes them, member by member
+            const int off = kStacks[m->stack].routing_velocity;
+            std::vector<double> cell_routing(size_t(ne) * n * 5);
+            for (int64_t e = 0; e < ne; ++e)
+                for (int64_t i = 0; i < n; ++i) {
+                    auto f = m->catch_param.find(m->geo[i].catchment_id);
+                    const double* p = f != m->catch_param.end() ? f->second.data() : sets[size_t(e)];
+                    double* cr = &cell_routing[(size_t(e) * n + i) * 5];
+                    cr[0] = double(m->geo[i].routing_id); cr[1] = m->geo[i].routing_distance;
+                    cr[2] = p[off]; cr[3] = p[off + 1]; cr[4] = p[off + 2];
+                }
+            route = build_routing_plan(m->rivers, cell_routing, n, m->dt, m->stream);
+            for (size_t k = 0; k < gt.size(); ++k)  // sb2_river_flows' checks, in its order
+                if (m->targets[k]->property == SB2_TARGET_ROUTED_DISCHARGE && riv_ix[k] < 0)
+                    throw Error("river network: river id " + std::to_string(m->targets[k]->river_id) + " not found");
+            if (!(m->collect_bits & SB2_COLLECT_DISCHARGE))
+                throw Error("river flows need avg_discharge over the whole time axis (run_cells with a discharge collector, or run_windowed with the river network set)");
+            if (route->cell_max_len - 1 > H) throw Error("routing: cell unit hydrograph longer than the batch's history");
+        }
         for (int64_t e = 0; e < ne; ++e)  // reset_states(): every member starts from the initial state (:833)
             CUDA_OK(cudaMemcpyAsync(d_state.p + e * state_sz, m->d_initial_state.p, state_sz * sizeof(double), cudaMemcpyDeviceToDevice, m->stream));
-        for (int64_t done = 0; done < T; done += ps) launch_step_chunk(m, t, done, int(std::min<int64_t>(ps, T - done)), false);
+        int cur = 0;
+        for (int64_t done = 0; done < T; done += ps) {
+            const int chunk = int(std::min<int64_t>(ps, T - done));
+            if (routed) { t.q = d_qbuf[cur].p + H * n; t.charge = d_qbuf[cur ^ 1].p + H * n; }
+            launch_step_chunk(m, t, done, chunk, false);
+            if (routed) {
+                routing_local_inflow(*route, t.q, n, chunk, H, done, T, d_rlocal.p, m->stream, &m->launches, int(ne), qrows * n);
+                if (H > 0 && done + chunk < T) {
+                    route_history_kernel<<<dim3((unsigned)std::min<int64_t>(grid_for(H * n, 256), 1024), (unsigned)ne), 256, 0, m->stream>>>(
+                        d_qbuf[cur].p, d_qbuf[cur ^ 1].p, qrows * n, int64_t(chunk) * n, H * n);
+                    CUDA_OK(cudaGetLastError());
+                    ++m->launches;
+                }
+                cur ^= 1;
+            }
+        }
+        if (routed) routing_network(*route, T, d_rlocal.p, d_rup.p, d_rout.p, m->stream, &m->launches, int(ne));
         goal_kernel<<<dim3((unsigned)gt.size(), (unsigned)ne), 256, 0, m->stream>>>(d_gt.p, int(gt.size()), d_out.p);
         CUDA_OK(cudaGetLastError());
         ++m->launches;
@@ -2369,7 +2465,9 @@ int sb2_calculate_goal_function_batch(sb2_model* m, int64_t n_sets, const double
         // pt_ss_k is not among them: its batch goes one set at a time
         bool device_batch = m->stack == SB2_PT_GS_K || m->stack == SB2_PT_HS_K || m->stack == SB2_HBV_STACK || m->stack == SB2_PT_HPS_K;
         for (auto& t : m->targets)
-            if ((t->property != SB2_TARGET_DISCHARGE && t->property != SB2_TARGET_CELL_CHARGE) || !t->aligned) device_batch = false;
+            if ((t->property != SB2_TARGET_DISCHARGE && t->property != SB2_TARGET_CELL_CHARGE && t->property != SB2_TARGET_ROUTED_DISCHARGE) ||
+                !t->aligned)
+                device_batch = false;
         if (device_batch) {
             if (!m->has_initial) throw Error("Initial state not yet established or set");
             if (!m->d_forcing[0].p || m->forcing_first != 0 || m->forcing_rows != m->T)

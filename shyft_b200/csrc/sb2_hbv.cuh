@@ -95,6 +95,7 @@ struct HbvRunArgs {
     // [members] and progress [members][cell groups].  Last in the struct so that the fields above keep their constant-bank offsets.
     const HbvParam* __restrict__ ens_params;  // null = no ensemble
     int64_t ens_state_stride, ens_partial_stride;
+    int64_t ens_resp_stride;  // elements between two members' avg_discharge / charge rows (a batch that routes each member)
 };
 
 // hbv_snow_common::integrate(f, x, n, a = x[0], b, f_b_is_zero), core/hbv_snow_common.h:14-43
@@ -270,6 +271,8 @@ __global__ void __launch_bounds__(128, (HBV_STACK ? SB2_HBV_MINBLOCKS_S : SB2_HB
     // __ldcg: the state may have been written by the previous time slice on another SM a moment ago -- read it from L2
     // this member's state rows start at a.state + so, its partial sums at a.partial + ens * a.ens_partial_stride (both 0 without an ensemble)
     const int64_t so = (int64_t)ens * a.ens_state_stride;
+    double* __restrict__ const resp_q = a.resp[0] + (int64_t)ens * a.ens_resp_stride;  // this member's avg_discharge / charge rows
+    double* __restrict__ const resp_c = a.resp[1] + (int64_t)ens * a.ens_resp_stride;
     double swe = __ldcg(a.state + so + 0 * n + cc), sca = __ldcg(a.state + so + 1 * n + cc);
     double sp[HBV_NB], sw[HBV_NB];
 #pragma unroll
@@ -362,7 +365,7 @@ __global__ void __launch_bounds__(128, (HBV_STACK ? SB2_HBV_MINBLOCKS_S : SB2_HB
                 +mmh_to_m3s(prec, cell_area_m2) - mmh_to_m3s(ae, cell_area_m2) + gm_melt_m3s - mmh_to_m3s(total_discharge, cell_area_m2);
             out_q = mmh_to_m3s(total_discharge, cell_area_m2);
             out_charge = charge_m3s;
-            if (a.collect & 1) { a.resp[0][orow] = out_q; a.resp[1][orow] = charge_m3s; }
+            if (a.collect & 1) { resp_q[orow] = out_q; resp_c[orow] = charge_m3s; }
             if (a.collect & 2) {
                 // hbv_stack never assigns response.snow.snow_state (hbv_stack.h:324-357) -> its collectors record 0
                 a.resp[2][orow] = HBV_STACK ? 0.0 : sca;

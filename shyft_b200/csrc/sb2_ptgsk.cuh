@@ -103,6 +103,9 @@ struct PtgskRunArgs {
     int unit_steps;
     int* __restrict__ tickets;
     int* __restrict__ progress;
+    // elements between two members' avg_discharge / charge rows (a calibration batch that routes each member's cell discharge); last in
+    // the struct so that the fields above keep their constant-bank offsets
+    int64_t ens_resp_stride;
 };
 enum : int { SCR_POT = 0, SCR_LW = 1, SCR_TADD = 2, SCR_OUTFLOW = 3, SCR_SCA = 4 };
 
@@ -992,6 +995,8 @@ __global__ void __launch_bounds__(SB2_BLOCK_C, SB2_MINBLOCKS_C) ptgsk_response_k
     const double* __restrict__ s_pot = a.scr[SCR_POT] + (int64_t)ens * a.ens_scr_stride;
     const double* __restrict__ s_outflow = a.scr[SCR_OUTFLOW] + (int64_t)ens * a.ens_scr_stride;
     const double* __restrict__ s_sca = a.scr[SCR_SCA] + (int64_t)ens * a.ens_scr_stride;
+    double* __restrict__ const resp_q = a.resp[0] + (int64_t)ens * a.ens_resp_stride;  // this member's avg_discharge / charge rows
+    double* __restrict__ const resp_c = a.resp[1] + (int64_t)ens * a.ens_resp_stride;
     // Per-cell constants of the step (run_pt_gs_k prologue, pt_gs_k.h:347-357) live in shared memory, one column per thread: each is
     // read once or twice per step, and twelve doubles less in registers is one more resident warp per scheduler for the ODE solver.
     __shared__ double cst[14][SB2_BLOCK_C];
@@ -1077,7 +1082,7 @@ __global__ void __launch_bounds__(SB2_BLOCK_C, SB2_MINBLOCKS_C) ptgsk_response_k
                 kq = kq_new;
                 out_q = mmh_to_m3s(total_discharge, cell_area_m2);
                 out_charge = charge_m3s;
-                if (COLLECT & 1) { a.resp[0][orow] = out_q; a.resp[1][orow] = charge_m3s; }
+                if (COLLECT & 1) { resp_q[orow] = out_q; resp_c[orow] = charge_m3s; }
                 if (COLLECT & 4) {
                     a.resp[5][orow] = gm_melt_m3s;
                     a.resp[6][orow] = ae;

@@ -87,6 +87,7 @@ struct HpsRunArgs {
     // constant-bank offsets.
     const HpsParam* __restrict__ ens_params;  // null = no ensemble
     int64_t ens_state_stride, ens_partial_stride;
+    int64_t ens_resp_stride;  // elements between two members' avg_discharge / charge rows (a batch that routes each member)
 };
 
 struct HpsState { double sp[HBV_NB], sw[HBV_NB], albedo[HBV_NB], iso[HBV_NB], surface_heat, swe, sca; };
@@ -307,6 +308,8 @@ __global__ void __launch_bounds__(128, SB2_HPS_MINBLOCKS) pthpsk_run_kernel(cons
 
     // this member's state rows start at a.state + so, its partial sums at a.partial + ens * a.ens_partial_stride (both 0 without an ensemble)
     const int64_t so = (int64_t)ens * a.ens_state_stride;
+    double* __restrict__ const resp_q = a.resp[0] + (int64_t)ens * a.ens_resp_stride;  // this member's avg_discharge / charge rows
+    double* __restrict__ const resp_c = a.resp[1] + (int64_t)ens * a.ens_resp_stride;
     HpsState hs;
 #pragma unroll
     for (int i = 0; i < HBV_NB; ++i) {
@@ -370,7 +373,7 @@ __global__ void __launch_bounds__(128, SB2_HPS_MINBLOCKS) pthpsk_run_kernel(cons
                 +mmh_to_m3s(prec, cell_area_m2) - mmh_to_m3s(ae, cell_area_m2) + gm_melt_m3s - mmh_to_m3s(total_discharge, cell_area_m2);
             out_q = mmh_to_m3s(total_discharge, cell_area_m2);
             out_charge = charge_m3s;
-            if (a.collect & 1) { a.resp[0][orow] = out_q; a.resp[1][orow] = charge_m3s; }
+            if (a.collect & 1) { resp_q[orow] = out_q; resp_c[orow] = charge_m3s; }
             if (a.collect & 2) { a.resp[2][orow] = r_sca; a.resp[3][orow] = r_storage * snow_storage_fraction; }
             if (a.collect & 4) {
                 a.resp[4][orow] = snow_outflow * snow_storage_fraction;  // hps_outflow: mm/h, as the reference collects it

@@ -28,15 +28,21 @@ constexpr int ROUTE_TT = 64;      // time steps per block
 // window); rows further back are before the start of the axis or not needed and read as zero (USE_ZERO, time_series.h:966-975).
 // uhg_w rows are w_stride apart; depth (>= every cell UHG length, <= w_stride) is the tile's history depth: the river UHGs that
 // share the table may be longer, but they never go through this tile.
-// grid (time tiles, rivers); dynamic smem: (ROUTE_TT + depth - 1) * ROUTE_CELLS doubles
+// blockIdx.z = member of a calibration batch: its q block, cell UHG ids and local inflow lie at z times q_stride, uhg_stride and
+// local_stride (0, 0, 0 with one member).
+// grid (time tiles, rivers, members); dynamic smem: (ROUTE_TT + depth - 1) * ROUTE_CELLS doubles
 __global__ void __launch_bounds__(ROUTE_CELLS) route_local_inflow_kernel(const double* __restrict__ q, int64_t n_cells, int64_t n_rows, int64_t hist,
                                                                          int64_t g0, int64_t T, const int32_t* __restrict__ riv_ptr,
                                                                          const int32_t* __restrict__ riv_cells,
                                                                          const int32_t* __restrict__ cell_uhg_id /* per gathered cell */,
                                                                          const int32_t* __restrict__ uhg_len, const double* __restrict__ uhg_w,
-                                                                         int w_stride, int depth, double* __restrict__ local /* [n_riv][T] */) {
+                                                                         int w_stride, int depth, double* __restrict__ local /* [n_riv][T] */,
+                                                                         int64_t q_stride, int64_t uhg_stride, int64_t local_stride) {
     extern __shared__ double sq[];  // [(ROUTE_TT + depth - 1)][ROUTE_CELLS]
     __shared__ double acc[ROUTE_TT];
+    q += blockIdx.z * q_stride;
+    cell_uhg_id += blockIdx.z * uhg_stride;
+    local += blockIdx.z * local_stride;
     const int r = blockIdx.y;
     const int64_t t0 = (int64_t)blockIdx.x * ROUTE_TT;
     const int nt = int(min((int64_t)ROUTE_TT, n_rows - t0));
@@ -76,13 +82,17 @@ __global__ void __launch_bounds__(ROUTE_CELLS) route_local_inflow_kernel(const d
 }
 
 // one network level: upstream[r][t] = sum of output[u][t] over upstream rivers u; output[r] = (local[r] + upstream[r]) (*) uhg_r
-// grid (time tiles, rivers of this level); dynamic smem: (ROUTE_TT + max_len - 1) doubles
+// blockIdx.z = member of a calibration batch: its local / upstream / output series lie at z times stride (0 with one member)
+// grid (time tiles, rivers of this level, members); dynamic smem: (ROUTE_TT + max_len - 1) doubles
 __global__ void __launch_bounds__(ROUTE_TT) route_river_level_kernel(const int32_t* __restrict__ level_rivers, const int32_t* __restrict__ up_ptr,
                                                                      const int32_t* __restrict__ up_idx, const int32_t* __restrict__ riv_uhg_id,
                                                                      const int32_t* __restrict__ uhg_len, const double* __restrict__ uhg_w, int max_len,
                                                                      int64_t T, const double* __restrict__ local, double* __restrict__ upstream,
-                                                                     double* __restrict__ output) {
+                                                                     double* __restrict__ output, int64_t stride) {
     extern __shared__ double sin_[];  // input sum rows [t0 - (max_len-1), t0 + ROUTE_TT)
+    local += blockIdx.z * stride;
+    upstream += blockIdx.z * stride;
+    output += blockIdx.z * stride;
     const int r = level_rivers[blockIdx.y];
     const int64_t t0 = (int64_t)blockIdx.x * ROUTE_TT;
     const int rows = ROUTE_TT + max_len - 1;
@@ -107,6 +117,14 @@ __global__ void __launch_bounds__(ROUTE_TT) route_river_level_kernel(const int32
         for (int j = 0; j < len; ++j) v += w[j] * sin_[threadIdx.x + max_len - 1 - j];
         output[(int64_t)r * T + t] = v;
     }
+}
+
+// the last `rows` rows of each member's [rows_src][n_cells] block become the first rows of its block in the other buffer of a pair:
+// dst[e][i] = src[e][i + shift] for i < rows * n_cells (the two never overlap, whatever rows and shift are).  grid (x, members)
+__global__ void route_history_kernel(const double* __restrict__ src, double* __restrict__ dst, int64_t stride, int64_t shift, int64_t count) {
+    src += blockIdx.y * stride + shift;
+    dst += blockIdx.y * stride;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (int64_t)gridDim.x * blockDim.x) dst[i] = src[i];
 }
 
 namespace routing_host {
@@ -144,10 +162,14 @@ struct UhgTable {
 }  // namespace routing_host
 
 // Everything about a river network that does not depend on the simulated discharge: cells gathered per river, the
-// unit-hydrograph table, upstream lists and levels.  cell_routing [n_cells][5] = routing id, distance, velocity, alpha,
-// beta (velocity/alpha/beta from the cell's parameter set); rivers [n][6] = id, downstream id, distance, velocity, alpha, beta.
+// unit-hydrograph table, upstream lists and levels.  cell_routing [members][n_cells][5] = routing id, distance, velocity, alpha,
+// beta (velocity/alpha/beta from the cell's parameter set; one member for a model's own run, one per parameter set of a
+// calibration batch, the routing id and distance the same in every member); rivers [n][6] = id, downstream id, distance,
+// velocity, alpha, beta.  The members share one table (equal (steps, alpha, beta) are one entry, so a member's weights are the
+// ones its own single-member plan has); d_cuhg is [members][n_gathered], max_len / cell_max_len the maxima over all members.
 struct RoutingPlan {
-    int n_riv = 0, max_len = 1, cell_max_len = 1, n_levels = 0;
+    int n_riv = 0, max_len = 1, cell_max_len = 1, n_levels = 0, members = 1;
+    int64_t n_gathered = 0;
     std::map<int64_t, int> ix_of_rid;
     std::vector<int> level_begin;
     routing_host::DevBuf b_ptr, b_cells, b_cuhg, b_len, b_w, b_ruhg, b_upp, b_upi, b_lvl;
@@ -163,26 +185,34 @@ inline std::unique_ptr<RoutingPlan> build_routing_plan(const std::vector<double>
     const int n_riv = int(rivers.size() / 6);
     if (n_riv == 0) throw std::runtime_error("routing: the river network is empty");
     pl->n_riv = n_riv;
+    const int members = int(cell_routing.size() / (5 * std::max<int64_t>(1, n_cells)));
+    pl->members = std::max(1, members);
     for (int i = 0; i < n_riv; ++i) pl->ix_of_rid[int64_t(rivers[6 * i])] = i;
     UhgTable tab;
     std::vector<std::vector<int32_t>> cells_of(n_riv);
-    std::vector<int32_t> cell_uhg(n_cells, 0);
-    for (int64_t c = 0; c < n_cells; ++c) {
-        const int64_t id = int64_t(cell_routing[5 * c]);
-        if (id <= 0) continue;
-        auto f = pl->ix_of_rid.find(id);
-        if (f == pl->ix_of_rid.end()) throw std::runtime_error("river network: river id " + std::to_string(id) + " not found");
-        cells_of[f->second].push_back(int32_t(c));
-        cell_uhg[c] = tab.id_of(host::uhg_steps(cell_routing[5 * c + 1], cell_routing[5 * c + 2], dt_us), cell_routing[5 * c + 3],
-                                cell_routing[5 * c + 4]);
+    std::vector<int32_t> cell_uhg(size_t(pl->members) * n_cells, 0);
+    for (int e = 0; e < members; ++e) {
+        const double* cr = cell_routing.data() + size_t(e) * n_cells * 5;
+        for (int64_t c = 0; c < n_cells; ++c) {
+            const int64_t id = int64_t(cr[5 * c]);
+            if (id <= 0) continue;
+            auto f = pl->ix_of_rid.find(id);
+            if (f == pl->ix_of_rid.end()) throw std::runtime_error("river network: river id " + std::to_string(id) + " not found");
+            if (e == 0) cells_of[f->second].push_back(int32_t(c));
+            cell_uhg[size_t(e) * n_cells + c] = tab.id_of(host::uhg_steps(cr[5 * c + 1], cr[5 * c + 2], dt_us), cr[5 * c + 3], cr[5 * c + 4]);
+        }
     }
     for (auto& w : tab.w) pl->cell_max_len = std::max(pl->cell_max_len, int(w.size()));
-    std::vector<int32_t> riv_ptr(n_riv + 1, 0), riv_cells, gathered_uhg, riv_uhg(n_riv);
+    std::vector<int32_t> riv_ptr(n_riv + 1, 0), riv_cells, riv_uhg(n_riv);
     for (int r = 0; r < n_riv; ++r) {
-        for (auto c : cells_of[r]) { riv_cells.push_back(c); gathered_uhg.push_back(cell_uhg[c]); }
+        for (auto c : cells_of[r]) riv_cells.push_back(c);
         riv_ptr[r + 1] = int32_t(riv_cells.size());
         riv_uhg[r] = tab.id_of(host::uhg_steps(rivers[6 * r + 2], rivers[6 * r + 3], dt_us), rivers[6 * r + 4], rivers[6 * r + 5]);
     }
+    pl->n_gathered = int64_t(riv_cells.size());
+    std::vector<int32_t> gathered_uhg(size_t(pl->members) * riv_cells.size());
+    for (int e = 0; e < pl->members; ++e)
+        for (size_t k = 0; k < riv_cells.size(); ++k) gathered_uhg[e * riv_cells.size() + k] = cell_uhg[size_t(e) * n_cells + riv_cells[k]];
     for (auto& w : tab.w) pl->max_len = std::max(pl->max_len, int(w.size()));
     // the shared-memory tiles: cell discharge of the local-inflow kernel, input sum of the river-level kernel
     if (size_t(ROUTE_TT + pl->cell_max_len - 1) * ROUTE_CELLS * sizeof(double) > 200 * 1024)
@@ -239,28 +269,34 @@ inline std::unique_ptr<RoutingPlan> build_routing_plan(const std::vector<double>
     return pl;
 }
 
-// cell -> river: the local inflow of every river over block rows [0, n_rows) = global steps [g0, g0 + n_rows)
+// cell -> river: the local inflow of every river over block rows [0, n_rows) = global steps [g0, g0 + n_rows); with members > 1,
+// member e's block row 0 is at d_q_row0 + e * q_stride and its local inflow [n_riv][T] at d_local + e * n_riv * T
 inline void routing_local_inflow(const RoutingPlan& pl, const double* d_q_row0, int64_t n_cells, int64_t n_rows, int64_t hist, int64_t g0, int64_t T,
-                                 double* d_local, cudaStream_t stream, int64_t* launches) {
+                                 double* d_local, cudaStream_t stream, int64_t* launches, int members = 1, int64_t q_stride = 0) {
+    if (members > pl.members) throw std::runtime_error("routing: more members than the plan has unit hydrographs for");
     const size_t smem = size_t(ROUTE_TT + pl.cell_max_len - 1) * ROUTE_CELLS * sizeof(double);
     if (smem > 48 * 1024) cudaFuncSetAttribute(route_local_inflow_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
     const unsigned tiles = unsigned((n_rows + ROUTE_TT - 1) / ROUTE_TT);
-    route_local_inflow_kernel<<<dim3(tiles, pl.n_riv), ROUTE_CELLS, smem, stream>>>(d_q_row0, n_cells, n_rows, hist, g0, T, pl.d_ptr, pl.d_cells, pl.d_cuhg,
-                                                                                  pl.d_len, pl.d_w, pl.max_len, pl.cell_max_len, d_local);
+    route_local_inflow_kernel<<<dim3(tiles, pl.n_riv, members), ROUTE_CELLS, smem, stream>>>(
+        d_q_row0, n_cells, n_rows, hist, g0, T, pl.d_ptr, pl.d_cells, pl.d_cuhg, pl.d_len, pl.d_w, pl.max_len, pl.cell_max_len, d_local,
+        members > 1 ? q_stride : 0, members > 1 ? pl.n_gathered : 0, members > 1 ? int64_t(pl.n_riv) * T : 0);
     ++*launches;
     if (cudaGetLastError() != cudaSuccess) throw std::runtime_error("routing: kernel launch failed");
 }
 
-// river network, leaves first: upstream inflow and routed output of every river over the whole axis
-inline void routing_network(const RoutingPlan& pl, int64_t T, const double* d_local, double* d_up, double* d_out, cudaStream_t stream, int64_t* launches) {
-    cudaMemsetAsync(d_up, 0, size_t(pl.n_riv) * T * sizeof(double), stream);
+// river network, leaves first: upstream inflow and routed output of every river over the whole axis; d_local, d_up and d_out hold
+// [members][n_riv][T]
+inline void routing_network(const RoutingPlan& pl, int64_t T, const double* d_local, double* d_up, double* d_out, cudaStream_t stream, int64_t* launches,
+                            int members = 1) {
+    cudaMemsetAsync(d_up, 0, size_t(members) * pl.n_riv * T * sizeof(double), stream);
     const unsigned tiles = unsigned((T + ROUTE_TT - 1) / ROUTE_TT);
     const size_t smem = size_t(ROUTE_TT + pl.max_len - 1) * sizeof(double);
     if (smem > 48 * 1024) cudaFuncSetAttribute(route_river_level_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
     for (int lv = 0; lv < pl.n_levels; ++lv) {
         const int cnt = pl.level_begin[lv + 1] - pl.level_begin[lv];
-        route_river_level_kernel<<<dim3(tiles, cnt), ROUTE_TT, smem, stream>>>(pl.d_order + pl.level_begin[lv], pl.d_upp, pl.d_upi, pl.d_ruhg, pl.d_len,
-                                                                              pl.d_w, pl.max_len, T, d_local, d_up, d_out);
+        route_river_level_kernel<<<dim3(tiles, cnt, members), ROUTE_TT, smem, stream>>>(pl.d_order + pl.level_begin[lv], pl.d_upp, pl.d_upi, pl.d_ruhg,
+                                                                                       pl.d_len, pl.d_w, pl.max_len, T, d_local, d_up, d_out,
+                                                                                       int64_t(pl.n_riv) * T);
         ++*launches;
     }
     if (cudaGetLastError() != cudaSuccess) throw std::runtime_error("routing: kernel launch failed");

@@ -113,6 +113,10 @@ void bind_model(py::module_& m, const char* name, int collect_bits, const char* 
                  return out;
              },
              py::arg("series"))
+        .def("set_river_network",
+             [](M& self, const darray& rivers) { self.set_river_network(flat(rivers)); }, py::arg("rivers"),
+             "rivers [n][6] = id, downstream id, downstream distance, uhg velocity, alpha, beta (core/routing.h:98-123)")
+        .def("river_output_flow_m3s", &M::river_output_flow_m3s, py::arg("river_id"))
         .def("statistics", &M::statistics, py::arg("kind"), py::arg("series"), py::arg("indexes"), py::arg("op"), py::arg("scope") = int(SB2_SCOPE_CATCHMENT_IX))
         .def("statistics_value", &M::statistics_value, py::arg("kind"), py::arg("series"), py::arg("indexes"), py::arg("ith_timestep"), py::arg("op"),
              py::arg("scope") = int(SB2_SCOPE_CATCHMENT_IX));

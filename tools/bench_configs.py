@@ -71,16 +71,25 @@ if 5 in which:  # calibration ensemble: parameter sets x 10k-cell catchment x 3 
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     # SB2_C5_STACK: pt_gs_k (default), pt_hs_k, hbv_stack or pt_hps_k -- the stacks whose batch runs as grid layers on the device
     stack = os.environ.get("SB2_C5_STACK", "pt_gs_k")
+    # SB2_C5_TARGET=routed: the target is the routed outflow of river 8, the outlet of a chain of eight (synthetic.river_chain over the
+    # 10 catchments), and every set also draws its own routing velocity
+    routed = os.environ.get("SB2_C5_TARGET", "discharge") == "routed"
     n, T, sets = 10000, 26280, int(os.environ.get("SB2_C5_SETS", "256"))
-    geo, ta, env = synthetic.make_region(n, T, 64, config_index=4)
+    geo, ta, env = synthetic.make_region(n, T, 64, config_index=4, with_routing=routed)
     cls, par, sid = {"pt_gs_k": (sb.PTGSKOptModel, PTGSK, 0), "pt_hs_k": (sb.PTHSKOptModel, PTHSK, 1), "hbv_stack": (sb.HbvStackOptModel, HBV, 2),
                      "pt_hps_k": (sb.PTHPSKOptModel, PTHPSK, 4)}[stack]
     m = cls(geo, par, device=local_rank)
     m.run_interpolation(sb.InterpolationParameter(), ta, env)
     m.set_states(synthetic.default_state(sid, n))
+    if routed:
+        m.set_river_network(synthetic.river_chain(10))
     m.run_cells()
-    obs = m.catchment_discharges().sum(axis=1).reshape(-1, 24).mean(axis=1)
-    opt = sb.Optimizer(m, [sb.TargetSpecification(obs, ta.start, 86400, list(range(1, 11)), 1.0, 0)])
+    if routed:
+        obs = m.river_output_flow_m3s(8).reshape(-1, 24).mean(axis=1)
+        opt = sb.Optimizer(m, [sb.TargetSpecification(obs, ta.start, 86400, [], 1.0, 0, catchment_property=3, river_id=8)])
+    else:
+        obs = m.catchment_discharges().sum(axis=1).reshape(-1, 24).mean(axis=1)
+        opt = sb.Optimizer(m, [sb.TargetSpecification(obs, ta.start, 86400, list(range(1, 11)), 1.0, 0)])
     rng = np.random.default_rng(5)
     P = np.tile(par, (sets, 1))
     if stack == "pt_gs_k":
@@ -100,6 +109,9 @@ if 5 in which:  # calibration ensemble: parameter sets x 10k-cell catchment x 3 
         P[:, 3] = rng.uniform(10, 40, sets); P[:, 4] = rng.uniform(0.2, 0.7, sets); P[:, 5] = rng.uniform(0.1, 0.4, sets)
         P[:, 6] = rng.uniform(0.4, 1.2, sets); P[:, 7] = rng.uniform(0.01, 0.05, sets); P[:, 9] = rng.uniform(-2, 2, sets)
         P[:, 13] = rng.uniform(0.8, 1.4, sets)
+    if routed:
+        off = {"pt_gs_k": 25, "pt_hs_k": 13, "hbv_stack": 17, "pt_hps_k": 20}[stack]   # routing.velocity
+        P[:, off] = par[off] * rng.uniform(0.5, 1.5, sets)
     b, e = sharding.partition_parameter_sets(sets, world, rank)
     if world > 1:
         dist.barrier()
@@ -120,7 +132,8 @@ if 5 in which:  # calibration ensemble: parameter sets x 10k-cell catchment x 3 
     s1 = (time.perf_counter() - t0) / 8
     gpu = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", str(local_rank)], capture_output=True,
                          text=True).stdout.strip()
-    print(json.dumps({"config": 5, **({} if stack == "pt_gs_k" else {"stack": stack, "gpu": gpu}), "n_gpus": world, "sets": sets, "cells": n, "steps": T, "batch_seconds": s, "cell_steps_per_s": sets * n * T / s,
+    print(json.dumps({"config": 5, **({} if stack == "pt_gs_k" and not routed else {"stack": stack, "gpu": gpu}),
+                      **({"target": "routed"} if routed else {}), "n_gpus": world, "sets": sets, "cells": n, "steps": T, "batch_seconds": s, "cell_steps_per_s": sets * n * T / s,
                       "one_at_a_time_seconds_per_set": s1, "cell_steps_per_s_one_at_a_time": n * T / s1, "batch_equals_single": bool(np.array_equal(g[:8], g1)),
                       "best_goal": float(g.min()), "extrapolated_4096_sets_seconds": s * 4096 / sets}))
     if world > 1:
