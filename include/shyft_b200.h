@@ -191,6 +191,23 @@ int sb2_run_cells(sb2_model* m, int start_step, int n_steps);
  * last window only, catchment sums and states cover the whole call. */
 int sb2_run_windowed(sb2_model* m, const sb2_interpolation_parameter* ip, int start_step, int n_steps, int window_steps);
 
+/* ---- forcing ensembles ------------------------------------------------------------------------------ */
+/* The members of a forecast ensemble (create_ensembles, shyft/orchestration/simulator.py) in one call instead of one
+ * set_sources + interpolate + run_cells + catchment_discharges per member.  Member e of sb2_run_ensemble is bit for bit what that
+ * loop gives: member e's stations set for every variable that has ensemble sources (the model's own sources for every other
+ * variable), sb2_interpolate(ip, best_effort = 0), sb2_run_cells(start_step, n_steps) from the model's current state, and the
+ * catchment sums of those rows.  The model is left as it was; initialize_cell_environment drops ensemble sources as it drops sources. */
+/* one variable's stations for every member of a forcing ensemble, on the model axis: values [member][T][src] (as sb2_set_sources);
+   n_members == 0 or n_src == 0 clears the variable's ensemble sources.  Every variable with ensemble sources has the same member count. */
+int sb2_set_ensemble_sources(sb2_model* m, int var, int64_t n_members, int64_t n_src, const double* xyz, const double* values);
+/* ... on one point axis shared by all members and stations: values [member][n_points][src] (as sb2_set_sources_on_axis) */
+int sb2_set_ensemble_sources_on_axis(sb2_model* m, int var, int64_t n_members, int64_t n_src, const double* xyz, int64_t n_points,
+                                     const int64_t* t_us, int64_t t_end_us, const double* values, int point_interpretation);
+/* interpolate and step every member over [start_step, start_step + n_steps), window_steps at a time, from the model's current state
+   (n_steps == 0: the whole axis); discharge and charge (nullable) [member][n_steps][n_catchments], cix order */
+int sb2_run_ensemble(sb2_model* m, const sb2_interpolation_parameter* ip, int start_step, int n_steps, int window_steps,
+                     double* discharge, double* charge);
+
 /* ---- results ------------------------------------------------------------------------------------- */
 /* cell.rc.<series> / cell.sc.<series> (api/boostpython/expose.h:98-120); out [n_steps][cell] or [cell][n_steps] */
 int sb2_get_response(const sb2_model* m, int series, int64_t start_step, int64_t n_steps, double* out, int layout);

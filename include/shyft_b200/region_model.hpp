@@ -151,6 +151,45 @@ class region_model {
 
     void run_cells(size_t /*use_ncore*/ = 0, int start_step = 0, int n_steps = 0) { ck(sb2_run_cells(h_, start_step, n_steps)); }                   // :578-597
 
+    // forcing ensemble (sb2_run_ensemble): every member's interpolation + run_cells(start_step, n_steps) from the current state in one
+    // pass; per variable every member gives stations (the same positions) or none does (the model's own sources serve all members).
+    // -> discharge and charge [member][cix][step], as catchment_discharges; the model is left as it was
+    struct ensemble_result { std::vector<std::vector<std::vector<double>>> discharge, charge; };
+    ensemble_result run_ensemble(const interpolation_parameter& ip, const std::vector<region_environment>& members, int start_step = 0,
+                                 int n_steps = 0, int window_steps = 4096) {
+        static const char* names[SB2_N_FORCING] = {"temperature", "precipitation", "radiation", "wind_speed", "rel_hum"};
+        const size_t E = members.size();
+        if (E == 0) throw std::runtime_error("run_ensemble: no members");
+        for (int v = 0; v < SB2_N_FORCING; ++v) ck(sb2_set_ensemble_sources(h_, v, 0, 0, nullptr, nullptr));  // the member counts must agree
+        for (int v = 0; v < SB2_N_FORCING; ++v) {
+            const geo_point_sources& s0 = members[0].of(v);
+            std::vector<double> values;
+            for (const region_environment& env : members) {
+                const geo_point_sources& s = env.of(v);
+                // as interpolate: the C ABI takes no element counts, so a mis-shaped vector is refused here
+                if (s.xyz != s0.xyz || s.xyz.size() % 3 != 0 || s.values.size() != time_axis.n * s.size())
+                    throw std::runtime_error(std::string("run_ensemble: ") + names[v] +
+                                             ": every member needs the same source positions [n_sources][3] and values [n_steps][n_sources]");
+                values.insert(values.end(), s.values.begin(), s.values.end());
+            }
+            ck(sb2_set_ensemble_sources(h_, v, s0.size() ? int64_t(E) : 0, int64_t(s0.size()), s0.size() ? s0.xyz.data() : nullptr,
+                                        s0.size() ? values.data() : nullptr));
+        }
+        const size_t count = n_steps > 0 ? size_t(n_steps) : time_axis.n, nc = number_of_catchments();
+        std::vector<double> q(E * count * nc), c(q.size());
+        ck(sb2_run_ensemble(h_, &ip, start_step, n_steps, window_steps, q.data(), c.data()));
+        ip_parameter = ip;
+        ensemble_result r;
+        for (auto* out : {&r.discharge, &r.charge}) out->assign(E, std::vector<std::vector<double>>(nc, std::vector<double>(count)));
+        for (size_t e = 0; e < E; ++e)
+            for (size_t t = 0; t < count; ++t)
+                for (size_t k = 0; k < nc; ++k) {
+                    r.discharge[e][k][t] = q[(e * count + t) * nc + k];
+                    r.charge[e][k][t] = c[(e * count + t) * nc + k];
+                }
+        return r;
+    }
+
     // catchment_discharges(TSV&) (:873-885): cr[cix] = the catchment's series over the whole axis
     void catchment_discharges(std::vector<std::vector<double>>& cr) const { fetch(cr, sb2_catchment_discharges); }
     void catchment_charges(std::vector<std::vector<double>>& cr) const { fetch(cr, sb2_catchment_charges); }

@@ -79,6 +79,7 @@ sb2_get_region_parameter sb2_set_catchment_parameter sb2_get_catchment_parameter
 sb2_has_catchment_parameter sb2_set_catchment_calculation_filter sb2_set_states sb2_get_states sb2_set_initial_state
 sb2_hbv_distribute_snow sb2_get_initial_state sb2_revert_to_initial_state sb2_adjust_q sb2_adjust_state_to_target_flow sb2_extract_state sb2_apply_state sb2_set_collector_mode sb2_initialize_cell_environment
 sb2_set_cell_forcing sb2_get_cell_forcing sb2_set_sources sb2_set_sources_on_axis sb2_set_sources_on_axes sb2_get_sources_on_model_axis sb2_interpolate sb2_is_cell_env_ts_ok sb2_run_cells sb2_run_windowed
+sb2_set_ensemble_sources sb2_set_ensemble_sources_on_axis sb2_run_ensemble
 sb2_get_response sb2_get_state_series sb2_catchment_discharges sb2_catchment_charges sb2_statistics_series sb2_statistics_cells
 sb2_statistics_geo sb2_set_river_network sb2_river_flows
 sb2_set_targets sb2_calculate_goal_function sb2_calculate_goal_function_batch sb2_unit_eval sb2_host_eval sb2_set_idw_dense sb2_set_stream sb2_device_catchment_discharges sb2_device_catchment_charges sb2_step_chunk_steps sb2_check_guards sb2_kernel_launches sb2_last_run_kernel_ms""".split()

@@ -28,6 +28,7 @@
 #include "sb2_unit.cuh"
 #include "sb2_goal.cuh"
 #include "sb2_stats.cuh"
+#include "sb2_ensemble.cuh"
 
 using namespace sb2;
 
@@ -265,6 +266,8 @@ inline int grid_for(int64_t n, int block) { return int((n + block - 1) / block);
 #define SB2_HBV_UNIT_STEPS 64      // steps per time slice of the pt_ss_k / pt_hps_k / pt_hs_k / hbv_stack step kernels (128: within +-0.7 %)
 #define SB2_DENSE_TILE_COMPACT 32  // steps staged per buffer, compacted inverse distance over 64-station rows
 
+struct MemberRegionDeleter { void operator()(sb2_model* p) const; };  // sb2_model_destroy
+
 struct sb2_model {
     int stack = 0, device = 0;
     cudaStream_t stream = 0;
@@ -306,6 +309,15 @@ struct sb2_model {
     IdwPlan idw[SB2_N_FORCING];
     std::vector<std::unique_ptr<BtkOps>> btk_cache;
     DevArray<double> d_btk_kbuf, d_btk_beta, d_btk_resid;
+    // forcing ensemble (sb2_set_ensemble_sources): a variable's stations for every member, one Source per member (none: the model's own
+    // sources serve every member), with a plan and kriging operators of their own, as their stations are not the model's
+    std::vector<std::unique_ptr<Source>> ens_src[SB2_N_FORCING];
+    IdwPlan ens_idw[SB2_N_FORCING];
+    std::vector<std::unique_ptr<BtkOps>> ens_btk_cache;
+    // the internal region of member copies sb2_run_ensemble steps (DESIGN.md section 3.7), kept between calls: its geometry, slots and
+    // parameter-set indices are built on the host once per number of copies; parameters, filter and axis are re-applied when they change
+    std::unique_ptr<sb2_model, MemberRegionDeleter> ens_region;
+    int64_t ens_region_copies = 0;
     // collected series
     bool force_sparse_idw = false;  // diagnostics: run IDW through the per-neighbour kernel even when the dense operator applies
     int collect_bits = SB2_COLLECT_DISCHARGE;
@@ -757,9 +769,9 @@ int idw_kind_of(int var) {
     }
 }
 
-void build_idw_plan(sb2_model* m, int var) {
-    IdwPlan& pl = m->idw[var];
-    const Source& s = m->src[var];
+// the plan, the kriging operators and the sources come in explicitly: the model's own (m->src, m->idw, m->btk_cache) or a forcing
+// ensemble's (m->ens_src, m->ens_idw, m->ens_btk_cache), whose stations differ from the model's own
+void build_idw_plan(sb2_model* m, int var, const Source& s, IdwPlan& pl) {
     pl.p = to_idw(idw_parameter_of(m->ip, var));
     if (pl.p.max_members < 1) throw Error("inverse_distance: max_members must be >= 1");
     pl.n_src = s.n_src;
@@ -782,10 +794,8 @@ int idw_tile_steps(int64_t n_src) {
     return int(std::max<int64_t>(1, std::min<int64_t>(64, budget / std::max<int64_t>(1, n_src))));
 }
 
-void run_idw(sb2_model* m, int var, int64_t first, int64_t n_steps, double* out) {
-    IdwPlan& pl = m->idw[var];
-    if (!pl.valid) build_idw_plan(m, var);
-    const Source& s = m->src[var];
+void run_idw(sb2_model* m, int var, const Source& s, IdwPlan& pl, int64_t first, int64_t n_steps, double* out) {
+    if (!pl.valid) build_idw_plan(m, var, s, pl);
     if (!s.has_nonfinite && !(var == SB2_TEMPERATURE && pl.p.gradient_by_equation) && s.n_src <= 96 && !m->force_sparse_idw) {
         // every station value is finite: the weighted means are one dense contraction on the FP64 tensor cores
         if (!pl.dense_valid) {
@@ -862,11 +872,11 @@ void run_idw(sb2_model* m, int var, int64_t first, int64_t n_steps, double* out)
     ++m->launches;
 }
 
-BtkOps* btk_ops_for(sb2_model* m, const std::vector<int>& valid, bool check_rank) {
-    for (auto& o : m->btk_cache)
+using BtkCache = std::vector<std::unique_ptr<BtkOps>>;
+BtkOps* btk_ops_for(sb2_model* m, const Source& s, BtkCache& cache, const std::vector<int>& valid, bool check_rank) {
+    for (auto& o : cache)
         if (o->valid == valid) return o.get();
-    if (m->btk_cache.size() >= 8) m->btk_cache.erase(m->btk_cache.begin() + 1);  // keep the full-set operators at slot 0
-    const Source& s = m->src[SB2_TEMPERATURE];
+    if (cache.size() >= 8) cache.erase(cache.begin() + 1);  // keep the full-set operators at slot 0
     const sb2_btk_parameter& bp = m->ip.temperature;
     host::BtkStationOps h = host::btk_station_ops(s.xyz, valid, bp.sill, bp.nug, bp.range, bp.zscale, bp.gradient_sd, check_rank);
     auto o = std::make_unique<BtkOps>();
@@ -893,16 +903,15 @@ BtkOps* btk_ops_for(sb2_model* m, const std::vector<int>& valid, bool check_rank
     CUDA_OK(cudaGetLastError());
     ++m->launches;
     CUDA_OK(cudaStreamSynchronize(m->stream));  // the temporaries above go out of scope
-    m->btk_cache.push_back(std::move(o));
-    return m->btk_cache.back().get();
+    cache.push_back(std::move(o));
+    return cache.back().get();
 }
 
-void run_btk(sb2_model* m, int64_t first, int64_t n_steps, double* out) {
-    const Source& s = m->src[SB2_TEMPERATURE];
+void run_btk(sb2_model* m, const Source& s, BtkCache& cache, int64_t first, int64_t n_steps, double* out) {
     const int S = int(s.n_src);
     std::vector<int> all(S);
     for (int i = 0; i < S; ++i) all[i] = i;
-    BtkOps* full = btk_ops_for(m, all, true);  // built (and rank-checked) before the time loop, bayesian_kriging.h:300-316
+    BtkOps* full = btk_ops_for(m, s, cache, all, true);  // built (and rank-checked) before the time loop, bayesian_kriging.h:300-316
     // segments of constant valid-station set (:333-381)
     int64_t i = 0;
     while (i < n_steps) {
@@ -928,7 +937,7 @@ void run_btk(sb2_model* m, int64_t first, int64_t n_steps, double* out) {
                 }
                 if (!same) break;
             }
-        BtkOps* op = int(valid.size()) == S ? full : btk_ops_for(m, valid, false);
+        BtkOps* op = int(valid.size()) == S ? full : btk_ops_for(m, s, cache, valid, false);
         const int nv = int(valid.size());
         const int64_t seg = j - i;
         m->d_btk_beta.ensure(size_t(seg) * 2);
@@ -966,19 +975,18 @@ void run_btk(sb2_model* m, int64_t first, int64_t n_steps, double* out) {
 }
 
 // One variable over [first, first+n_steps) into out[(i)*n + c]; the case analysis of region_model.h:456-515
-void interpolate_variable(sb2_model* m, int var, int64_t first, int64_t n_steps, double* out) {
-    const Source& s = m->src[var];
+void interpolate_variable(sb2_model* m, int var, const Source& s, IdwPlan& pl, BtkCache& cache, int64_t first, int64_t n_steps, double* out) {
     if (s.n_src == 0) return;  // env.<var> == nullptr: the cell series keep their NaN fill
     if (var == SB2_TEMPERATURE) {
         if (s.n_src > 1) {
-            if (m->ip.use_idw_for_temperature) run_idw(m, var, first, n_steps, out);
-            else run_btk(m, first, n_steps, out);
+            if (m->ip.use_idw_for_temperature) run_idw(m, var, s, pl, first, n_steps, out);
+            else run_btk(m, s, cache, first, n_steps, out);
         } else {
             broadcast_source_kernel<<<grid_for(m->n, 128), 128, 0, m->stream>>>(m->n, s.d_values.p + first, int(n_steps), m->d_active.p, out);
             CUDA_OK(cudaGetLastError());
             ++m->launches;
         }
-    } else run_idw(m, var, first, n_steps, out);
+    } else run_idw(m, var, s, pl, first, n_steps, out);
 }
 
 bool interpolate_range(sb2_model* m, int64_t first, int64_t n_steps, int best_effort) {
@@ -987,7 +995,7 @@ bool interpolate_range(sb2_model* m, int64_t first, int64_t n_steps, int best_ef
     bool all_ok = true;
     for (int var = 0; var < SB2_N_FORCING; ++var) {
         try {
-            interpolate_variable(m, var, first, n_steps, m->d_forcing[var].p + (first - m->forcing_first) * m->n);
+            interpolate_variable(m, var, m->src[var], m->idw[var], m->btk_cache, first, n_steps, m->d_forcing[var].p + (first - m->forcing_first) * m->n);
         } catch (const std::exception&) {
             if (!best_effort) throw;
             all_ok = false;
@@ -1003,6 +1011,8 @@ void set_interpolation_parameter(sb2_model* m, const sb2_interpolation_parameter
     m->ip_valid = true;
     for (auto& pl : m->idw) pl.valid = false;
     m->btk_cache.clear();
+    for (auto& pl : m->ens_idw) pl.valid = false;
+    m->ens_btk_cache.clear();
 }
 
 void ensure_forcing(sb2_model* m, int64_t first, int64_t rows, bool nan_fill) {
@@ -1503,6 +1513,7 @@ void sb2_model_destroy(sb2_model* m) {
     for (auto& ev : m->ev) if (ev) cudaEventDestroy(ev);
     delete m;
 }
+void MemberRegionDeleter::operator()(sb2_model* p) const { sb2_model_destroy(p); }
 
 const char* sb2_last_error(const sb2_model* m) { return m ? m->err.c_str() : g_create_error.c_str(); }
 
@@ -1812,6 +1823,11 @@ int sb2_initialize_cell_environment(sb2_model* m, int64_t t0_us, int64_t dt_us, 
             m->idw[v].valid = false; m->idw[v].dense_valid = false;
         }
         m->btk_cache.clear();
+        for (int v = 0; v < SB2_N_FORCING; ++v) {  // ensemble sources were laid out on the old axis too
+            m->ens_src[v].clear();
+            m->ens_idw[v].valid = false; m->ens_idw[v].dense_valid = false;
+        }
+        m->ens_btk_cache.clear();
         m->d_axis_t.release();
         m->targets.clear();
         m->rlocal_valid = m->rnet_valid = false;
@@ -1863,60 +1879,131 @@ static Source* begin_sources(sb2_model* m, int var, int64_t n_src, const double*
     s.d_xyz.upload(s.xyz, m->stream);
     return &s;
 }
+// values [T][src] on the model axis into s (geometry installed)
+static void load_sources(sb2_model* m, int var, Source& s, const double* values) {
+    const size_t count = size_t(m->T) * s.n_src;
+    s.d_values.upload(values, count, m->stream);
+    // average_accessor of a stair-case source on the model axis (time_series.h:202-310,2033-2072)
+    // ... which also reports whether any value is NaN / inf: the scan of the values runs on the device, not over the host buffer
+    m->d_scan_flag.ensure(1);
+    CUDA_OK(cudaMemsetAsync(m->d_scan_flag.p, 0, sizeof(int), m->stream));
+    average_accessor_same_axis_kernel<<<std::min<int64_t>(grid_for(count, 256), 148 * 16), 256, 0, m->stream>>>(s.d_values.p, int64_t(count),
+                                                                                                         double(m->dt) / 1e6, m->d_scan_flag.p);
+    CUDA_OK(cudaGetLastError());
+    ++m->launches;
+    int flag = 0;
+    CUDA_OK(cudaMemcpyAsync(&flag, m->d_scan_flag.p, sizeof(int), cudaMemcpyDeviceToHost, m->stream));
+    CUDA_OK(cudaStreamSynchronize(m->stream));
+    s.has_nonfinite = flag != 0;
+    // the host copy serves the valid-station bookkeeping of Bayesian kriging (run_btk), needed only when stations drop out
+    if (var == SB2_TEMPERATURE && s.has_nonfinite) s.h_values.assign(values, values + count);
+    else s.h_values.clear();
+}
+static void check_point_axis(int64_t n_src, int64_t n_points, const int64_t* t_us, int64_t t_end_us, const double* values) {
+    if (n_src > 0 && n_points > 0) {
+        if (!t_us || !values) throw Error("set_sources_on_axis: null time or value array");
+        for (int64_t i = 1; i < n_points; ++i)
+            if (!(t_us[i] > t_us[i - 1])) throw Error("set_sources_on_axis: point times must be strictly increasing");
+        if (t_end_us < t_us[n_points - 1]) throw Error("set_sources_on_axis: the total period ends before the last point");
+    }
+}
+// values [n_points][src] on the point axis t_us, projected onto the model axis into s (geometry installed)
+static void load_sources_on_axis(sb2_model* m, int var, Source& s, int64_t n_points, const int64_t* t_us, int64_t t_end_us, const double* values,
+                                 int point_interpretation) {
+    const int64_t n_src = s.n_src;
+    const size_t count = size_t(m->T) * n_src;
+    DevArray<int64_t> d_t;
+    DevArray<double> d_pts;
+    d_t.upload(t_us, size_t(n_points), m->stream);
+    d_pts.upload(values, size_t(n_points) * n_src, m->stream);
+    s.d_values.resize(count);
+    average_accessor_kernel<<<grid_for(int64_t(count), 256), 256, 0, m->stream>>>(d_t.p, d_pts.p, n_points, n_src, t_end_us,
+                                                                                 point_interpretation == SB2_POINT_INSTANT_VALUE ? 1 : 0, m->t0, m->dt,
+                                                                                 m->T, s.d_values.p);
+    CUDA_OK(cudaGetLastError());
+    ++m->launches;
+    // the projected series back on the host: NaN bookkeeping of interpolate(), BTK validity sets
+    std::vector<double> h(count);
+    CUDA_OK(cudaMemcpyAsync(h.data(), s.d_values.p, count * sizeof(double), cudaMemcpyDeviceToHost, m->stream));
+    CUDA_OK(cudaStreamSynchronize(m->stream));
+    s.has_nonfinite = false;
+    for (size_t i = 0; i < count && !s.has_nonfinite; ++i) s.has_nonfinite = !std::isfinite(h[i]);
+    if (var == SB2_TEMPERATURE) s.h_values = std::move(h);
+}
 int sb2_set_sources(sb2_model* m, int var, int64_t n_src, const double* xyz, const double* values) {
     return guarded(m, [&] {
         Source* sp = begin_sources(m, var, n_src, xyz);
         if (!sp) return;
-        Source& s = *sp;
-        const size_t count = size_t(m->T) * n_src;
-        s.d_values.upload(values, count, m->stream);
-        // average_accessor of a stair-case source on the model axis (time_series.h:202-310,2033-2072)
-        // ... which also reports whether any value is NaN / inf: the scan of the values runs on the device, not over the host buffer
-        m->d_scan_flag.ensure(1);
-        CUDA_OK(cudaMemsetAsync(m->d_scan_flag.p, 0, sizeof(int), m->stream));
-        average_accessor_same_axis_kernel<<<std::min<int64_t>(grid_for(count, 256), 148 * 16), 256, 0, m->stream>>>(s.d_values.p, int64_t(count),
-                                                                                                             double(m->dt) / 1e6, m->d_scan_flag.p);
-        CUDA_OK(cudaGetLastError());
-        ++m->launches;
-        int flag = 0;
-        CUDA_OK(cudaMemcpyAsync(&flag, m->d_scan_flag.p, sizeof(int), cudaMemcpyDeviceToHost, m->stream));
-        CUDA_OK(cudaStreamSynchronize(m->stream));
-        s.has_nonfinite = flag != 0;
-        // the host copy serves the valid-station bookkeeping of Bayesian kriging (run_btk), needed only when stations drop out
-        if (var == SB2_TEMPERATURE && s.has_nonfinite) s.h_values.assign(values, values + count);
-        else s.h_values.clear();
+        load_sources(m, var, *sp, values);
     });
 }
 int sb2_set_sources_on_axis(sb2_model* m, int var, int64_t n_src, const double* xyz, int64_t n_points, const int64_t* t_us, int64_t t_end_us,
                             const double* values, int point_interpretation) {
     return guarded(m, [&] {
-        if (n_src > 0 && n_points > 0) {
-            if (!t_us || !values) throw Error("set_sources_on_axis: null time or value array");
-            for (int64_t i = 1; i < n_points; ++i)
-                if (!(t_us[i] > t_us[i - 1])) throw Error("set_sources_on_axis: point times must be strictly increasing");
-            if (t_end_us < t_us[n_points - 1]) throw Error("set_sources_on_axis: the total period ends before the last point");
-        }
+        check_point_axis(n_src, n_points, t_us, t_end_us, values);
         Source* sp = begin_sources(m, var, n_src, xyz);
         if (!sp) return;
-        Source& s = *sp;
-        const size_t count = size_t(m->T) * n_src;
-        DevArray<int64_t> d_t;
-        DevArray<double> d_pts;
-        d_t.upload(t_us, size_t(n_points), m->stream);
-        d_pts.upload(values, size_t(n_points) * n_src, m->stream);
-        s.d_values.resize(count);
-        average_accessor_kernel<<<grid_for(int64_t(count), 256), 256, 0, m->stream>>>(d_t.p, d_pts.p, n_points, n_src, t_end_us,
-                                                                                     point_interpretation == SB2_POINT_INSTANT_VALUE ? 1 : 0, m->t0, m->dt,
-                                                                                     m->T, s.d_values.p);
-        CUDA_OK(cudaGetLastError());
-        ++m->launches;
-        // the projected series back on the host: NaN bookkeeping of interpolate(), BTK validity sets
-        std::vector<double> h(count);
-        CUDA_OK(cudaMemcpyAsync(h.data(), s.d_values.p, count * sizeof(double), cudaMemcpyDeviceToHost, m->stream));
-        CUDA_OK(cudaStreamSynchronize(m->stream));
-        s.has_nonfinite = false;
-        for (size_t i = 0; i < count && !s.has_nonfinite; ++i) s.has_nonfinite = !std::isfinite(h[i]);
-        if (var == SB2_TEMPERATURE) s.h_values = std::move(h);
+        load_sources_on_axis(m, var, *sp, n_points, t_us, t_end_us, values, point_interpretation);
+    });
+}
+// ---- forcing ensembles -----------------------------------------------------------------------------------------------
+// the member count of the ensemble variables other than `var` (0: none has ensemble sources)
+static int64_t ensemble_members(const sb2_model* m, int except_var = -1) {
+    for (int v = 0; v < SB2_N_FORCING; ++v)
+        if (v != except_var && !m->ens_src[v].empty()) return int64_t(m->ens_src[v].size());
+    return 0;
+}
+// drops the variable's ensemble sources (n_members == 0) or installs n_members empty ones with the stations' geometry; null when dropped
+static std::vector<std::unique_ptr<Source>>* begin_ensemble_sources(sb2_model* m, int var, int64_t n_members, int64_t n_src, const double* xyz) {
+    if (var < 0 || var >= SB2_N_FORCING) throw Error("unknown forcing variable");
+    if (!(m->T > 0)) throw Error("initialize_cell_environment has not been called");
+    if (n_members < 0 || n_src < 0) throw Error("set_ensemble_sources: negative member or source count");
+    const int64_t others = ensemble_members(m, var);
+    if (n_members > 0 && n_src > 0 && others > 0 && others != n_members)
+        throw Error("set_ensemble_sources: " + std::to_string(n_members) + " members given, but the other ensemble variables have " +
+                    std::to_string(others));
+    if (n_members > 0 && n_src > 0 && !xyz) throw Error("set_ensemble_sources: null station positions");
+    auto& ens = m->ens_src[var];
+    ens.clear();
+    m->ens_idw[var].valid = false;
+    m->ens_idw[var].dense_valid = false;
+    if (var == SB2_TEMPERATURE) m->ens_btk_cache.clear();
+    if (n_members == 0 || n_src == 0) return nullptr;
+    for (int64_t e = 0; e < n_members; ++e) {
+        auto s = std::make_unique<Source>();
+        s->n_src = n_src;
+        s->xyz.assign(xyz, xyz + 3 * n_src);
+        s->d_xyz.upload(s->xyz, m->stream);
+        ens.push_back(std::move(s));
+    }
+    return &ens;
+}
+int sb2_set_ensemble_sources(sb2_model* m, int var, int64_t n_members, int64_t n_src, const double* xyz, const double* values) {
+    return guarded(m, [&] {
+        auto* ens = begin_ensemble_sources(m, var, n_members, n_src, xyz);
+        if (!ens) return;
+        try {
+            if (!values) throw Error("set_ensemble_sources: null values");
+            for (int64_t e = 0; e < n_members; ++e) load_sources(m, var, *(*ens)[size_t(e)], values + size_t(e) * m->T * n_src);
+        } catch (...) {
+            ens->clear();
+            throw;
+        }
+    });
+}
+int sb2_set_ensemble_sources_on_axis(sb2_model* m, int var, int64_t n_members, int64_t n_src, const double* xyz, int64_t n_points,
+                                     const int64_t* t_us, int64_t t_end_us, const double* values, int point_interpretation) {
+    return guarded(m, [&] {
+        if (n_members > 0) check_point_axis(n_src, n_points, t_us, t_end_us, values);
+        auto* ens = begin_ensemble_sources(m, var, n_members, n_src, xyz);
+        if (!ens) return;
+        try {
+            for (int64_t e = 0; e < n_members; ++e)
+                load_sources_on_axis(m, var, *(*ens)[size_t(e)], n_points, t_us, t_end_us, values + size_t(e) * n_points * n_src, point_interpretation);
+        } catch (...) {
+            ens->clear();
+            throw;
+        }
     });
 }
 int sb2_set_sources_on_axes(sb2_model* m, int var, int64_t n_src, const double* xyz, const int64_t* n_points, const int64_t* t_us,
@@ -2192,6 +2279,191 @@ int sb2_run_windowed(sb2_model* m, const sb2_interpolation_parameter* ip, int st
         m->ran_first = first; m->ran_steps = count;
         if (route) m->rlocal_valid = true;
         check_device_errors(m);
+    });
+}
+
+// ---- forcing ensembles: every member interpolated and stepped in one pass (DESIGN.md section 3.7) ------------------------------
+namespace {
+// The members are stepped as one internal region of copies of the model (sb2_ensemble.cuh): member e's copy of cell c is internal cell
+// e * np + c and its catchment k internal catchment e * kp + k.  np is n rounded up to the 32-cell warp, so every copy starts on a warp
+// boundary and has the model's slots (build_slots) in the same lanes and order; the np - n padding cells of a copy form catchment
+// kp - 1 = n_catch of their own, outside the calculation filter.
+struct EnsembleLayout {
+    int64_t np = 0, kp = 0;     // cells and catchments of one member copy
+    int64_t window = 0;         // steps per forcing window
+    int64_t per_pass = 0, passes = 0;
+};
+constexpr int64_t kEnsembleBudget = 32LL << 30;  // the device buffers of one call (the model's own resident buffers are not counted)
+EnsembleLayout ensemble_layout(int stack, int64_t n, int64_t n_catch, int64_t n_state, int64_t T, int64_t count, int64_t window_steps, int64_t members) {
+    EnsembleLayout L;
+    L.np = (n + 31) / 32 * 32;
+    L.kp = n_catch + (L.np > n ? 1 : 0);
+    L.window = std::min<int64_t>(window_steps, count);
+    // whatever the member count: the [W][n] window a member is interpolated into and up to five of the variables from the model's own
+    // sources, and the internal region's per-slot partial sums, which launch_step_range keeps within 1 GB
+    const int64_t fixed = 6 * 8 * L.window * n + (1LL << 30);
+    // per member: five [W][np] forcing windows, the state, pt_gs_k's five [<= W][np] phase-pipeline arrays, the [T][kp] discharge and charge sums
+    const int64_t per_member = 8 * L.np * (5 * L.window * (stack == SB2_PT_GS_K ? 2 : 1) + n_state) + 16 * T * L.kp;
+    const int64_t cap = std::max<int64_t>(1, std::min<int64_t>({members, int64_t(65535), std::max<int64_t>(0, kEnsembleBudget - fixed) / per_member}));
+    L.passes = (members + cap - 1) / cap;
+    L.per_pass = (members + L.passes - 1) / L.passes;  // members spread evenly over the passes; a shorter last pass leaves copies spare
+    return L;
+}
+
+
+// rows of the model's geometry ([rows][n] per member at src + e * src_stride, e < members) into members e0 .. of a [rows][dst_cols] region
+void scatter_members(sb2_model* m, const double* src, int64_t src_stride, int64_t rows, int64_t np, double* dst, int64_t dst_cols, int64_t e0,
+                     int64_t members) {
+    if (rows <= 0) return;
+    const dim3 grid((unsigned)grid_for(np, 256), (unsigned)std::min<int64_t>(rows, 128), (unsigned)members);
+    ensemble_scatter_kernel<<<grid, 256, 0, m->stream>>>(src, src_stride, m->n, np, rows, dst, dst_cols, e0);
+    CUDA_OK(cudaGetLastError());
+    ++m->launches;
+}
+
+// the internal region of `copies` member copies, built like any model: geometry, catchments and slots.  Host work over every internal
+// cell, so the model keeps the region for the next call (sb2_model::ens_region).
+void build_member_region(sb2_model* m, const EnsembleLayout& L, int64_t copies) {
+    const int64_t n = m->n, np = L.np, kp = L.kp, K = m->n_catch(), cells = copies * np;
+    m->ens_region.reset();
+    m->ens_region_copies = 0;
+    std::vector<sb2_geo_cell> geo(static_cast<size_t>(cells));
+    for (int64_t e = 0; e < copies; ++e)
+        for (int64_t c = 0; c < np; ++c) {
+            sb2_geo_cell g = m->geo[size_t(std::min(c, n - 1))];
+            g.catchment_id = e * kp + (c < n ? m->cix_of_cell[c] : K);  // first appearance in this order: internal cix == internal id
+            g.routing_id = 0;
+            geo[size_t(e * np + c)] = g;
+        }
+    sb2_model* raw = nullptr;
+    if (sb2_model_create(m->stack, cells, geo.data(), m->device, &raw) != 0) throw Error(sb2_last_error(nullptr));
+    m->ens_region.reset(raw);
+    if (raw->n_catch() != copies * kp) throw Error("run_ensemble: internal catchment numbering");
+    raw->collect_bits = SB2_COLLECT_NONE;  // catchment sums only
+    raw->region_param.clear();             // nothing configured yet: configure_member_region applies it all
+    m->ens_region_copies = copies;
+}
+
+// the model's parameter set, catchment overrides, calculation filter and time axis on every copy; only what changed since the last call is
+// applied again (a changed parameter set or filter is re-uploaded by sync_parameters / sync_filter at the next launch)
+void configure_member_region(sb2_model* m, const EnsembleLayout& L) {
+    sb2_model* im = m->ens_region.get();
+    const int64_t copies = m->ens_region_copies, kp = L.kp, K = m->n_catch();
+    im->stream = m->stream;
+    if (im->region_param != m->region_param) { im->region_param = m->region_param; im->param_dirty = true; }
+    std::map<int64_t, std::vector<double>> catch_param;
+    for (auto& kv : m->catch_param) {
+        auto f = m->cid_to_cix.find(kv.first);
+        if (f == m->cid_to_cix.end()) continue;
+        for (int64_t e = 0; e < copies; ++e) catch_param[e * kp + f->second] = kv.second;
+    }
+    if (im->catch_param != catch_param) { im->catch_param = std::move(catch_param); im->param_dirty = true; }
+    std::vector<uint8_t> filter;  // the padding catchments are never calculated
+    if (L.np > m->n || !m->catchment_filter.empty()) {
+        filter.assign(size_t(copies * kp), 0);
+        for (int64_t e = 0; e < copies; ++e)
+            for (int64_t k = 0; k < K; ++k) filter[size_t(e * kp + k)] = m->catchment_filter.empty() ? 1 : m->catchment_filter[size_t(k)];
+    }
+    if (im->catchment_filter != filter) { im->catchment_filter = std::move(filter); im->filter_dirty = true; }
+    if (im->t0 != m->t0 || im->dt != m->dt || im->T != m->T || im->d_doy_soy.n != size_t(m->T)) {
+        if (im->dt != m->dt) im->param_dirty = true;  // the per-run constants of the parameter tables depend on dt
+        im->t0 = m->t0; im->dt = m->dt; im->T = m->T;
+        im->d_doy_soy.resize(size_t(m->T));
+        CUDA_OK(cudaMemcpyAsync(im->d_doy_soy.p, m->d_doy_soy.p, size_t(m->T) * sizeof(int2), cudaMemcpyDeviceToDevice, m->stream));
+    }
+    // the buffers of this call; release_member_buffers hands them back to the device pool at its end
+    const size_t cells = size_t(copies * L.np);
+    im->d_state.resize(size_t(m->n_state) * cells);
+    for (auto& f : im->d_forcing) f.resize(size_t(L.window) * cells);
+    im->forcing_rows = L.window;
+    im->d_cq.resize(size_t(m->T) * copies * kp);
+    im->d_cc.resize(size_t(m->T) * copies * kp);
+}
+
+// the large buffers of the region go back to the device pool after a call: the model keeps only the region's per-cell tables
+void release_member_buffers(sb2_model* im) {
+    for (auto& f : im->d_forcing) f.release();
+    im->forcing_rows = 0;
+    for (auto& b : im->d_scr) b.release();
+    im->d_partial.release();
+    im->partial_steps = 0;
+    im->d_state.release();
+    im->d_cq.release();
+    im->d_cc.release();
+}
+}  // namespace
+
+int sb2_run_ensemble(sb2_model* m, const sb2_interpolation_parameter* ip, int start_step, int n_steps, int window_steps, double* discharge,
+                     double* charge) {
+    return guarded(m, [&] {
+        validate_run_args(m, start_step, n_steps);
+        const int64_t E = ensemble_members(m);
+        if (E == 0) throw Error("run_ensemble: no ensemble sources set");
+        if (window_steps <= 0) throw Error("run_ensemble: window_steps must be positive");
+        if (!discharge) throw Error("run_ensemble: null discharge output");
+        set_interpolation_parameter(m, ip);
+        sync_filter(m);
+        const int64_t first = n_steps > 0 ? start_step : 0;  // as run_cells: n_steps == 0 runs the whole axis
+        const int64_t count = n_steps > 0 ? n_steps : m->T;
+        const int64_t n = m->n, K = m->n_catch();
+        const EnsembleLayout L = ensemble_layout(m->stack, n, K, m->n_state, m->T, count, window_steps, E);
+        const int64_t W = L.window, np = L.np, kp = L.kp;
+        // a member's interpolated window in the model's geometry; a variable from the model's own sources is interpolated once per
+        // window for all members.  Both start NaN, as the cell series of interpolate() do for cells and variables it does not reach.
+        DevArray<double> d_stage, d_own[SB2_N_FORCING];
+        d_stage.resize(size_t(W) * n);
+        fill_nan(m, d_stage.p, W * n);
+        for (int v = 0; v < SB2_N_FORCING; ++v)
+            if (m->ens_src[v].empty()) { d_own[v].resize(size_t(W) * n); fill_nan(m, d_own[v].p, W * n); }
+        std::vector<double> h_cq, h_cc;
+        // the region holds per_pass copies; a shorter last pass fills its spare copies with its last member, whose sums are not read
+        if (!m->ens_region || m->ens_region_copies != L.per_pass || m->ens_region->n != L.per_pass * np) build_member_region(m, L, L.per_pass);
+        sb2_model* im = m->ens_region.get();
+        const int64_t R = L.per_pass, cols = R * np, kcols = R * kp;
+        struct CallEnd {  // the internal region's launches are the model's; its large buffers go back to the pool
+            sb2_model *m, *im;
+            ~CallEnd() { m->launches += im->launches; im->launches = 0; release_member_buffers(im); }
+        } call_end{m, im};
+        configure_member_region(m, L);
+        for (int64_t e0 = 0; e0 < E; e0 += R) {
+            const int64_t ne = std::min<int64_t>(R, E - e0);
+            // every pass starts from the model's current state
+            scatter_members(m, m->d_state.p, 0, m->n_state, np, im->d_state.p, cols, 0, R);
+            for (int64_t w0 = first; w0 < first + count; w0 += W) {
+                const int64_t wn = std::min<int64_t>(W, first + count - w0);
+                NvtxRange nv_window("ensemble window " + std::to_string((w0 - first) / W));
+                im->forcing_first = w0;
+                for (int v = 0; v < SB2_N_FORCING; ++v) {
+                    if (m->ens_src[v].empty()) {
+                        interpolate_variable(m, v, m->src[v], m->idw[v], m->btk_cache, w0, wn, d_own[v].p);
+                        scatter_members(m, d_own[v].p, 0, wn, np, im->d_forcing[v].p, cols, 0, R);
+                    } else
+                    {
+                        for (int64_t e = 0; e < ne; ++e) {
+                            interpolate_variable(m, v, *m->ens_src[v][size_t(e0 + e)], m->ens_idw[v], m->ens_btk_cache, w0, wn, d_stage.p);
+                            scatter_members(m, d_stage.p, 0, wn, np, im->d_forcing[v].p, cols, e, 1);
+                        }
+                        if (ne < R) scatter_members(m, d_stage.p, 0, wn, np, im->d_forcing[v].p, cols, ne, R - ne);
+                    }
+                }
+                launch_step_range(im, w0, wn, false);
+            }
+            check_device_errors(im);
+            // [count][ne * kp] rows of the run back in one copy each, then member by member into [member][step][n_catch]
+            h_cq.resize(size_t(count) * kcols);
+            CUDA_OK(cudaMemcpyAsync(h_cq.data(), im->d_cq.p + first * kcols, h_cq.size() * sizeof(double), cudaMemcpyDeviceToHost, m->stream));
+            if (charge) {
+                h_cc.resize(h_cq.size());
+                CUDA_OK(cudaMemcpyAsync(h_cc.data(), im->d_cc.p + first * kcols, h_cc.size() * sizeof(double), cudaMemcpyDeviceToHost, m->stream));
+            }
+            CUDA_OK(cudaStreamSynchronize(m->stream));
+            for (int64_t e = 0; e < ne; ++e)
+                for (int64_t i = 0; i < count; ++i) {
+                    const size_t from = size_t(i * kcols + e * kp), to = size_t(((e0 + e) * count + i) * K);
+                    std::copy(h_cq.begin() + from, h_cq.begin() + from + K, discharge + to);
+                    if (charge) std::copy(h_cc.begin() + from, h_cc.begin() + from + K, charge + to);
+                }
+        }
     });
 }
 

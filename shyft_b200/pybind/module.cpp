@@ -96,6 +96,22 @@ void bind_model(py::module_& m, const char* name, int collect_bits, const char* 
              "run_interpolation(interpolation_parameter defaults, fixed_dt{t0, dt, n} in microseconds, {name: (xyz [s][3], values [n][s])})")
         .def("is_cell_env_ts_ok", &M::is_cell_env_ts_ok)
         .def("run_cells", &M::run_cells, py::arg("use_ncore") = 0, py::arg("start_step") = 0, py::arg("n_steps") = 0)
+        .def("run_ensemble",
+             [](M& self, const py::list& members, int start_step, int n_steps, int window_steps) {
+                 std::vector<sb::region_environment> envs;
+                 for (const py::handle& d : members) envs.push_back(env_from(d.cast<py::dict>()));
+                 const auto r = self.run_ensemble(self.ip_parameter, envs, start_step, n_steps, window_steps);
+                 auto to_array = [](const std::vector<std::vector<std::vector<double>>>& v) {
+                     const py::ssize_t E = py::ssize_t(v.size()), K = E ? py::ssize_t(v[0].size()) : 0, T = K ? py::ssize_t(v[0][0].size()) : 0;
+                     darray out({E, K, T});
+                     for (py::ssize_t e = 0; e < E; ++e)
+                         for (py::ssize_t k = 0; k < K; ++k) std::memcpy(out.mutable_data(e, k, 0), v[size_t(e)][size_t(k)].data(), size_t(T) * sizeof(double));
+                     return out;
+                 };
+                 return py::make_tuple(to_array(r.discharge), to_array(r.charge));
+             },
+             py::arg("members"), py::arg("start_step") = 0, py::arg("n_steps") = 0, py::arg("window_steps") = 4096,
+             "forcing ensemble: a list of run_interpolation's dicts, one per member -> (discharge, charge), each [member][catchment][step]")
         .def("catchment_discharges",
              [](const M& self) {
                  std::vector<std::vector<double>> cr;

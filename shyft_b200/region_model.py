@@ -393,6 +393,53 @@ class RegionModel:
         self._ck(self._L.sb2_run_windowed(self._h, C.byref(ip_parameter), C.c_int(start_step), C.c_int(n_steps), C.c_int(window_steps)))
         self.ip_parameter = ip_parameter
 
+    def run_ensemble(self, ip_parameter, members, start_step=0, n_steps=0, window_steps=4096):
+        """Interpolate and step every member of a forcing ensemble (a list of RegionEnvironment) in one device pass, from the current
+        state -> (discharge, charge), each [member][n_steps][n_catchment] (n_steps == 0: the whole axis).
+
+        Member e equals, bit for bit, setting member e's sources, interpolate(ip_parameter, env, best_effort=False), run_cells(0,
+        start_step, n_steps) from the same state and reading catchment_discharges / catchment_charges of those rows.  Per variable,
+        every member gives a (xyz, values [T][S]) tuple with the same xyz, or a GeoPointSources with the same xyz, times, t_end and
+        point_fx; or every member leaves it None, and the model's own sources serve all members.  The model is left as it was."""
+        members = list(members)
+        if not members:
+            raise RuntimeError("run_ensemble: no members")
+        if self.time_axis is None:
+            raise RuntimeError("initialize_cell_environment has not been called")
+        E, T = len(members), self.time_axis.n
+        for vi in range(len(FORCING_NAMES)):   # every variable's earlier ensemble sources go first: the member counts must agree
+            self._ck(self._L.sb2_set_ensemble_sources(self._h, C.c_int(vi), C.c_int64(0), C.c_int64(0), None, None))
+        for vi, name in enumerate(FORCING_NAMES):
+            srcs = [getattr(env, name) for env in members]
+            if all(s is None for s in srcs):
+                continue
+            if all(isinstance(s, GeoPointSources) for s in srcs):
+                s0 = srcs[0]
+                if not all(np.array_equal(s.xyz, s0.xyz) and np.array_equal(s.times_us, s0.times_us) and s.t_end_us == s0.t_end_us
+                           and s.point_fx == s0.point_fx and s.values.shape == (s0.times_us.size, s0.xyz.shape[0]) for s in srcs):
+                    raise RuntimeError(f"{name}: every member needs the same stations, times, t_end and point_fx, values [n_points][n_sources]")
+                values = np.ascontiguousarray(np.stack([s.values for s in srcs]))
+                self._ck(self._L.sb2_set_ensemble_sources_on_axis(self._h, C.c_int(vi), C.c_int64(E), C.c_int64(s0.xyz.shape[0]), dptr(s0.xyz),
+                                                                  C.c_int64(s0.times_us.size), s0.times_us.ctypes.data_as(capi.c_i64p),
+                                                                  C.c_int64(s0.t_end_us), dptr(values), C.c_int(1 if s0.point_fx == "instant" else 0)))
+            elif all(isinstance(s, tuple) and len(s) == 2 for s in srcs):
+                xyz = f64(srcs[0][0])
+                if xyz.ndim != 2 or xyz.shape[1] != 3 or not all(np.array_equal(f64(s[0]), xyz) for s in srcs):
+                    raise RuntimeError(f"{name}: every member needs the same source positions [n_sources][3]")
+                if not all(np.shape(s[1]) == (T, xyz.shape[0]) for s in srcs):
+                    raise RuntimeError(f"{name}: source values must be [n_steps][n_sources] in every member")
+                values = np.ascontiguousarray(np.stack([f64(s[1]) for s in srcs]))
+                self._ck(self._L.sb2_set_ensemble_sources(self._h, C.c_int(vi), C.c_int64(E), C.c_int64(xyz.shape[0]), dptr(xyz), dptr(values)))
+            else:
+                raise RuntimeError(f"{name}: the members must all give (xyz, values) tuples, all GeoPointSources, or all None")
+        count = max(0, n_steps if n_steps > 0 else T)
+        q = np.zeros((E, count, self.number_of_catchments()))
+        c = np.zeros_like(q)
+        self._ck(self._L.sb2_run_ensemble(self._h, C.byref(ip_parameter), C.c_int(start_step), C.c_int(n_steps), C.c_int(window_steps), dptr(q),
+                                          dptr(c)))
+        self.ip_parameter = ip_parameter
+        return q, c
+
     # -- results -----------------------------------------------------------------------------------------------------------
     def response(self, name, start_step=0, n_steps=None, layout=capi.TIME_MAJOR):
         """cell.rc.<name> for all cells: [n_steps][cell] (or [cell][n_steps])."""
