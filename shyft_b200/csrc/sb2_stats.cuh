@@ -5,7 +5,8 @@
 // gamma_snow_response.sca(cids), ...): a selection of cells (by catchment id or by cell index, empty = all) is summed, or
 // averaged with the cell areas as weights (r += ts * area per cell, then r *= 1 / sum_area), step by step.
 // The reference adds cell after cell; here a block reduces one step's row in a fixed tree (deterministic; differs from the
-// sequential sum by rounding only, tests compare at 1e-12).
+// sequential sum by rounding only: tests compare with the oracle at 1e-12, and with the exact sum within gamma(strides + 13) of the
+// sum of |terms|, tests/test_gpu_statistics_paths.py).
 #pragma once
 #include <stdint.h>
 
